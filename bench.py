@@ -35,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -386,6 +387,33 @@ def hbm_stage_rates(mb, dev, hbm_peak, n=2_000_000):
     return {k: {"GB/s": round(v, 1), "frac_of_hbm_peak": round(v / hbm_peak, 3)} for k, v in res.items()}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, out, info):
+    """Write what the last timed rollout returned as ``out_dir/<name>.npy``: the kept transitions (the dict MOBODY.rollout
+    hands its caller, float32) and the info scalars (float64).  The inputs are seeded, so two builds run with the same
+    arguments can be compared file for file.  Transitions above DUMP_BYTES are replaced by a fixed, seeded sample of rows
+    (``row_index.npy`` holds their positions)."""
+    os.makedirs(out_dir, exist_ok=True)
+    M = int(info["kept_dev"].item())
+    counts, stats = info["counts_dev"].cpu().numpy(), info["stats_dev"].cpu().numpy()
+    rows = {k: v[:M] for k, v in out.items()}
+    row_bytes = sum(v.shape[1] for v in rows.values()) * 4
+    budget = DUMP_BYTES - (1 << 20)                  # headroom for the info arrays and the .npy headers
+    if M * row_bytes > budget:
+        idx = np.sort(np.random.default_rng(0).choice(M, budget // (row_bytes + 8), replace=False))
+        sel = torch.from_numpy(idx).to(next(iter(rows.values())).device)
+        rows = {k: v[sel] for k, v in rows.items()}
+        np.save(os.path.join(out_dir, "row_index.npy"), idx.astype(np.float64))
+    for k, v in rows.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.cpu().numpy().astype(np.float32))
+    T = len(counts) - 2
+    np.save(os.path.join(out_dir, "rows_per_step.npy"), counts[:T].astype(np.float64))
+    np.save(os.path.join(out_dir, "num_transitions.npy"), np.float64(stats[1]))
+    np.save(os.path.join(out_dir, "reward_mean.npy"), np.float64(stats[0] / max(stats[1], 1.0)))
+
+
 def run_reference(args, rank):
     if rank != 0:
         return
@@ -468,9 +496,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the per-config lines and the strong-scaling arm (short ncu runs)")
     ap.add_argument("--exchange", default=os.environ.get("MOBODY_EXCHANGE", "p2p"), choices=["p2p", "nccl"],
                     help="N>1: peer-memory push (default) or the NCCL padded all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the transitions of the last timed rollout as DIR/<name>.npy (single GPU)")
     args = ap.parse_args()
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and world > 1:
+        ap.error("--dump-outputs writes a single-GPU rollout: run it without torchrun")
     if args.impl == "reference":
         return run_reference(args, rank)
     W = max(args.warmup, 3)
@@ -539,6 +573,7 @@ def main():
     side = ag.rollout_streams() if two_streams else None
     produced_side = [torch.zeros(1, dtype=torch.float64, device=dev) for _ in range(2)]
     last_handle = [None]
+    last_rollout = [None]   # N = 1: (transitions dict, info) of the latest rollout, for --dump-outputs
     last_epoch = [None]     # (epoch parity) xor (stream index) of the first two-stream exchange: constant afterwards
 
     def fork_streams():
@@ -562,6 +597,7 @@ def main():
             with torch.cuda.stream(side[i & 1]):
                 o, info = ag.rollout_device(x, T, row0=rank * Bn, sync=False, ws_slot=10 + (i & 1), verify_images=False)
                 produced_side[i & 1].add_(info["stats_dev"][1:2])
+                last_rollout[0] = o, info
             return
         if side:
             st = side[i & 1]
@@ -578,6 +614,7 @@ def main():
             return
         if dist is None:
             o, info = ag.rollout_device(x, T, row0=rank * Bn, sync=False)
+            last_rollout[0] = o, info
         elif exchange == "p2p":
             # shard = this rank's start states; the pack stage pushes the kept transitions into every rank's receive buffer
             h = P.sharded_rollout(ag, x, T, sharded_input=True, gather="p2p")
@@ -619,6 +656,9 @@ def main():
     wall = time.perf_counter() - wall0
     dev_ms = e0.elapsed_time(e1)
     n_trans = float(produced.item())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_rollout[0])
+    last_rollout[0] = None
     if last_handle[0] is not None and check is not None and not os.environ.get("MOBODY_PROBE"):
         # the last timed step, as every rank received it: the headers in MY receive buffer must add up to what the ranks
         # say they produced (device counters, all-reduced) -- the two-stream pipeline delivered complete results
