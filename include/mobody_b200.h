@@ -20,6 +20,7 @@ extern "C" {
 #endif
 
 #define MOBODY_ABI_VERSION 2
+#define MOBODY_TC_TRAIN_MIN_ROWS 1280  /* mobody_train_step runs on tcgen05 GEMM tiles from this many batch rows, below on mma.sync */
 #define MOBODY_E 7            /* ensemble members      (train_mobody.py:795) */
 #define MOBODY_H 256          /* hidden width          (train_mobody.py:794) */
 #define MOBODY_N_DYN_LAYERS 13

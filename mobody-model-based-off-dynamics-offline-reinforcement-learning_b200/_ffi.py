@@ -22,6 +22,7 @@ DYN_LAYER_NAMES = ("zs1", "zs2", "zs3", "za_src1", "za_src2", "za_trg1", "za_trg
 PREC = {"fp32": 0, "bf16x2": 1, "fp16": 3}
 ENABLED_PRECISIONS = ("fp32", "bf16x2", "fp16")
 ABI_VERSION = 2
+TC_TRAIN_MIN_ROWS = 1280   # MOBODY_TC_TRAIN_MIN_ROWS: mobody_train_step runs on tcgen05 GEMM tiles from this many batch rows
 KEEP_U8_ZERO, KEEP_F32_LE, KEEP_F32_LT, KEEP_U8_VALID = 0, 1, 2, 3
 
 

@@ -1,7 +1,6 @@
 // C-ABI entry points (include/mobody_b200.h).  Argument checking + kernel launches only.
 #include <stdio.h>
 #include <string.h>
-#include <stdlib.h>
 #include "../../include/mobody_b200.h"
 #include "common.cuh"
 #include "tc_layout.h"
@@ -130,15 +129,11 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
       if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
       {   // one CTA per 128-row tile; the single bf16 plane (diagnostic mode) fits two row tiles per SM -> two-tiles-in-flight kernel
         if (d->precision == MOBODY_PREC_BF16) {
-          static int duo = -1;
-          if (duo < 0) { const char* e = getenv("MOBODY_TC_DUO"); duo = (e && atoi(e) == 0) ? 0 : 1; }
-          if (duo) {
-            bool launched = false;
-            err = mb_tc_duo_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr, 0,
-                                        (cudaStream_t)stream, &launched);
-            if (err) return fail(MOBODY_ERR_UNSUPPORTED, err);
-            if (launched) return check_launch("mobody_step");
-          }
+          bool launched = false;
+          err = mb_tc_duo_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr, 0,
+                                      (cudaStream_t)stream, &launched);
+          if (err) return fail(MOBODY_ERR_UNSUPPORTED, err);
+          if (launched) return check_launch("mobody_step");
         }
         err = mb_tc_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr,
                                 d->precision == MOBODY_PREC_BF16X2 ? 2 : 1, (cudaStream_t)stream);

@@ -6,7 +6,6 @@
 //     [ state(S) | action(A) | next_state(S) | reward | not_done | 0-pad ]
 // so that sample() is a 128-bit-vectorised row gather and add_batch() a row scatter.
 #include "common.cuh"
-#include <stdlib.h>
 #include "philox.cuh"
 #include "term.cuh"
 #include "../../include/mobody_b200.h"
@@ -409,8 +408,7 @@ void mb_pack_rows_launch(const float* s, const float* a, const float* ns, const 
   const bool aligned = ((reinterpret_cast<uintptr_t>(s) | reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(ns) |
                          reinterpret_cast<uintptr_t>(r) | reinterpret_cast<uintptr_t>(d) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
   const size_t smem = (size_t)buf::PACK_TR * rw * sizeof(float);
-  static const int threads = [] { const char* e = getenv("MOBODY_PACK_THREADS"); return e && atoi(e) >= 32 && atoi(e) <= 256 ? atoi(e) : 128; }();   // measured: 128 x 16 CTAs per SM 0.91 of the HBM peak, 256 x 8: 0.73
-  static const int per_sm = [] { const char* e = getenv("MOBODY_PACK_CTAS"); return e && atoi(e) > 0 ? atoi(e) : 16; }();
+  constexpr int threads = 128, per_sm = 16;   // measured: 128 x 16 CTAs per SM 0.91 of the HBM peak, 256 x 8: 0.73
   const int nvs = (buf::PACK_TR / 4 * S + threads - 1) / threads, nva = (buf::PACK_TR / 4 * A + threads - 1) / threads;   // 128-bit loads per thread per array
   if (aligned && n >= 4096 && smem <= 48 * 1024 && nvs <= 8 && nva <= 4) {
     const long long tiles = (n + buf::PACK_TR - 1) / buf::PACK_TR;

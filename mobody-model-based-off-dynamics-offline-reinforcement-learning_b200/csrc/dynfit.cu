@@ -443,7 +443,7 @@ const char* mb_dynfit_step_launch(const mobody_dynfit_desc& dsc, cudaStream_t st
       j.A = X + (size_t)e * rows * ldx; j.lda = ldx; j.a_src = ug::SRC_KCONTIG;
       j.B = dsc.params.w[l.idx] + (size_t)e * l.in * l.out; j.ldb = l.out; j.b_src = ug::SRC_RCONTIG;
       j.M = rows; j.N = l.out; j.K = l.in; j.bias = dsc.params.b[l.idx] + (size_t)e * l.out;
-      j.epi = pre ? ug::EPI_SWISH : ug::EPI_STORE; j.scale = 1.f;
+      j.epi = pre ? ug::EPI_SWISH : ug::EPI_STORE;
       j.C = C + (size_t)e * rows * ldc; j.ldc = ldc; j.pre = pre ? pre + (size_t)e * rows * ldc : nullptr;
     }
     return g;
@@ -456,7 +456,7 @@ const char* mb_dynfit_step_launch(const mobody_dynfit_desc& dsc, cudaStream_t st
       ug::Job& j = g.job[e];
       j.A = dY + (size_t)e * rows * ldy; j.lda = ldy; j.a_src = ug::SRC_KCONTIG;
       j.B = dsc.params.w[l.idx] + (size_t)e * l.in * l.out; j.ldb = l.out; j.b_src = ug::SRC_KCONTIG;
-      j.M = rows; j.N = l.in; j.K = l.out; j.scale = 1.f;
+      j.M = rows; j.N = l.in; j.K = l.out;
       j.epi = pre ? ug::EPI_DSWISH : ug::EPI_STORE;
       j.mask = pre ? pre + (size_t)e * rows * ldc : nullptr; j.ldmask = ldc;
       j.C = C + (size_t)e * rows * ldc; j.ldc = ldc;
@@ -470,7 +470,7 @@ const char* mb_dynfit_step_launch(const mobody_dynfit_desc& dsc, cudaStream_t st
       ug::Job& j = g.job[e];
       j.A = dY + (size_t)e * rows * ldy; j.lda = ldy; j.a_src = ug::SRC_RCONTIG;
       j.B = X + (size_t)e * rows * ldx; j.ldb = ldx; j.b_src = ug::SRC_RCONTIG;
-      j.M = l.out; j.N = l.in; j.K = rows; j.epi = ug::EPI_PART; j.scale = 1.f;
+      j.M = l.out; j.N = l.in; j.K = rows; j.epi = ug::EPI_PART;
       j.C = w.gw[li] + (size_t)e * ns * l.out * l.in; j.db = w.gb[li] + (size_t)e * ns * l.out;
     }
     return g;

@@ -201,10 +201,7 @@ __device__ void big_layer_mma(const float* __restrict__ Xs, int ldx, int K, cons
       }
     }
   };
-#ifndef MOBODY_PF2
-#define MOBODY_PF2 4
-#endif
-  constexpr int PF = (RPT <= 2) ? MOBODY_PF2 : 2;              // k16 blocks of weights in flight (deeper did not pay at 64 rows)
+  constexpr int PF = (RPT <= 2) ? 4 : 2;              // k16 blocks of weights in flight (deeper did not pay at 64 rows)
   float rb[PF][4][4];
 #pragma unroll
   for (int p = 0; p < PF; ++p) if (p < kblocks) load_b(p, rb[p]);

@@ -22,7 +22,7 @@
 //
 // Precision: NS = 2 -> bf16 hi+lo split of both operands, 3 MMAs per K step (hi*hi + lo*hi + hi*lo), ~2^-16 per
 // product: inside the 1e-4 bound (the default mode).  NS = 1 -> single bf16 pass (bound 2e-2; used when the two-tile
-// kernel does not fit or MOBODY_TC_DUO=0).  Biases come from a shared-memory ring staged by the producer warp; swish
+// kernel does not fit).  Biases come from a shared-memory ring staged by the producer warp; swish
 // layers are packed pre-scaled (tc_layout.h: tc_swish_scales) so the epilogue needs no multiply before the SFU op.
 #include "common.cuh"
 #include "philox.cuh"
@@ -31,13 +31,13 @@
 #include "tc_layout.h"
 #include "tc_epi.cuh"
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 namespace tcs {
 using namespace tce;
 
 
 constexpr int TM = 128;
+constexpr int NG = 4;                    // epilogue groups of 4 warps (one warp per TMEM lane quadrant)
 constexpr uint32_t MAIN_PLANE = 65536;   // 128 rows x 256 k x bf16
 constexpr int MAX_NST = 12;
 constexpr int NB = 4;                    // bias ring slots (one layer's bias each)
@@ -59,11 +59,7 @@ struct Bars {
 // NG groups of 4 epilogue warps (one warp per TMEM lane quadrant).  Every 32-column accumulator chunk is
 // processed by ALL groups at once (group g takes columns [g*CW, (g+1)*CW) of the chunk, CW = 32/NG), so
 // chunks complete in order and the next layer's MMAs trail the epilogue by one chunk.
-// MC: the CTAs of a 2-CTA cluster (two row tiles on two SMs) share the weight stream: each producer fetches HALF of every
-// ring stage and multicasts it into both CTAs' rings (each CTA's "full" barrier collects both halves); a stage is free when
-// BOTH CTAs' MMAs have committed it (multicast commit, "empty" barriers count 2).  Halves the L2 -> SMEM weight traffic,
-// the measured limiter of the 256-deep layers.
-template <int NS, int NG, bool MC = false>
+template <int NS>
 __global__ void __launch_bounds__(32 * (4 * NG + 2), 1)
 step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const unsigned char* __restrict__ polb,
                const __grid_constant__ TcSched sched, const Cfg cfg) {
@@ -73,8 +69,7 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
   const int S = a.S, A = a.A, B = a.B;
   const int live = a.n_rows_dev ? min(*a.n_rows_dev, B) : B;
   const int row0 = blockIdx.x * TM;
-  if ((MC ? (int)(blockIdx.x & ~1u) * TM : row0) >= live) return;      // MC: a tile-less CTA next to a live one still takes part in the ring protocol
-  const uint32_t crank = MC ? tc::cluster_ctarank() : 0u;
+  if (row0 >= live) return;
 
   unsigned char* A_main = smem;
   unsigned char* A_small = A_main + NS * MAIN_PLANE;
@@ -86,7 +81,7 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   if (tid == 0) {
-    for (int i = 0; i < cfg.nst; ++i) { tc::mbar_init(&bars->w_full[i], 1); tc::mbar_init(&bars->w_empty[i], MC ? 2 : 1); }
+    for (int i = 0; i < cfg.nst; ++i) { tc::mbar_init(&bars->w_full[i], 1); tc::mbar_init(&bars->w_empty[i], 1); }
     for (int i = 0; i < 8; ++i) tc::mbar_init(&bars->a_ready[i], EPI_WARPS);   // every epilogue warp announces every chunk
     for (int i = 0; i < 2; ++i) { tc::mbar_init(&bars->d_full[i], 1); tc::mbar_init(&bars->d_empty[i], EPI_WARPS); }
     for (int i = 0; i < NB; ++i) { tc::mbar_init(&bars->b_full[i], 1); tc::mbar_init(&bars->b_empty[i], EPI_WARPS); }
@@ -95,7 +90,6 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
   if (warp == PROD_WARP) tc::tmem_alloc(&bars->tmem_slot, 512);
   tc::tc_fence_before();
   __syncthreads();
-  if (MC) tc::cluster_sync();                                            // both CTAs' barriers exist before anything remote touches them
   tc::tc_fence_after();
   const uint32_t tmem = bars->tmem_slot;
 
@@ -118,11 +112,6 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
         for (int s = 0; s < L.ksteps; ++s) {
           tc::mbar_wait(&bars->w_empty[stage], phase ^ 1u);
           tc::mbar_arrive_expect_tx(&bars->w_full[stage], bytes);
-          if (MC) {
-            const uint32_t half = bytes >> 1;
-            tc::bulk_g2s_multicast(wst + (size_t)stage * cfg.stage_bytes + crank * half, src + (size_t)s * bytes + crank * half, half,
-                                   &bars->w_full[stage], (uint16_t)3);
-          } else
           tc::bulk_g2s(wst + (size_t)stage * cfg.stage_bytes, src + (size_t)s * bytes, bytes, &bars->w_full[stage]);
           if (++stage == cfg.nst) { stage = 0; phase ^= 1u; }
         }
@@ -162,7 +151,7 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
             tc::umma_bf16(dcol, al, bh, idesc, 1u);
             tc::umma_bf16(dcol, ah, bl, idesc, 1u);
           }
-          if (MC) tc::umma_commit_multicast(&bars->w_empty[stage], (uint16_t)3); else tc::umma_commit(&bars->w_empty[stage]);
+          tc::umma_commit(&bars->w_empty[stage]);
           if (++stage == cfg.nst) { stage = 0; wphase ^= 1u; }
         }
         tc::umma_commit(&bars->d_full[buf]);
@@ -543,7 +532,6 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
 
   tc::tc_fence_before();
   __syncthreads();
-  if (MC) tc::cluster_sync();                                            // the peer may still arrive on this CTA's barriers
   if (warp == PROD_WARP) tc::tmem_dealloc(tmem, 512);
 }
 
@@ -755,37 +743,24 @@ const char* mb_tc_step_launch(const StepArgs& a, const unsigned char* dynb, cons
   if (nst > tcs::MAX_NST) nst = tcs::MAX_NST;
   cfg.nst = nst;
   const size_t bytes = fixed + (size_t)nst * cfg.stage_bytes;
-  static int ng = 0;
-  if (!ng) { const char* e = getenv("MOBODY_TC_GROUPS"); ng = (e && atoi(e) == 2) ? 2 : 4; }
-  static const bool mc = [] { const char* e = getenv("MOBODY_TC_MULTICAST"); return e && e[0] == '1'; }();
-  const bool use_mc = mc && ns == 2 && ng == 4;
-  auto kern = use_mc ? tcs::step_tc_kernel<2, 4, true>
-            : ns == 2 ? (ng == 2 ? tcs::step_tc_kernel<2, 2> : tcs::step_tc_kernel<2, 4>)
-                      : (ng == 2 ? tcs::step_tc_kernel<1, 2> : tcs::step_tc_kernel<1, 4>);
+  auto kern = ns == 2 ? tcs::step_tc_kernel<2> : tcs::step_tc_kernel<1>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
     return "cudaFuncSetAttribute(step_tc_kernel) failed";
-  int grid = (a.B + tcs::TM - 1) / tcs::TM;
-  if (use_mc) grid = (grid + 1) & ~1;
   // Every tile streams the whole weight image (6.5 MB at obs 17 / act 6) from L2: mark it persisting so that the rows
-  // flowing through L2 -- this kernel's own I/O and, on a multi-GPU box, the peers' incoming transitions -- cannot evict it
-  // (MOBODY_L2_PERSIST=0 turns the hint off for A/B runs).
-  static const bool persist = [] { const char* e = getenv("MOBODY_L2_PERSIST"); return !(e && e[0] == '0'); }();
+  // flowing through L2 -- this kernel's own I/O and, on a multi-GPU box, the peers' incoming transitions -- cannot evict it.
+  static thread_local int limit_dev = -1;
+  int dev = 0; cudaGetDevice(&dev);
+  if (limit_dev != dev) { cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)32 << 20); limit_dev = dev; }
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeAccessPolicyWindow;
+  at[0].val.accessPolicyWindow.base_ptr = const_cast<unsigned char*>(dynb);
+  at[0].val.accessPolicyWindow.num_bytes = DL.total_bytes;
+  at[0].val.accessPolicyWindow.hitRatio = 1.0f;
+  at[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
+  at[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
   cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3(grid); lc.blockDim = dim3(32 * (4 * ng + 2)); lc.dynamicSmemBytes = bytes; lc.stream = st;
-  cudaLaunchAttribute at[2];
-  if (use_mc) { at[1].id = cudaLaunchAttributeClusterDimension; at[1].val.clusterDim.x = 2; at[1].val.clusterDim.y = 1; at[1].val.clusterDim.z = 1; }
-  if (persist) {
-    static thread_local int limit_dev = -1;
-    int dev = 0; cudaGetDevice(&dev);
-    if (limit_dev != dev) { cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)32 << 20); limit_dev = dev; }
-    at[0].id = cudaLaunchAttributeAccessPolicyWindow;
-    at[0].val.accessPolicyWindow.base_ptr = const_cast<unsigned char*>(dynb);
-    at[0].val.accessPolicyWindow.num_bytes = DL.total_bytes;
-    at[0].val.accessPolicyWindow.hitRatio = 1.0f;
-    at[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    at[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    lc.attrs = at; lc.numAttrs = use_mc ? 2 : 1;
-  } else if (use_mc) { lc.attrs = at + 1; lc.numAttrs = 1; }
+  lc.gridDim = dim3((a.B + tcs::TM - 1) / tcs::TM); lc.blockDim = dim3(32 * (4 * tcs::NG + 2)); lc.dynamicSmemBytes = bytes; lc.stream = st;
+  lc.attrs = at; lc.numAttrs = 1;
   const unsigned char* polp = polb ? polb : dynb;
   if (cudaLaunchKernelEx(&lc, kern, a, dynb, polp, sc, cfg) != cudaSuccess) return "step_tc_kernel launch failed";
   return nullptr;

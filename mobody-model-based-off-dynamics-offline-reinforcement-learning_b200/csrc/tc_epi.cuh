@@ -4,10 +4,6 @@
 #pragma once
 #include "tc_prims.cuh"
 
-#ifndef MOBODY_EPI_SHARE
-#define MOBODY_EPI_SHARE 2   // elements per reciprocal in the exact-mode swish: 0 (= one each), 2 or 4 (measured: 2 is best)
-#endif
-
 namespace tce {
 
 template <int W> __device__ __forceinline__ void epi_bar() { asm volatile("bar.sync 1, %0;" ::"n"(32 * W) : "memory"); }   // epilogue warps only
@@ -47,25 +43,15 @@ __device__ __forceinline__ void act8(const uint32_t* x, const float* b, float (&
     for (int i = 0; i < 8; ++i) v[i] = fmaf(t[i], th[i], t[i]);
   } else {
     float e[8];
-#if MOBODY_EPI_SHARE == 0
-#pragma unroll
-    for (int i = 0; i < 8; ++i) asm volatile("ex2.approx.ftz.f32 %0, %1;" : "=f"(e[i]) : "f"(t[i]));
-#pragma unroll
-    for (int i = 0; i < 8; ++i) e[i] += 1.0f;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) asm volatile("rcp.approx.ftz.f32 %0, %1;" : "=f"(e[i]) : "f"(e[i]));
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = t[i] * e[i];
-#else
-    // One reciprocal serves MOBODY_EPI_SHARE elements: 1/a_i = (prod_{j != i} a_j) * (1 / prod_j a_j), a = 1 + 2^t >= 1.
-    // The exponent argument is clamped so the product stays finite (2^60 per pair, 2^30 per quad): beyond the clamp
-    // swish(x) is below 3e-8 in magnitude either way (x < -20.8), far inside the fp32-parity bound.
-    constexpr float kClamp = MOBODY_EPI_SHARE == 2 ? 60.f : 30.f;
+    // One reciprocal serves a pair: 1/a_0 = a_1 * (1 / (a_0 a_1)), 1/a_1 = a_0 * (1 / (a_0 a_1)), a = 1 + 2^t >= 1 (measured
+    // against one reciprocal per element and one per quad: the pair is fastest).  The exponent argument is clamped so the
+    // product stays finite (2^60 per factor): beyond the clamp swish(x) is below 3e-8 in magnitude either way (x < -20.8), far
+    // inside the fp32-parity bound.
+    constexpr float kClamp = 60.f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) asm volatile("ex2.approx.ftz.f32 %0, %1;" : "=f"(e[i]) : "f"(fminf(t[i], kClamp)));
 #pragma unroll
     for (int i = 0; i < 8; ++i) e[i] += 1.0f;
-#if MOBODY_EPI_SHARE == 2
     float r[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) asm volatile("rcp.approx.ftz.f32 %0, %1;" : "=f"(r[i]) : "f"(e[2 * i] * e[2 * i + 1]));
@@ -74,22 +60,6 @@ __device__ __forceinline__ void act8(const uint32_t* x, const float* b, float (&
       v[2 * i] = (t[2 * i] * e[2 * i + 1]) * r[i];
       v[2 * i + 1] = (t[2 * i + 1] * e[2 * i]) * r[i];
     }
-#else
-    float p01[2], p23[2], r[2];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) { p01[i] = e[4 * i] * e[4 * i + 1]; p23[i] = e[4 * i + 2] * e[4 * i + 3]; }
-#pragma unroll
-    for (int i = 0; i < 2; ++i) asm volatile("rcp.approx.ftz.f32 %0, %1;" : "=f"(r[i]) : "f"(p01[i] * p23[i]));
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      const float r01 = r[i] * p23[i], r23 = r[i] * p01[i];
-      v[4 * i] = (t[4 * i] * e[4 * i + 1]) * r01;
-      v[4 * i + 1] = (t[4 * i + 1] * e[4 * i]) * r01;
-      v[4 * i + 2] = (t[4 * i + 2] * e[4 * i + 3]) * r23;
-      v[4 * i + 3] = (t[4 * i + 3] * e[4 * i + 2]) * r23;
-    }
-#endif
-#endif
   }
 }
 
@@ -131,6 +101,5 @@ __device__ __forceinline__ void store8_f16(unsigned char* base, uint32_t off, co
 
 template <int CW> __device__ __forceinline__ void tmem_ldw(uint32_t taddr, uint32_t (&x)[CW]);
 template <> __device__ __forceinline__ void tmem_ldw<8>(uint32_t taddr, uint32_t (&x)[8]) { tc::tmem_ld8(taddr, x); }
-template <> __device__ __forceinline__ void tmem_ldw<16>(uint32_t taddr, uint32_t (&x)[16]) { tc::tmem_ld16(taddr, x); }
 
 }  // namespace tce

@@ -146,17 +146,6 @@ __device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t pa
 __device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
   while (!mbar_try_wait_cluster(bar, parity)) {}
 }
-// bulk copy global -> the SAME shared-memory offset in every CTA of `cta_mask`; each destination's mbarrier (same offset)
-// receives the byte count
-__device__ __forceinline__ void bulk_g2s_multicast(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;"
-               ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
-// commit of THIS CTA's MMAs: arrives on the barrier at this offset in every CTA of `cta_mask`
-__device__ __forceinline__ void umma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 __device__ __forceinline__ void tmem_alloc2(uint32_t* smem_slot, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)), "r"(ncols) : "memory");
@@ -192,22 +181,13 @@ __device__ __forceinline__ bool elect_one() {
 
 // ---------------- bf16 split helpers ----------------
 // hi = top 16 bits of v (truncation; exact, so v - hi is exact in fp32 and has the sign of v),
-// lo = bf16(v - hi) rounded to nearest (one F2FP for two values; MOBODY_LO_F2FP=0: integer add + byte permute, half-away).  hi+lo carries ~16 significand bits of v (error <= 2^-16 |v|);
+// lo = bf16(v - hi) rounded to nearest (one F2FP for two values).  hi+lo carries ~16 significand bits of v (error <= 2^-16 |v|);
 // the rounding of lo is unbiased, the truncation of hi is fully compensated by lo.
 // Packing two values into one 32-bit word is a byte permute (low half = first value).
-#ifndef MOBODY_LO_F2FP
-#define MOBODY_LO_F2FP 1   // 1: pack the lo plane with one F2FP (cvt.rn.bf16x2.f32) instead of two adds + a byte permute
-#endif
 __device__ __forceinline__ void split2(float v0, float v1, uint32_t& hi, uint32_t& lo) {
   const uint32_t u0 = __float_as_uint(v0), u1 = __float_as_uint(v1);
   hi = __byte_perm(u0, u1, 0x7632);
-#if MOBODY_LO_F2FP
   asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(v1 - __uint_as_float(u1 & 0xFFFF0000u)), "f"(v0 - __uint_as_float(u0 & 0xFFFF0000u)));
-#else
-  const uint32_t l0 = __float_as_uint(v0 - __uint_as_float(u0 & 0xFFFF0000u)) + 0x8000u;
-  const uint32_t l1 = __float_as_uint(v1 - __uint_as_float(u1 & 0xFFFF0000u)) + 0x8000u;
-  lo = __byte_perm(l0, l1, 0x7632);
-#endif
 }
 __device__ __forceinline__ uint32_t pack_bf16(float v0, float v1) {
   return __byte_perm(__float_as_uint(v0) + 0x8000u, __float_as_uint(v1) + 0x8000u, 0x7632);

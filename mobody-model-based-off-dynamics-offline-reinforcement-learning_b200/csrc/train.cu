@@ -923,15 +923,13 @@ __global__ void __launch_bounds__(128) policy_grad_kernel(const PolicyBwdArgs a)
 }  // namespace trn
 
 // ---------------- host launchers ----------------
-// Row tile: 16 rows per CTA for small batches so that a 320-row batch still spreads over 20 SMs; 32 rows once the 16-row
-// tiles would exceed one CTA per SM (>= 2 368 rows; measured cross-over between 1 280 and 2 560 rows, MOBODY_TRAIN_TM_ROWS),
-// two CTAs per SM (128 registers, 70 KB shared memory each): 16 warps per SM hide the L2 / HMMA latencies that one 64-row
-// CTA per SM (8 warps) exposes -- batch 4096: 1 025 -> 1 304 updates/s.  MOBODY_TRAIN_TM=64 selects the old tiling (A/B).
-static int pick_tm(int N) {
-  static const int big = [] { const char* e = getenv("MOBODY_TRAIN_TM"); const int v = e ? atoi(e) : 32; return v == 64 ? 64 : 32; }();
-  static const int min_rows = [] { const char* e = getenv("MOBODY_TRAIN_TM_ROWS"); return e ? atoi(e) : 148 * 16; }();
-  return N >= min_rows ? big : 16;
-}
+// Row tile of the mma.sync kernels: 16 rows per CTA so that a 320-row batch still spreads over 20 SMs.  The train step runs
+// them only below MOBODY_TC_TRAIN_MIN_ROWS, where 16-row tiles are always used.  The classifier takes 32 rows per CTA once the
+// 16-row tiles would exceed one CTA per SM (>= 2 368 rows; measured cross-over between 1 280 and 2 560 rows), two CTAs per SM
+// (128 registers, 70 KB shared memory each): 16 warps per SM hide the L2 / HMMA latencies that one 64-row CTA per SM (8 warps)
+// exposes -- train step at batch 4096: 1 025 -> 1 304 updates/s.
+constexpr int TRAIN_TM = 16;
+static int pick_tm(int N) { return N >= 148 * 16 ? 32 : 16; }
 template <typename K> static const char* set_smem(K kern, size_t bytes) {
   if (bytes > 227 * 1024) return "train step: shared memory budget exceeded for this (S, A)";
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess) return "cudaFuncSetAttribute failed";
@@ -939,11 +937,12 @@ template <typename K> static const char* set_smem(K kern, size_t bytes) {
 }
 
 const char* mb_train_critic_launch(const trn::CriticArgs& a, cudaStream_t st) {
-  const int tm = pick_tm(a.N), ntiles = (a.N + tm - 1) / tm;
+  constexpr int tm = TRAIN_TM;
+  const int ntiles = (a.N + tm - 1) / tm;
   const size_t bytes = (2 * (size_t)tm * simt::H + (size_t)tm * simt::rup16(a.S + a.A) + 2 * tm + 8) * sizeof(float);
-  auto k1 = tm == 64 ? trn::critic_fwd_kernel<8> : tm == 32 ? trn::critic_fwd_kernel<4> : trn::critic_fwd_kernel<2>;
-  auto k2 = tm == 64 ? trn::critic_tgt_kernel<8> : tm == 32 ? trn::critic_tgt_kernel<4> : trn::critic_tgt_kernel<2>;
-  auto k3 = tm == 64 ? trn::critic_bwd_kernel<8> : tm == 32 ? trn::critic_bwd_kernel<4> : trn::critic_bwd_kernel<2>;
+  auto k1 = trn::critic_fwd_kernel<tm / 8>;
+  auto k2 = trn::critic_tgt_kernel<tm / 8>;
+  auto k3 = trn::critic_bwd_kernel<tm / 8>;
   if (const char* e = set_smem(k1, bytes)) return e;
   if (const char* e = set_smem(k2, bytes)) return e;
   if (const char* e = set_smem(k3, bytes)) return e;
@@ -953,17 +952,18 @@ const char* mb_train_critic_launch(const trn::CriticArgs& a, cudaStream_t st) {
   return nullptr;
 }
 const char* mb_train_actor_launch(const trn::ActorArgs& a, cudaStream_t st) {
-  const int tm = pick_tm(a.N), ntiles = (a.N + tm - 1) / tm;
+  constexpr int tm = TRAIN_TM;
+  const int ntiles = (a.N + tm - 1) / tm;
   const size_t bytes = (2 * (size_t)tm * simt::H + (size_t)tm * simt::rup16(a.S + a.A) + 2 * tm + (size_t)tm * a.A + 8) * sizeof(float);
-  auto k2 = tm == 64 ? trn::actor_q_kernel<8> : tm == 32 ? trn::actor_q_kernel<4> : trn::actor_q_kernel<2>;
+  auto k2 = trn::actor_q_kernel<tm / 8>;
   if (const char* e = set_smem(k2, bytes)) return e;
   mb_launch(k2, dim3(ntiles, 4), dim3(simt::NT), bytes, st, a);
   return nullptr;
 }
 const char* mb_train_policy_bwd_launch(const trn::PolicyBwdArgs& a, cudaStream_t st) {
-  const int tm = pick_tm(a.N);
+  constexpr int tm = TRAIN_TM;
   size_t bytes = (2 * (size_t)tm * simt::H + (size_t)tm * simt::rup16(a.A) + tm + 40) * sizeof(float);
-  auto kern = tm == 64 ? trn::policy_bwd_kernel<8> : tm == 32 ? trn::policy_bwd_kernel<4> : trn::policy_bwd_kernel<2>;
+  auto kern = trn::policy_bwd_kernel<tm / 8>;
   if (const char* e = set_smem(kern, bytes)) return e;
   mb_launch(kern, dim3((a.N + tm - 1) / tm), dim3(simt::NT), bytes, st, a);
   return nullptr;
@@ -991,14 +991,14 @@ const char* mb_train_adam_launch(const trn::AdamArgs& a, cudaStream_t st) {
 
 // ---------------- whole train step (C ABI: mobody_train_step) ----------------
 struct TrainWs {   // float offsets into the workspace
-  size_t Hq[2][2], Dq[2][2], d3[2], part, Hp[2], Dp[2], api, a2, qk[2], qtk[2], qv[2], qh[2], gak[2], d3p, scal, part2, cnt, gq[2][6], gp[6], T[2], img[17], pa[5], total;
+  size_t Hq[2][2], Dq[2][2], d3[2], part, Hp[2], Dp[2], api, a2, qk[2], qtk[2], qv[2], qh[2], gak[2], d3p, scal, part2, cnt, gq[2][6], gp[6], T[2], img[17], total;
   int ntiles;
 };
 static TrainWs train_ws(int N, int S, int A, int nsplit) {
   TrainWs w{}; size_t o = 0;
   auto take = [&](size_t n) { size_t r = o; o += (n + 3) & ~(size_t)3; return r; };
   const size_t act = (size_t)N * 256;
-  w.ntiles = (N + 15) / 16;                          // upper bound over both row-tile sizes
+  w.ntiles = (N + TRAIN_TM - 1) / TRAIN_TM;          // upper bound: the tcgen05 path's 256-row blocks need fewer
   for (int k = 0; k < 2; ++k) for (int l = 0; l < 2; ++l) { w.Hq[k][l] = take(act); w.Dq[k][l] = take(act); }
   for (int k = 0; k < 2; ++k) w.d3[k] = take(N);
   w.part = take((size_t)w.ntiles * 4);
@@ -1015,9 +1015,6 @@ static TrainWs train_ws(int N, int S, int A, int nsplit) {
     const int ik[17] = {S, 256, 256, S + A, S + A, 256, 256, S + A, S + A, 256, 256, 256, 256, A, 256, 256, 256};
     const int inp[17] = {256, 256, 64, 256, 256, 256, 256, 256, 256, 256, 256, 256, 256, 256, 256, 64, 64};
     for (int i = 0; i < 17; ++i) w.img[i] = take(ug::packed_floats(ik[i], inp[i]));
-    // packed A images of the five layer-1 outputs that feed a 256-deep layer (T0, T1, Hq[0][0], Hq[1][0], Hp[0]): emitted by the producing
-    // launch's epilogue, streamed by the consumer's TMA
-    for (int i = 0; i < 5; ++i) w.pa[i] = take((size_t)((N + 127) / 128) * ug::packed_a_tile_floats(256));
   }
   w.total = o;
   return w;
@@ -1026,12 +1023,12 @@ long long mb_train_workspace_bytes(int N, int S, int A, int nsplit) { return (lo
 
 static MlpPtrs as_ptrs(const mobody_mlp_state& s) { MlpPtrs p; for (int i = 0; i < 3; ++i) { p.w[i] = s.w[i]; p.b[i] = s.b[i]; } return p; }
 
-// ---------------- large-batch update on tcgen05 (rows >= 2368: the GEMMs are throughput bound) ----------------
+// ---------------- large-batch update on tcgen05 (rows >= MOBODY_TC_TRAIN_MIN_ROWS: the GEMMs are throughput bound) ----------------
 const char* mb_gemm_launch(const ug::Args& a, cudaStream_t st);     // train_tc.cu
 
 static ug::Job gemm_job(const float* A, int lda, int a_src, const float* B, int ldb, int b_src, int M, int N, int K) {
   ug::Job j{}; j.A = A; j.lda = lda; j.a_src = a_src; j.B = B; j.ldb = ldb; j.b_src = b_src; j.M = M; j.N = N; j.K = K;
-  j.epi = ug::EPI_STORE; j.scale = 1.f;
+  j.epi = ug::EPI_STORE;
   return j;
 }
 // forward layer: C = act(A W^T + b); nn.Linear weight [out][in] is the K-contiguous B operand
@@ -1052,7 +1049,6 @@ static ug::Job wgrad_job(const float* D, int ldd, int O, const float* X, int ldx
   j.epi = ug::EPI_PART; j.C = dW; j.db = db;
   return j;
 }
-static ug::Job packed(ug::Job j, const float* image) { j.B = image; j.b_src = ug::SRC_PACKED; return j; }
 const char* mb_pack_b_launch(const ug::PackArgs& a, cudaStream_t st);     // train_tc.cu
 static ug::PackJob pack_job(const float* src, int ld, int mode, int N, int K, int NP, float* dst) {
   return ug::PackJob{src, ld, mode, N, K, NP, reinterpret_cast<uint32_t*>(dst)};
@@ -1112,20 +1108,9 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
   // ---- weight images: every weight matrix the GEMMs use as a B operand, split into TF32 hi / lo planes ONCE (one launch) ----
   // slots: 0-2 pi W1 W2 W3 (forward) | 3,4 Q_k W1 | 5,6 Q_k W2 | 7,8 Q'_k W1 | 9,10 Q'_k W2 | 11,12 Q_k W2 (backward) |
   //        13 pi W3 (backward) | 14 pi W2 (backward) | 15,16 action columns of Q_k W1 (backward)
-  static const bool use_img = [] { const char* v = getenv("MOBODY_TRAIN_PACKED"); return !(v && v[0] == '0'); }();
   float* img[17];
   for (int i = 0; i < 17; ++i) img[i] = ws + w.img[i];
-  auto P = [&](ug::Job j, int slot) { return use_img ? packed(j, img[slot]) : j; };
-  // Activations as packed images too (the producing launch's epilogue emits the TF32 hi / lo stage image, the 256-deep consumer
-  // streams both operands by TMA from one thread): bit-identical, and SLOWER -- 2 050 against 2 260 updates/s at batch 4096: ten
-  // layer-1 jobs write 21 MB of image each and their consumers read it back (+420 MB of HBM traffic per update) for a K loop
-  // that was not the whole problem.  Opt-in (MOBODY_TRAIN_PACKED_A=1) for A/B runs.
-  static const bool use_pa = use_img && [] { const char* v = getenv("MOBODY_TRAIN_PACKED_A"); return v && v[0] == '1'; }();
-  float* pa[5];
-  for (int i = 0; i < 5; ++i) pa[i] = ws + w.pa[i];
-  enum { PA_T0 = 0, PA_T1, PA_Q0, PA_Q1, PA_P0 };
-  auto EMIT = [&](ug::Job j, int slot) { if (use_pa) j.apack = pa[slot]; return j; };                 // producer: also write the packed A image
-  auto FROM = [&](ug::Job j, int slot) { if (use_pa) { j.A = pa[slot]; j.a_src = ug::SRC_PACKED; } return j; };   // consumer: stream it
+  auto P = [&](ug::Job j, int slot) { j.B = img[slot]; j.b_src = ug::SRC_PACKED; return j; };   // B operand: weight image `slot`
   auto pack_q = [&](ug::PackArgs& pa, bool with_slices) {
     for (int k = 0; k < 2; ++k) {
       pa.job[pa.njobs++] = pack_job(q[k].w[0], SA, ug::SRC_KCONTIG, 256, SA, 256, img[3 + k]);
@@ -1134,7 +1119,7 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
       if (with_slices) pa.job[pa.njobs++] = pack_job(q[k].w[0] + S, SA, ug::SRC_RCONTIG, A, 256, 64, img[15 + k]);
     }
   };
-  if (use_img) {
+  {
     ug::PackArgs pa{};
     pa.job[pa.njobs++] = pack_job(pi.w[0], S, ug::SRC_KCONTIG, 256, S, 256, img[0]);
     pa.job[pa.njobs++] = pack_job(pi.w[1], 256, ug::SRC_KCONTIG, 256, 256, 256, img[1]);
@@ -1149,13 +1134,13 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
     if ((e = mb_pack_b_launch(pa, st))) return e;
   }
   // ---- critic forward.  layer 1 of pi(s'), Q1(s,a), Q2(s,a), pi(s) side by side; then layer 2 (+ Q heads); then the policy tails ----
-  if ((e = run_gemms(st, 1, EMIT(P(fwd_job(X + SA, rw, N, S, pi.w[0], pi.b[0], 256, T[0]), 0), PA_T0), EMIT(P(fwd_job(X, rw, N, SA, q[0].w[0], q[0].b[0], 256, Hq[0][0]), 3), PA_Q0),
-                     EMIT(P(fwd_job(X, rw, N, SA, q[1].w[0], q[1].b[0], 256, Hq[1][0]), 4), PA_Q1), EMIT(P(fwd_job(X, rw, N, S, pi.w[0], pi.b[0], 256, Hp[0]), 0), PA_P0)))) return e;
+  if ((e = run_gemms(st, 1, P(fwd_job(X + SA, rw, N, S, pi.w[0], pi.b[0], 256, T[0]), 0), P(fwd_job(X, rw, N, SA, q[0].w[0], q[0].b[0], 256, Hq[0][0]), 3),
+                     P(fwd_job(X, rw, N, SA, q[1].w[0], q[1].b[0], 256, Hq[1][0]), 4), P(fwd_job(X, rw, N, S, pi.w[0], pi.b[0], 256, Hp[0]), 0)))) return e;
   {
     ug::Job j1 = fwd_job(Hq[0][0], 256, N, 256, q[0].w[1], q[0].b[1], 256, Hq[0][1]), j2 = fwd_job(Hq[1][0], 256, N, 256, q[1].w[1], q[1].b[1], 256, Hq[1][1]);
     j1.epi = j2.epi = ug::EPI_HEAD; j1.w3 = q[0].w[2]; j1.b3 = q[0].b[2]; j1.out1 = qk[0]; j2.w3 = q[1].w[2]; j2.b3 = q[1].b[2]; j2.out1 = qk[1];
-    if ((e = run_gemms(st, 1, FROM(P(fwd_job(T[0], 256, N, 256, pi.w[1], pi.b[1], 256, T[1]), 1), PA_T0), FROM(P(j1, 5), PA_Q0), FROM(P(j2, 6), PA_Q1),
-                       FROM(P(fwd_job(Hp[0], 256, N, 256, pi.w[1], pi.b[1], 256, Hp[1]), 1), PA_P0)))) return e;
+    if ((e = run_gemms(st, 1, P(fwd_job(T[0], 256, N, 256, pi.w[1], pi.b[1], 256, T[1]), 1), P(j1, 5), P(j2, 6),
+                       P(fwd_job(Hp[0], 256, N, 256, pi.w[1], pi.b[1], 256, Hp[1]), 1)))) return e;
   }
   {
     trn::RowDotArgs rd{}; rd.njobs = 2; rd.A = A; rd.scale = d.max_action; rd.tanh_act = 1;
@@ -1166,11 +1151,11 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
   {
     ug::Job j1 = fwd_job(X + SA, rw, N, SA, qt[0].w[0], qt[0].b[0], 256, T[0]), j2 = fwd_job(X + SA, rw, N, SA, qt[1].w[0], qt[1].b[0], 256, T[1]);
     j1.A2 = j2.A2 = a2; j1.lda2 = j2.lda2 = A; j1.ksplit = j2.ksplit = S;
-    if ((e = run_gemms(st, 1, EMIT(P(j1, 7), PA_T0), EMIT(P(j2, 8), PA_T1)))) return e;
+    if ((e = run_gemms(st, 1, P(j1, 7), P(j2, 8)))) return e;
     // layer 2 + head in place is not possible (C would overwrite A of another tile's... no: tiles own their rows) -> no C store at all
     ug::Job h1 = fwd_job(T[0], 256, N, 256, qt[0].w[1], qt[0].b[1], 256, nullptr), h2 = fwd_job(T[1], 256, N, 256, qt[1].w[1], qt[1].b[1], 256, nullptr);
     h1.epi = h2.epi = ug::EPI_HEAD; h1.w3 = qt[0].w[2]; h1.b3 = qt[0].b[2]; h1.out1 = qtk[0]; h2.w3 = qt[1].w[2]; h2.b3 = qt[1].b[2]; h2.out1 = qtk[1];
-    if ((e = run_gemms(st, 1, FROM(P(h1, 9), PA_T0), FROM(P(h2, 10), PA_T1)))) return e;
+    if ((e = run_gemms(st, 1, P(h1, 9), P(h2, 10)))) return e;
   }
   // ---- TD target + MSE gradient, head backward, backward-data ----
   {
@@ -1209,7 +1194,7 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
       }
   }
   if ((e = mb_train_adam_launch(ad, st))) return e;
-  if (use_img) {   // the critics just changed: their images again (+ the action columns of W1 for dQ/da)
+  {   // the critics just changed: their images again (+ the action columns of W1 for dQ/da)
     ug::PackArgs pa{};
     pack_q(pa, true);
     if ((e = mb_pack_b_launch(pa, st))) return e;
@@ -1218,12 +1203,12 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
   {
     ug::Job j1 = fwd_job(X, rw, N, SA, q[0].w[0], q[0].b[0], 256, Hq[0][0]), j2 = fwd_job(X, rw, N, SA, q[1].w[0], q[1].b[0], 256, Hq[1][0]);
     j1.A2 = j2.A2 = api; j1.lda2 = j2.lda2 = A; j1.ksplit = j2.ksplit = S;
-    if ((e = run_gemms(st, 1, EMIT(P(j1, 3), PA_Q0), EMIT(P(j2, 4), PA_Q1), EMIT(P(fwd_job(X, rw, nt, SA, q[0].w[0], q[0].b[0], 256, T[0]), 3), PA_T0),
-                       EMIT(P(fwd_job(X, rw, nt, SA, q[1].w[0], q[1].b[0], 256, T[1]), 4), PA_T1)))) return e;
+    if ((e = run_gemms(st, 1, P(j1, 3), P(j2, 4), P(fwd_job(X, rw, nt, SA, q[0].w[0], q[0].b[0], 256, T[0]), 3),
+                       P(fwd_job(X, rw, nt, SA, q[1].w[0], q[1].b[0], 256, T[1]), 4)))) return e;
     ug::Job h[4] = {fwd_job(Hq[0][0], 256, N, 256, q[0].w[1], q[0].b[1], 256, Hq[0][1]), fwd_job(Hq[1][0], 256, N, 256, q[1].w[1], q[1].b[1], 256, Hq[1][1]),
                     fwd_job(T[0], 256, nt, 256, q[0].w[1], q[0].b[1], 256, nullptr), fwd_job(T[1], 256, nt, 256, q[1].w[1], q[1].b[1], 256, nullptr)};
     for (int i = 0; i < 4; ++i) { h[i].epi = ug::EPI_HEAD; h[i].w3 = q[i & 1].w[2]; h[i].b3 = q[i & 1].b[2]; h[i].out1 = i < 2 ? qv[i] : qh[i - 2]; }
-    if ((e = run_gemms(st, 1, FROM(P(h[0], 5), PA_Q0), FROM(P(h[1], 6), PA_Q1), FROM(P(h[2], 5), PA_T0), FROM(P(h[3], 6), PA_T1)))) return e;
+    if ((e = run_gemms(st, 1, P(h[0], 5), P(h[1], 6), P(h[2], 5), P(h[3], 6)))) return e;
   }
   trn::ActorArgs ac{};
   ac.X = X; ac.N = N; ac.n_true = nt; ac.S = S; ac.A = A; ac.rw = rw; ac.max_action = d.max_action;
@@ -1279,12 +1264,9 @@ const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st) {
   if (N < 1 || d.n_true < 1 || d.n_true > N || S < 1 || S > 128 || A < 1 || A > 32 || ns < 1 || ns > 64) return "train step: bad N/n_true/S/A/nsplit";
   const TrainWs w = train_ws(N, S, A, ns);
   if (!d.workspace || d.workspace_bytes < (long long)w.total * 4) return "train step: workspace too small";
-  // large batches: every contraction as tcgen05 GEMM tiles (MOBODY_TRAIN_TC=0 keeps the mma.sync path for A/B runs)
-  static const bool use_tc = [] { const char* e = getenv("MOBODY_TRAIN_TC"); return !(e && e[0] == '0'); }();
-  // cross-over measured on the tuned tiles (S17/A6, updates/s tcgen05 vs mma.sync): 640 rows 4 540 vs 6 435, 1 280 rows 4 350 vs 4 220,
-  // 1 920 rows 3 920 vs 3 340, 2 560 rows 4 180 vs 3 600
-  static const int tc_rows = [] { const char* e = getenv("MOBODY_TRAIN_TC_ROWS"); return e ? atoi(e) : 1280; }();
-  if (use_tc && N >= tc_rows) return mb_train_step_tc_launch(d, w, st);
+  // large batches: every contraction as tcgen05 GEMM tiles.  Cross-over measured on the tuned tiles (S17/A6, updates/s tcgen05
+  // vs mma.sync): 640 rows 4 540 vs 6 435, 1 280 rows 4 350 vs 4 220, 1 920 rows 3 920 vs 3 340, 2 560 rows 4 180 vs 3 600
+  if (N >= MOBODY_TC_TRAIN_MIN_ROWS) return mb_train_step_tc_launch(d, w, st);
   float* ws = (float*)d.workspace;
   const mobody_mlp_state* qs[2] = {&d.q1, &d.q2};
   const mobody_mlp_state* qts[2] = {&d.q1_target, &d.q2_target};
@@ -1330,7 +1312,7 @@ const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st) {
   ac.q[0] = as_ptrs(d.q1); ac.q[1] = as_ptrs(d.q2); ac.max_action = d.max_action;
   ac.Hp[0] = ws + w.Hp[0]; ac.Hp[1] = ws + w.Hp[1]; ac.api = ws + w.api;
   for (int k = 0; k < 2; ++k) { ac.qv[k] = ws + w.qv[k]; ac.qh[k] = ws + w.qh[k]; ac.gak[k] = ws + w.gak[k]; }
-  ac.part = ws + w.part; ac.ntiles_c = (N + pick_tm(N) - 1) / pick_tm(N); ac.weight = d.weight; ac.out = ws + w.scal;
+  ac.part = ws + w.part; ac.ntiles_c = (N + TRAIN_TM - 1) / TRAIN_TM; ac.weight = d.weight; ac.out = ws + w.scal;
   ac.counter = reinterpret_cast<int*>(ws + w.cnt);
   if (const char* e = mb_train_actor_launch(ac, st)) return e;
   trn::PolicyBwdArgs pb{}; pb.N = N; pb.n_true = d.n_true; pb.S = S; pb.A = A; pb.rw = d.row_width; pb.pi = ac.pi;
@@ -1401,7 +1383,7 @@ const char* mb_classifier_step_launch(const mobody_classifier_desc& d, cudaStrea
   c.part = ws + w.part;
   const int tm = pick_tm(N);
   const size_t bytes = (2 * (size_t)tm * simt::H + (size_t)tm * simt::rup16(2 * S + A) + 4 * tm + 8) * sizeof(float);
-  auto kern = tm == 64 ? trn::classifier_kernel<8> : tm == 32 ? trn::classifier_kernel<4> : trn::classifier_kernel<2>;
+  auto kern = tm == 32 ? trn::classifier_kernel<4> : trn::classifier_kernel<2>;
   if (const char* e = set_smem(kern, bytes)) return e;
   const int ntiles = (N + tm - 1) / tm;
   mb_launch(kern, dim3(ntiles), dim3(simt::NT), bytes, st, c);

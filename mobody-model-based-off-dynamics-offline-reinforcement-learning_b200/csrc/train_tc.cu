@@ -32,19 +32,13 @@ const char* mb_gemm_launch(const ug::Args& a, cudaStream_t st) {
   const int as = a.job[0].a_src, bs = a.job[0].b_src, ec = ug::epi_class(a.job[0].epi);
   const bool narrow = max_n <= 64;
   using namespace ug;
-  if (as == SRC_PACKED) {                                  // forward layers whose input was emitted pre-split by the producing launch
-    if (bs != SRC_PACKED || narrow) return "gemm: a packed A operand needs a packed B operand and a 256-wide tile";
-    if (ec == EPI_STORE) return launch_gemm<256, 2, 2, EPI_STORE>(a, max_m, st);
-  } else if (as == SRC_KCONTIG && bs == SRC_PACKED) {           // forward / backward-data layers on packed weight images
+  if (as == SRC_KCONTIG && bs == SRC_PACKED) {           // forward / backward-data layers on packed weight images
     if (ec == EPI_STORE) return launch_np<0, 2, EPI_STORE>(a, max_m, narrow, st);
-    if (ec == EPI_TANH) return launch_np<0, 2, EPI_TANH>(a, max_m, narrow, st);
     if (ec == EPI_MASK) return launch_np<0, 2, EPI_MASK>(a, max_m, narrow, st);
   } else if (as == SRC_KCONTIG && bs == SRC_KCONTIG) {   // forward layers
     if (ec == EPI_STORE) return launch_np<0, 0, EPI_STORE>(a, max_m, narrow, st);
-    if (ec == EPI_TANH) return launch_np<0, 0, EPI_TANH>(a, max_m, narrow, st);
     if (ec == EPI_DSWISH) return launch_np<0, 0, EPI_DSWISH>(a, max_m, narrow, st);   // ensemble layers backward: W[e][in][out] is K-contiguous in `out`
   } else if (as == SRC_KCONTIG && bs == SRC_RCONTIG) {   // backward-data
-    if (ec == EPI_MASK) return launch_np<0, 1, EPI_MASK>(a, max_m, narrow, st);
     if (ec == EPI_STORE) return launch_np<0, 1, EPI_STORE>(a, max_m, narrow, st);
     if (ec == EPI_SWISH) return launch_np<0, 1, EPI_SWISH>(a, max_m, narrow, st);     // ensemble layers forward
   } else if (as == SRC_RCONTIG && bs == SRC_RCONTIG) {   // weight gradients (and the test hook)

@@ -8,7 +8,7 @@
 // global -> registers (next chunk in flight) -> split -> shared memory in the UMMA K-major no-swizzle layout, and one thread
 // issues the chunk's 12 MMAs asynchronously (tcgen05.commit -> mbarrier frees the stage): the tensor pipe works on chunk c
 // while the CUDA cores split chunk c + 1.  Epilogues read the accumulator with tcgen05.ld and fuse bias / ReLU / ReLU mask /
-// the one-output Q head / tanh.
+// the one-output Q head.
 //
 // Operand sources (element (row, k) of a K-major operand plane; row = m for A, n for B):
 //   SRC_KCONTIG : src[row * ld + k]      (activations, nn.Linear weight used "forward")
@@ -27,17 +27,15 @@ constexpr int KC = 16;           // K per pipeline stage = 2 UMMA K steps of 8 (
 constexpr int NT = 256;          // threads per CTA
 
 enum { SRC_KCONTIG = 0, SRC_RCONTIG = 1,
-       SRC_PACKED = 2 };   // pre-split TF32 hi/lo image in stage layout, streamed by TMA bulk copies: B from pack_b_kernel, A from a
-                           // producing launch's epilogue (Job::apack); a packed A requires a packed B
+       SRC_PACKED = 2 };   // B only: pre-split TF32 hi/lo image in stage layout (pack_b_kernel), streamed by TMA bulk copies
 // Epilogue kinds.  EPI_STORE and EPI_HEAD share one compiled epilogue (a job without w3 has no head), the others are their own
 // instantiations: the epilogue body is unrolled per 32 x 32 block, so every variant compiled into it is paid in issue slots.
 enum { EPI_STORE = 0,   // C = act(acc + bias)                       -> C[m][n]
        EPI_MASK = 1,    // C = mask[m][n] > 0 ? acc : 0              -> C[m][n]          (ReLU backward)
        EPI_HEAD = 2,    // h = relu(acc + bias); out1[m] = h . w3 + b3; optional C = h     (Q network tail)
-       EPI_TANH = 3,    // C = tanh(acc + bias) * scale              -> C[m][n]          (policy tail)
-       EPI_PART = 4,    // C[split][m][n] = acc, db[split][m] = row sums of the A operand (weight gradient partials)
-       EPI_SWISH = 5,   // x = acc + bias -> pre[m][n] (kept for the backward pass); C = x * sigmoid(x)   (ensemble layers, dynfit.cu)
-       EPI_DSWISH = 6 };// C = acc * swish'(mask[m][n]), mask = the layer's stored pre-activation         (Swish backward)
+       EPI_PART = 3,    // C[split][m][n] = acc, db[split][m] = row sums of the A operand (weight gradient partials)
+       EPI_SWISH = 4,   // x = acc + bias -> pre[m][n] (kept for the backward pass); C = x * sigmoid(x)   (ensemble layers, dynfit.cu)
+       EPI_DSWISH = 5 };// C = acc * swish'(mask[m][n]), mask = the layer's stored pre-activation         (Swish backward)
 __host__ __device__ constexpr int epi_class(int epi) { return epi == EPI_HEAD ? EPI_STORE : epi; }
 
 struct Job {
@@ -47,15 +45,12 @@ struct Job {
   int a_src, b_src, epi, relu;
   const float* bias; const float* mask; int ldmask;
   const float* w3; const float* b3;
-  float* C; int ldc; float* out1; float* db; float scale;
+  float* C; int ldc; float* out1; float* db;
   float* pre;                                                           // EPI_SWISH: pre-activation copy, same pitch as C (may be null)
-  float* apack;   // EPI_STORE / EPI_HEAD: also emit the output tile as the NEXT layer's packed A image (TF32 hi / lo planes in stage layout,
-                  // [row tile][chunk][plane][kgroup][row][4 k]); a consumer with a_src = SRC_PACKED streams it by TMA -- no operand conversion
 };
 struct Args { Job job[8]; int njobs, nsplit; };
 
 __host__ __device__ inline int rup16(int x) { return (x + 15) & ~15; }
-__host__ __device__ inline size_t packed_a_tile_floats(int K) { return (size_t)((K + KC - 1) / KC) * 2 * BM * (KC / 4) * 4; }   // one 128-row tile of a packed A image
 __host__ __device__ inline size_t stage_bytes(int np) { return (size_t)2 * (BM + np) * (KC / 4) * 16; }   // hi + lo planes of A and B
 
 __device__ __forceinline__ float swish_f(float x) { return x / (1.f + expf(-x)); }
@@ -180,7 +175,7 @@ __global__ void __launch_bounds__(NT, 2) gemm_kernel(const __grid_constant__ Arg
     tc::mbar_init(&bar_free[0], 1); tc::mbar_init(&bar_free[1], 1); tc::mbar_init(&bar_done, 1);
     tc::mbar_init(&bar_fullb[0], 1); tc::mbar_init(&bar_fullb[1], 1); tc::mbar_fence_init();
   }
-  if (EPI == EPI_STORE || EPI == EPI_TANH || EPI == EPI_SWISH) {
+  if (EPI == EPI_STORE || EPI == EPI_SWISH) {
     bias_s[tid] = (jb.bias && tid < jb.N) ? __ldg(jb.bias + tid) : 0.f;
     w3_s[tid] = (EPI == EPI_STORE && jb.w3 && tid < jb.N) ? __ldg(jb.w3 + tid) : 0.f;
   }
@@ -248,49 +243,12 @@ __global__ void __launch_bounds__(NT, 2) gemm_kernel(const __grid_constant__ Arg
       if (c + 1 == nchunks) tc::umma_commit(&bar_done);
     } else if (B_SRC == SRC_PACKED && tid == 32 && c + 1 < nchunks) tma_b(c + 1);
   };
-  if constexpr (A_SRC == SRC_PACKED) {
-    // Both operands arrive as packed images: ONE thread requests chunk c + 1 (A and B, one barrier) as soon as the MMAs of
-    // chunk c - 1 have left that stage, then issues the MMAs of chunk c.  No operand conversion, no block barrier in the loop.
-    static_assert(B_SRC == SRC_PACKED, "a packed A operand needs a packed B operand");
-    if (tid == 0) {
-      const unsigned char* aimg = reinterpret_cast<const unsigned char*>(jb.A) + (size_t)blockIdx.x * packed_a_tile_floats(jb.K) * 4;
-      auto tma_ab = [&](int c) {
-        const int nb = c & 1;
-        if (c >= 2) tc::mbar_wait(&bar_free[nb], (uint32_t)(((c >> 1) - 1) & 1));
-        tc::mbar_arrive_expect_tx(&bar_fullb[nb], 2 * A_PLANE + 2 * B_PLANE);
-        tc::bulk_g2s(smem + (size_t)nb * STAGE, aimg + (size_t)(kbeg / KC + c) * (2 * A_PLANE), 2 * A_PLANE, &bar_fullb[nb]);
-        tc::bulk_g2s(smem + (size_t)nb * STAGE + 2 * A_PLANE, reinterpret_cast<const unsigned char*>(jb.B) + (size_t)(kbeg / KC + c) * (2 * B_PLANE),
-                     2 * B_PLANE, &bar_fullb[nb]);
-      };
-      if (nchunks > 0) tma_ab(0);
-#pragma unroll 1
-      for (int c = 0; c < nchunks; ++c) {
-        if (c + 1 < nchunks) tma_ab(c + 1);
-        const int buf = c & 1;
-        tc::mbar_wait(&bar_fullb[buf], (uint32_t)((c >> 1) & 1));
-        tc::tc_fence_after();
-        const uint32_t a0 = tc::smem_u32(smem + (size_t)buf * STAGE), b0 = a0 + 2 * A_PLANE;
-#pragma unroll
-        for (int s2 = 0; s2 < KC / 8; ++s2) {
-          const uint32_t ao = a0 + (uint32_t)s2 * 2u * (BM * 16), bo = b0 + (uint32_t)s2 * 2u * (NP * 16);
-          const uint64_t ah = tc::make_smem_desc(ao, BM * 16, 128), al = tc::make_smem_desc(ao + A_PLANE, BM * 16, 128);
-          const uint64_t bh = tc::make_smem_desc(bo, NP * 16, 128), bl = tc::make_smem_desc(bo + B_PLANE, NP * 16, 128);
-          umma_tf32(tmem, al, bh, idesc, (c > 0 || s2 > 0) ? 1u : 0u);
-          umma_tf32(tmem, ah, bl, idesc, 1u);
-          umma_tf32(tmem, ah, bh, idesc, 1u);
-        }
-        tc::umma_commit(&bar_free[buf]);
-        if (c + 1 == nchunks) tc::umma_commit(&bar_done);
-      }
-    }
-  } else {
   if (nchunks > 0) { fetch(oa0, ob0, 0); if (B_SRC == SRC_PACKED && tid == 32) tma_b(0); }
   if (nchunks > 1) fetch(oa1, ob1, 1);
 #pragma unroll 1
   for (int c = 0; c < nchunks; c += 2) {
     step(oa0, ob0, c);
     if (c + 1 < nchunks) step(oa1, ob1, c + 1);
-  }
   }
 #ifdef UG_TRACE
   t_[2] = clock64();
@@ -340,24 +298,13 @@ __global__ void __launch_bounds__(NT, 2) gemm_kernel(const __grid_constant__ Arg
 #pragma unroll
       for (int jj = 0; jj < 32; ++jj) x[jj] = 0u;
     }
-    if (EPI == EPI_STORE && jb.apack) {   // the next layer's packed A image: this lane's row, 8 k-groups of this block (coalesced along rows)
-      unsigned char* img = reinterpret_cast<unsigned char*>(jb.apack) + (size_t)blockIdx.x * packed_a_tile_floats(jb.N) * 4;
-#pragma unroll
-      for (int jj = 0; jj < 32; jj += 4) {
-        const int nn = n0 + jj;
-        float pv[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) { const float t = __uint_as_float(x[jj + i]) + bias_s[nn + i]; pv[i] = jb.relu ? fmaxf(t, 0.f) : t; }
-        put_unit(img + (size_t)(nn / KC) * (2 * A_PLANE), A_PLANE, (uint32_t)((nn % KC) / 4) * (BM * 16) + (uint32_t)(q * 32 + lane) * 16, pv);
-      }
-    }
 #pragma unroll
     for (int jj = 0; jj < 32; jj += 4)
       *reinterpret_cast<uint4*>(tb + lane * 36 + jj) = make_uint4(x[jj], x[jj + 1], x[jj + 2], x[jj + 3]);
     __syncwarp();
     if (fast) {
       float4 bq = make_float4(0.f, 0.f, 0.f, 0.f), wq = bq;
-      if (EPI == EPI_STORE || EPI == EPI_TANH || EPI == EPI_SWISH) { bq = *reinterpret_cast<const float4*>(bias_s + n); wq = *reinterpret_cast<const float4*>(w3_s + n); }
+      if (EPI == EPI_STORE || EPI == EPI_SWISH) { bq = *reinterpret_cast<const float4*>(bias_s + n); wq = *reinterpret_cast<const float4*>(w3_s + n); }
 #pragma unroll
       for (int it = 0; it < 8; ++it) {
         const int rr = it * 4 + rl;
@@ -372,8 +319,7 @@ __global__ void __launch_bounds__(NT, 2) gemm_kernel(const __grid_constant__ Arg
           v.x = swish_f(v.x); v.y = swish_f(v.y); v.z = swish_f(v.z); v.w = swish_f(v.w);
         } else if (EPI != EPI_PART) {
           v.x += bq.x; v.y += bq.y; v.z += bq.z; v.w += bq.w;
-          if (EPI == EPI_TANH) { v.x = tanhf(v.x) * jb.scale; v.y = tanhf(v.y) * jb.scale; v.z = tanhf(v.z) * jb.scale; v.w = tanhf(v.w) * jb.scale; }
-          else if (jb.relu) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
+          if (jb.relu) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
           if (EPI == EPI_STORE) head[it] = fmaf(v.x, wq.x, fmaf(v.y, wq.y, fmaf(v.z, wq.z, fmaf(v.w, wq.w, head[it]))));
         }
         if (cbase && colok && q * 32 + rr < rows) *reinterpret_cast<float4*>(cbase + (size_t)it * 4 * ldc + n) = v;
@@ -392,8 +338,7 @@ __global__ void __launch_bounds__(NT, 2) gemm_kernel(const __grid_constant__ Arg
           t = swish_f(t);
         } else if (EPI != EPI_PART) {
           t += bias_s[nn];
-          if (EPI == EPI_TANH) t = tanhf(t) * jb.scale;
-          else if (jb.relu) t = fmaxf(t, 0.f);
+          if (jb.relu) t = fmaxf(t, 0.f);
         }
         if (jb.C) jb.C[(EPI == EPI_PART ? (size_t)blockIdx.z * jb.M * jb.N : 0) + (size_t)(m0 + r) * ldc + nn] = t;
       }

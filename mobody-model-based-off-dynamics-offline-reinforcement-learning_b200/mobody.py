@@ -188,8 +188,6 @@ class MOBODY(object):
         self.PIPE_FIRST = sm * 128      # first chunk of a pipelined rollout(): one wave of 128-row tiles, so the first kernel starts after a short H2D
         self.PIPE_ROWS = 2 * sm * 128   # later chunks: two full waves
         self._wave = sm * 128
-        import os
-        self.TC_TRAIN_ROWS = int(os.environ.get("MOBODY_TRAIN_TC_ROWS", 1280)) if os.environ.get("MOBODY_TRAIN_TC", "1") != "0" else 1 << 62
 
     # ------------------------------------------------------------------ optimizers (mobody.py:127-135)
     _OPT_COUNTER = {"q": "_t_q", "pi": "_t_pi", "cls": "_t_cls"}
@@ -566,7 +564,7 @@ class MOBODY(object):
         if nsplit is None:
             # row splits of the weight-gradient GEMMs (partials summed in Adam, fixed order); 128 x 64 tiles per split:
             # critic 2 x (256 x 256 -> 8, 256 x (S+A) -> 2 per 64 columns), actor 8 + 2 per 64 columns of S
-            if N >= self.TC_TRAIN_ROWS:   # tcgen05 path: 128 x 256 GEMM tiles, two CTAs per SM; critic launch 4 x 2 + 2 x 1 tiles, actor 2 x 2 + 1
+            if N >= _ffi.TC_TRAIN_MIN_ROWS:   # tcgen05 path: 128 x 256 GEMM tiles, two CTAs per SM; critic launch 4 x 2 + 2 x 1 tiles, actor 2 x 2 + 1
                 nsplit = _wgrad_splits(N, (10, 5), self.device, ctas_per_sm=2, cta_overhead=4.0, per_split=0.36)
             else:
                 nsplit = _wgrad_splits(N, (2 * (8 + 2 * ((S + A + 63) // 64)), 8 + 2 * ((S + 63) // 64)), self.device)

@@ -1,5 +1,5 @@
 # A/B of an environment switch on the train step (run under gpurun):  bash scripts/ab_env.sh MOBODY_PDL 0 1
-#                                                                     bash scripts/ab_env.sh MOBODY_TRAIN_TM 64 32
+#                                                                     bash scripts/ab_env.sh MOBODY_TRAIN_SIDE 0 1
 var=$1; shift
 for v in "$@"; do
   export $var=$v

@@ -1,6 +1,6 @@
 """Build libmobody_b200 with extra -D flags into variants/<name>/ (A/B experiments on the GPU box).
 
-usage: python scripts/build_variant.py NAME -DMOBODY_EPI_SHARE=4 ...   ->  variants/NAME/libmobody_b200.so
+usage: python scripts/build_variant.py NAME -DUG_TRACE ...   ->  variants/NAME/libmobody_b200.so
 Select it at run time with MOBODY_B200_LIB=variants/NAME/libmobody_b200.so.
 """
 import os, subprocess, sys

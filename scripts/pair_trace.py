@@ -1,5 +1,5 @@
-"""Debug aid: per-(layer, tile) timeline (clock64) of CTA 0 of the two-tile step kernels: the CTA-pair kernel
-(MOBODY_TC_PAIR=1, precision bf16x2) or the two-tiles-per-CTA kernel (precision fp16 / bf16)."""
+"""Debug aid: per-(layer, tile) timeline (clock64) of CTA 0 of the two-tiles-per-CTA step kernel (step_duo.cu), which
+runs the fp16 precision mode."""
 import sys, os, ctypes
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -8,7 +8,7 @@ from helpers import cuda_dynamics, cuda_agent
 from mobody_b200 import _ffi
 from mobody_b200.dynamics import StepWorkspace
 
-prec = sys.argv[1] if len(sys.argv) > 1 else "bf16x2"
+prec = sys.argv[1] if len(sys.argv) > 1 else "fp16"
 B = int(sys.argv[2]) if len(sys.argv) > 2 else 256 * 148
 S, A = 17, 6
 dyn, p = cuda_dynamics(S, A, 1, "halfcheetah", 5.0, precision=prec)

@@ -36,6 +36,7 @@ def test_abi_version_and_pure_host_calls(libpath):
     from mobody_b200 import _ffi
     L = _ffi.lib()
     assert L.mobody_abi_version() == 2 == _ffi.ABI_VERSION
+    assert int(re.search(r"#define MOBODY_TC_TRAIN_MIN_ROWS (\d+)", open(HEADER).read()).group(1)) == _ffi.TC_TRAIN_MIN_ROWS
     assert L.mobody_row_width(17, 6) == 44 and L.mobody_row_width(11, 3) == 28 and L.mobody_row_width(27, 8) == 64
     assert L.mobody_compact_scratch_ints(1) == 2 and L.mobody_compact_scratch_ints(1025) == 3
 
