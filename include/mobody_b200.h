@@ -45,6 +45,13 @@ extern "C" {
 #define MOBODY_PREC_BF16X2 1  /* tcgen05 bf16 hi+lo split (3 MMAs), ~1e-5 rel: inside the 1e-4 bound */
 #define MOBODY_PREC_BF16 2    /* tcgen05 single-pass bf16: DIAGNOSTIC ONLY, outside the stated bounds (measured 1.6e-2); the Python mirror does not offer it */
 #define MOBODY_PREC_FP16 3    /* tcgen05 single-pass fp16, two tiles per SM, packed-half epilogue; measured <= 4.6e-3, inside the stated looser bound 5e-3; |activations| < 6e4 */
+/* Shapes of the tensor-core modes: S <= 64, A <= 16, and the [s, a, s'] operand plane of the reward model must fit in
+   shared memory next to the other planes: 2S+A <= 96 (bf16x2: hi and lo planes, one row tile per CTA) or 112 (fp16: two
+   row tiles per CTA).  mobody_step rejects other shapes with MOBODY_ERR_ARG; the fp32 mode takes S <= 128, A <= 32. */
+#define MOBODY_TC_MAX_S 64
+#define MOBODY_TC_MAX_A 16
+#define MOBODY_TC_BF16X2_MAX_SAS 96
+#define MOBODY_TC_FP16_MAX_SAS 112
 
 /* compaction predicates */
 #define MOBODY_KEEP_U8_ZERO 0 /* keep rows with flag == 0      (non-terminal rows, mobody.py:635)   */

@@ -21,6 +21,8 @@ DYN_LAYER_NAMES = ("zs1", "zs2", "zs3", "za_src1", "za_src2", "za_trg1", "za_trg
 # it is a kernel-development diagnostic and is not offered here.
 PREC = {"fp32": 0, "bf16x2": 1, "fp16": 3}
 ENABLED_PRECISIONS = ("fp32", "bf16x2", "fp16")
+# shapes the tensor-core modes take (MOBODY_TC_* in include/mobody_b200.h): S <= 64, A <= 16, 2S+A <= the mode's limit
+TC_MAX_S, TC_MAX_A, TC_MAX_SAS = 64, 16, {"bf16x2": 96, "fp16": 112}
 ABI_VERSION = 2
 TC_TRAIN_MIN_ROWS = 1280   # MOBODY_TC_TRAIN_MIN_ROWS: mobody_train_step runs on tcgen05 GEMM tiles from this many batch rows
 KEEP_U8_ZERO, KEEP_F32_LE, KEEP_F32_LT, KEEP_U8_VALID = 0, 1, 2, 3

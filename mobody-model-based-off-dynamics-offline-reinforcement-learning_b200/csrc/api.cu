@@ -97,6 +97,11 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
   if (!d->idx && (!d->elites || d->n_elites < 1)) return fail(MOBODY_ERR_ARG, "mobody_step: need idx or elites");
   if (d->term_kind < 0 || d->term_kind > MOBODY_TERM_PEN) return fail(MOBODY_ERR_ARG, "mobody_step: bad term_kind");
   if (d->term_kind == MOBODY_TERM_PEN && d->S < 27) return fail(MOBODY_ERR_ARG, "mobody_step: pen termination needs S >= 27");
+  if (d->precision == MOBODY_PREC_BF16X2 || d->precision == MOBODY_PREC_FP16) {
+    const int max_sas = d->precision == MOBODY_PREC_FP16 ? MOBODY_TC_FP16_MAX_SAS : MOBODY_TC_BF16X2_MAX_SAS;
+    if (d->S > MOBODY_TC_MAX_S || d->A > MOBODY_TC_MAX_A || 2 * d->S + d->A > max_sas)
+      return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core modes take S <= 64, A <= 16 and 2S+A <= 96 (bf16x2) / 112 (fp16)");
+  }
   StepArgs a;
   memset(&a, 0, sizeof(a));
   a.obs = d->obs; a.act = d->policy ? nullptr : d->act; a.eps = d->eps; a.idx = d->idx; a.elites = d->elites;

@@ -224,7 +224,9 @@ policy_kernel(const float* __restrict__ obs, int B, int S, int A, MlpPtrs pol, f
 const char* mb_simt_step_launch(const StepArgs& a, const DynPtrs& dp, const MlpPtrs* pol, cudaStream_t st) {
   if (a.B <= 0) return nullptr;
   if (a.S < 2 || a.S > 128 || a.A < 1 || a.A > 32) return "fp32 step kernel supports 2 <= S <= 128, 1 <= A <= 32";
-  const int tm = a.S <= 64 ? 64 : 32;                       // wide observations: 32-row tiles (shared-memory budget)
+  // 64-row tiles, or 32-row tiles where 64 rows of operands exceed the shared-memory budget (observations wider than
+  // about 40 columns: the [s, a, s'] plane of the reward model grows with 2S+A)
+  const int tm = simt::smem_floats(a.S, a.A, 64) * sizeof(float) <= 227 * 1024 ? 64 : 32;
   size_t bytes = simt::smem_floats(a.S, a.A, tm) * sizeof(float);
   if (bytes > 227 * 1024) return "fp32 step kernel: shared memory budget exceeded for this (S, A)";
   auto kern = tm == 64 ? simt::step_kernel<8> : simt::step_kernel<4>;

@@ -60,6 +60,11 @@ class StepWorkspace:
         self.act = torch.empty(B, A, **f) if want_act else None
 
 
+def tc_step_supports(S, A, precision):
+    """Whether the tensor-core step kernels take observation / action widths (S, A) in ``precision`` (mobody_step's check)."""
+    return 2 <= S <= _ffi.TC_MAX_S and 1 <= A <= _ffi.TC_MAX_A and 2 * S + A <= _ffi.TC_MAX_SAS[precision]
+
+
 class MOBODYEnsembleDynamics(DynamicsFitting):
     def __init__(self, config, model, optim=None, scaler=None,
                  terminal_fn: Optional[Callable] = None, penalty_coef: float = 0.0,
@@ -84,7 +89,7 @@ class MOBODYEnsembleDynamics(DynamicsFitting):
         self.precision = precision or (config or {}).get("b200_precision", "auto")
         if self.precision == "auto":
             S_, A_ = getattr(model, "obs_dim", 0), getattr(model, "action_dim", 0)
-            self.precision = "bf16x2" if (2 <= S_ <= 64 and 1 <= A_ <= 16) else "fp32"
+            self.precision = "bf16x2" if tc_step_supports(S_, A_, "bf16x2") else "fp32"
         if self.precision not in _ffi.PREC:
             raise ValueError(f"precision {self.precision!r}: choose one of {_ffi.ENABLED_PRECISIONS} (single-pass bf16 is outside "
                              "the stated error bounds and is not a product mode)")
