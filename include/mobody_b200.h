@@ -240,6 +240,31 @@ int mobody_peer_wait(const mobody_peer_desc* p, void* stream);
 int mobody_rollout_stats_doubles(void);   /* size of mobody_rollout_desc.stats in doubles */
 int mobody_rollout(const mobody_rollout_desc* d, void* stream);
 
+/* ---- policy evaluation in the learned model: the episode return eval_policy reports (train_mobody.py:53-205), with the
+ * dynamics model standing in for the environment, one episode per start state, as ONE host call ----
+ * Step t (t < H) runs the fused step (policy forward + dynamics step) on the live rows with Philox step word
+ * `step.step + t`, each row keyed on its global start id (step.row0 + its index in step.obs), exactly as mobody_rollout
+ * keys them: a start state's episode does not depend on the batch it runs in.  The step reward is the step's `reward`
+ * (raw reward, or reward - coef * penalty with use_penalty).  A row whose next state is terminal keeps that step's reward
+ * and stops; survivors are compacted stably into the next step's input.  Memory is O(B) whatever H: nothing per step is
+ * kept.  Returns accumulate in float64, one add per row and step in step order: ret += r; ret_disc += disc * r (product
+ * rounded, then added), where disc starts at 1.0 and is multiplied by gamma after every step -- reproducible bit for bit
+ * on a host.  Once every row has ended, the remaining steps launch kernels that exit at once.
+ * `step` is the template as in mobody_rollout: obs = dense start states [B,S], policy required, eps / idx must be NULL
+ * (Philox draws only); its per-step fields are overridden from the workspace. */
+typedef struct mobody_model_eval_desc {
+  mobody_step_desc step;
+  int H;                      /* horizon, 1 .. 100000; step.step + H must not exceed 2^32                             */
+  double gamma;
+  void* workspace; long long workspace_bytes;   /* device, >= mobody_model_eval_workspace_bytes(B, S, A) (no H in it) */
+  double* ret;                /* device [B] sum of the step rewards up to and including the terminating step (or H-1) */
+  double* ret_disc;           /* device [B] sum over the same steps of gamma^t r_t                                     */
+  int* length;                /* device [B] steps taken: t+1 for a row whose next state at step t is terminal, else H */
+  int* counts;                /* device [H+1] live rows entering step t; counts[H] = rows still live after the last   */
+} mobody_model_eval_desc;
+long long mobody_model_eval_workspace_bytes(int B, int S, int A);
+int mobody_model_eval(const mobody_model_eval_desc* d, void* stream);
+
 /* ---- steady-state train step: twin-critic TD update + Polyak + Q-weighted BC actor update ----
  * Replaces MOBODY.update_q_functions / update_target / update_policy / bc_loss and the three
  * torch.optim.Adam steps inside MOBODY.train (algo/offline_offline/mobody.py:183-208, 246-276, 314-345,

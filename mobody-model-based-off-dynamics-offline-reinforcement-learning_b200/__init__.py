@@ -7,7 +7,7 @@ Public names mirror the reference modules they replace:
   algo.utils                      -> ReplayBuffer
   algo.offline_offline.mobody     -> MOBODY, Policy, DoubleQFunc, MLPNetwork, ValueFunc
   dataset.call_dataset            -> call_tar_dataset (+ transitions_from_raw, read_raw, load_buffers)
-  train_mobody (evaluators)       -> eval_policy, eval_policy_batch
+  train_mobody (evaluators)       -> eval_policy, eval_policy_batch (+ eval_policy_in_model: no simulator)
 """
 from . import _ffi, parallel                                          # noqa: F401
 from .module import MOBODYModule, EnsembleLinear, Swish, soft_clamp   # noqa: F401
@@ -15,7 +15,7 @@ from .dynamics import MOBODYEnsembleDynamics, StandardScaler          # noqa: F4
 from .terminal_funs import get_termination_fn, TERM_KINDS             # noqa: F401
 from .buffer import ReplayBuffer                                      # noqa: F401
 from .dataset import call_tar_dataset, transitions_from_raw, read_raw, load_buffers   # noqa: F401
-from .evaluate import eval_policy, eval_policy_batch                   # noqa: F401
+from .evaluate import eval_policy, eval_policy_batch, eval_policy_in_model   # noqa: F401
 from .mobody import MOBODY, Policy, DoubleQFunc, MLPNetwork, ValueFunc, Classifier  # noqa: F401
 
 __all__ = ["MOBODYModule", "EnsembleLinear", "Swish", "MOBODYEnsembleDynamics", "StandardScaler",

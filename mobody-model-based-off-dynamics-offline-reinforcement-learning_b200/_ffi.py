@@ -61,6 +61,13 @@ class RolloutDesc(C.Structure):
     ]
 
 
+class ModelEvalDesc(C.Structure):
+    _fields_ = [
+        ("step", StepDesc), ("H", C.c_int), ("gamma", C.c_double), ("workspace", C.c_void_p), ("workspace_bytes", C.c_longlong),
+        ("ret", C.c_void_p), ("ret_disc", C.c_void_p), ("length", C.c_void_p), ("counts", C.c_void_p),
+    ]
+
+
 class PeerDesc(C.Structure):
     _fields_ = [("world", C.c_int), ("rank", C.c_int), ("base", C.c_void_p * 8), ("multicast", C.c_void_p), ("cap_rows", C.c_longlong), ("W", C.c_int),
                 ("epoch", C.c_uint), ("ctas", C.c_int)]
@@ -143,6 +150,9 @@ def lib():
         L.mobody_peer_wait.argtypes = [C.POINTER(PeerDesc), C.c_void_p]
         L.mobody_peer_slot.argtypes = [C.POINTER(PeerDesc), C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]
         L.mobody_rollout.argtypes = [C.POINTER(RolloutDesc), C.c_void_p]
+        L.mobody_model_eval_workspace_bytes.restype = C.c_longlong
+        L.mobody_model_eval_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int]
+        L.mobody_model_eval.argtypes = [C.POINTER(ModelEvalDesc), C.c_void_p]
         L.mobody_policy_forward.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(MlpParams), C.c_float,
                                             C.c_void_p, C.c_void_p]
         L.mobody_termination.argtypes = [C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p, C.c_void_p]

@@ -32,6 +32,10 @@ void mb_rollout_pack_launch(const float* obss, const float* acts, const float* n
                             cudaStream_t st);
 void mb_rollout_stats_launch(const float* rews, const unsigned char* terms, long long n, double* partial, unsigned int* ticket,
                              double* stats, cudaStream_t st);
+void mb_model_eval_init_launch(long long* row_ids, unsigned long long row0, int B, double* ret, double* ret_disc, int* length,
+                               int* counts, cudaStream_t st);
+void mb_model_eval_accumulate_launch(const float* reward, const long long* row_ids, unsigned long long row0, const int* n_dev,
+                                     long long n_cap, int t, double disc, double* ret, double* ret_disc, int* length, cudaStream_t st);
 
 const char* mb_tc_dyn_pack(const DynPtrs& dp, int S, int A, int ns, int fp16, unsigned char* blob, unsigned long long* state, cudaStream_t st);
 const char* mb_tc_mlp_pack(const MlpPtrs& mp, int din, int dout, int ns, int fp16, unsigned char* blob, unsigned long long* state, cudaStream_t st);
@@ -299,6 +303,84 @@ int mobody_rollout(const mobody_rollout_desc* d, void* stream) {
                          d->packed, st);
   mb_rollout_stats_launch(d->rews, d->terms, (long long)T * B, d->stats + 2, d->ticket, d->stats, st);
   return check_launch("mobody_rollout");
+}
+
+// mobody_model_eval workspace: start-state ping-pong [2][B,S] | next_obs [B,S] | act [B,A] | mean [E,B,S] | reward [B] |
+// penalty [B] | row ids [2][B] | compaction positions [B] | compaction scratch | terminal [B]; each region 256-byte aligned.
+struct EvalWs {
+  float *obs[2], *next, *act, *mean, *rew, *pen;
+  long long* ids[2];
+  int *pos, *scratch;
+  unsigned char* term;
+  long long bytes;
+};
+static EvalWs eval_ws_layout(void* base, int B, int S, int A) {
+  EvalWs w;
+  uintptr_t p = (uintptr_t)base;
+  auto take = [&](size_t bytes) { void* r = (void*)p; p += (bytes + 255) & ~(size_t)255; return r; };
+  const size_t b = (size_t)B;
+  for (int k = 0; k < 2; ++k) w.obs[k] = (float*)take(b * S * sizeof(float));
+  w.next = (float*)take(b * S * sizeof(float));
+  w.act = (float*)take(b * A * sizeof(float));
+  w.mean = (float*)take((size_t)MOBODY_E * b * S * sizeof(float));
+  w.rew = (float*)take(b * sizeof(float));
+  w.pen = (float*)take(b * sizeof(float));
+  for (int k = 0; k < 2; ++k) w.ids[k] = (long long*)take(b * sizeof(long long));
+  w.pos = (int*)take(b * sizeof(int));
+  w.scratch = (int*)take((size_t)mobody_compact_scratch_ints(B) * sizeof(int));
+  w.term = (unsigned char*)take(b);
+  w.bytes = (long long)(p - (uintptr_t)base);
+  return w;
+}
+
+long long mobody_model_eval_workspace_bytes(int B, int S, int A) {
+  if (B < 1 || S < 1 || A < 1) return 0;
+  return eval_ws_layout(nullptr, B, S, A).bytes;
+}
+
+int mobody_model_eval(const mobody_model_eval_desc* d, void* stream) {
+  if (!d) return fail(MOBODY_ERR_ARG, "mobody_model_eval: null descriptor");
+  const mobody_step_desc& s0 = d->step;
+  const int B = s0.B, S = s0.S, A = s0.A, H = d->H;
+  if (H < 1 || H > 100000) return fail(MOBODY_ERR_ARG, "mobody_model_eval: bad H (1 <= H <= 100000)");
+  if ((unsigned long long)s0.step + (unsigned long long)H > 0x100000000ULL)
+    return fail(MOBODY_ERR_ARG, "mobody_model_eval: step + H overflows the 32-bit Philox step word");
+  if (B < 0) return fail(MOBODY_ERR_ARG, "mobody_model_eval: bad B");
+  if (s0.eps || s0.idx) return fail(MOBODY_ERR_ARG, "mobody_model_eval: Philox draws only (eps and idx must be NULL)");
+  if (!s0.policy) return fail(MOBODY_ERR_ARG, "mobody_model_eval: the step template needs a policy (actions come from pi(s))");
+  if (s0.obs_ld && s0.obs_ld != S) return fail(MOBODY_ERR_ARG, "mobody_model_eval: start states must be dense [B,S]");
+  if (!d->ret || !d->ret_disc || !d->length || !d->counts) return fail(MOBODY_ERR_ARG, "mobody_model_eval: null output pointer");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (B == 0) {
+    if (cudaMemsetAsync(d->counts, 0, (size_t)(H + 1) * sizeof(int), st) != cudaSuccess)
+      return fail(MOBODY_ERR_CUDA, "mobody_model_eval: clearing counts failed");
+    return MOBODY_OK;
+  }
+  if (!s0.obs) return fail(MOBODY_ERR_ARG, "mobody_model_eval: null start states");
+  const long long need = mobody_model_eval_workspace_bytes(B, S, A);
+  if (need <= 0) return fail(MOBODY_ERR_ARG, "mobody_model_eval: bad S / A");
+  if (!d->workspace || d->workspace_bytes < need)
+    return fail(MOBODY_ERR_ARG, "mobody_model_eval: workspace missing or smaller than mobody_model_eval_workspace_bytes(B, S, A)");
+  const EvalWs w = eval_ws_layout(d->workspace, B, S, A);
+  double disc = 1.0;
+  for (int t = 0; t < H; ++t) {
+    const int cur = t & 1, nxt = cur ^ 1;
+    mobody_step_desc s = s0;
+    // step 0 reads the caller's start states with the default keying row0 + i (what the ids of step 0 hold), so it is
+    // enqueued first: mobody_step validates the template (shapes the precision takes, parameters) before anything runs
+    s.obs = t == 0 ? s0.obs : w.obs[cur]; s.obs_ld = 0; s.act = nullptr; s.act_ld = 0; s.act_out = w.act;
+    s.row_ids = t == 0 ? nullptr : w.ids[cur]; s.n_rows_dev = t == 0 ? nullptr : d->counts + t;
+    s.next_obs = w.next; s.reward = w.rew; s.raw_reward = nullptr; s.penalty = w.pen; s.terminal = w.term; s.mean = w.mean;
+    s.step = s0.step + (unsigned)t;
+    if (int rc = mobody_step(&s, stream)) return rc;
+    if (t == 0) mb_model_eval_init_launch(w.ids[0], s0.row0, B, d->ret, d->ret_disc, d->length, d->counts, st);
+    mb_model_eval_accumulate_launch(w.rew, w.ids[cur], s0.row0, d->counts + t, B, t, disc, d->ret, d->ret_disc, d->length, st);
+    mb_compact_launch(MOBODY_KEEP_U8_ZERO, w.term, nullptr, 0.f, B, d->counts + t, w.scratch, w.pos, d->counts + t + 1, st);
+    if (t + 1 < H)
+      mb_rollout_advance_launch(w.next, w.ids[cur], S, w.pos, d->counts + t + 1, B, w.obs[nxt], w.ids[nxt], st);
+    disc *= d->gamma;
+  }
+  return check_launch("mobody_model_eval");
 }
 
 int mobody_peer_push(const mobody_peer_desc* p, const int* kept_dev, const double* stats_dev, void* stream) {

@@ -357,6 +357,32 @@ __global__ void __launch_bounds__(SB) rollout_stats_kernel(const float* __restri
   }
 }
 
+// ---------------- policy evaluation in the model (mobody_model_eval) ----------------
+// init: zeroed per-start outputs, row ids of step 0, live rows entering step 0
+__global__ void model_eval_init_kernel(long long* __restrict__ row_ids, unsigned long long row0, int B, double* __restrict__ ret,
+                                       double* __restrict__ ret_disc, int* __restrict__ length, int* __restrict__ counts) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < B; i += gridDim.x * blockDim.x) {
+    row_ids[i] = (long long)(row0 + (unsigned long long)i);
+    ret[i] = 0.0; ret_disc[i] = 0.0; length[i] = 0;
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) counts[0] = B;
+}
+
+// live row i < *n_dev of step t: its start row gets the step's reward.  Explicitly rounded product and sum (no FMA
+// contraction): the host reproduces the same float64 sequence bit for bit.
+__global__ void model_eval_accumulate_kernel(const float* __restrict__ reward, const long long* __restrict__ row_ids,
+                                             unsigned long long row0, const int* __restrict__ n_dev, int t, double disc,
+                                             double* __restrict__ ret, double* __restrict__ ret_disc, int* __restrict__ length) {
+  const int n = *n_dev;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const long long id = (long long)((unsigned long long)row_ids[i] - row0);
+    const double r = (double)reward[i];
+    ret[id] = __dadd_rn(ret[id], r);
+    ret_disc[id] = __dadd_rn(ret_disc[id], __dmul_rn(disc, r));
+    length[id] = t + 1;
+  }
+}
+
 // `par` reward penalty (mobody.py:428-434): reward[i] -= coef * mean_j (next_state[i,j] - pred[i,j])^2 on the first n batch
 // rows, in place; mean_out = batch mean of the penalty.  One CTA (n is a batch size): thread t owns rows t, t+1024, ...;
 // the per-thread sums are combined in a fixed tree, so the logged mean is deterministic.
@@ -484,6 +510,16 @@ void mb_rollout_stats_launch(const float* rews, const unsigned char* terms, long
                              double* stats, cudaStream_t st) {
   int nb = (int)((n + 4095) / 4096); if (nb < 1) nb = 1; if (nb > MB_STATS_BLOCKS) nb = MB_STATS_BLOCKS;
   buf::rollout_stats_kernel<<<nb, buf::SB, 0, st>>>(rews, terms, n, partial, ticket, stats);
+}
+
+void mb_model_eval_init_launch(long long* row_ids, unsigned long long row0, int B, double* ret, double* ret_disc, int* length,
+                               int* counts, cudaStream_t st) {
+  buf::model_eval_init_kernel<<<grid_for(B, buf::NT), buf::NT, 0, st>>>(row_ids, row0, B, ret, ret_disc, length, counts);
+}
+void mb_model_eval_accumulate_launch(const float* reward, const long long* row_ids, unsigned long long row0, const int* n_dev,
+                                     long long n_cap, int t, double disc, double* ret, double* ret_disc, int* length, cudaStream_t st) {
+  buf::model_eval_accumulate_kernel<<<grid_for(n_cap, buf::NT), buf::NT, 0, st>>>(reward, row_ids, row0, n_dev, t, disc, ret,
+                                                                                 ret_disc, length);
 }
 
 void mb_sample_rows_launch(const mobody_sample_job* jobs, int njobs, int rw, cudaStream_t st) {

@@ -2,6 +2,7 @@
 environments stepped in lock step) and :142-205 (``eval_policy``).  The environments are the caller's (gym / mujoco are not
 part of this image); the policy forward is the CUDA policy kernel, one launch for the whole vector of states per step, and
 the optional model check (``eval_trg`` with a dynamics object) is one fused dynamics step over every visited transition.
+``eval_policy_in_model`` needs no environment: it scores the policy in the agent's learned target-domain dynamics.
 """
 import numpy as np
 import torch
@@ -68,3 +69,13 @@ def eval_policy(policy, env, policy_distribution, eval_episodes=10, eval_cnt=Non
         _model_check(dynamics, states, actions, next_states, rewards)
     print("[{}] Evaluation on {} over {} episodes: {}".format(eval_cnt, "target" if eval_trg else "source", eval_episodes, avg_reward))
     return avg_reward
+
+
+def eval_policy_in_model(agent, init_states, horizon=1000, penalized=False, eval_cnt=None):
+    """The evaluators' average return with the learned target dynamics standing in for the environment: one episode per start
+    state (``init_states`` [N, S], e.g. target-domain dataset states), at most ``horizon`` steps, the policy acting
+    deterministically (MOBODY.evaluate_in_model).  Prints in the evaluators' format and returns the average return."""
+    res, info = agent.evaluate_in_model(init_states, horizon, penalized=penalized)
+    n = int(res["returns"].shape[0])
+    print("[{}] Evaluation in the learned target model over {} episodes: {}".format(eval_cnt, n, info["return_mean"]))
+    return info["return_mean"]

@@ -181,6 +181,8 @@ class MOBODY(object):
         self._par_mean = torch.zeros(1, dtype=torch.float32, device=self.device)
         self._par_ws = None
         self._roll_ws = {}                                       # (T, B, S, A) -> rollout scratch
+        self._eval_ws = {}                                       # (B, S, A, slot) -> evaluate_in_model scratch
+        self._eval_draw = 0                                      # Philox step counter of evaluate_in_model
         self._host_slabs = []                                    # pinned staging slabs of rollout() results (reused when idle)
         self._pipe_streams, self._pipe_hdr = None, None          # side streams / pinned header of the pipelined rollout()
         self._pipe_plan_cache = None                             # (key, per-chunk launch plan)
@@ -356,6 +358,72 @@ class MOBODY(object):
             out[name] = packed[:M, c0:c0 + w]
             c0 += w
         info["packed"] = packed
+        return out, info
+
+    # ------------------------------------------------------------------ policy evaluation in the learned model
+    @property
+    def eval_seed(self):
+        """Philox key of evaluate_in_model: a stream of its own under the dynamics seed, so evaluations never reuse the
+        training rollouts' draws."""
+        return ReplayBuffer.stream_seed(self.dynamics.seed, "eval")
+
+    def _eval_workspace(self, B, S, A, slot=0):
+        """Device scratch of mobody_model_eval for B start states (its size does not depend on the horizon).  ``slot``
+        separates workspaces of evaluations in flight at the same time on different streams."""
+        key = (B, S, A, slot)
+        ws = self._eval_ws.get(key)
+        if ws is None:
+            ws = torch.empty(int(_ffi.lib().mobody_model_eval_workspace_bytes(B, S, A)), dtype=torch.uint8, device=self.device)
+            if len(self._eval_ws) >= 4:
+                self._eval_ws.pop(next(iter(self._eval_ws)))
+            self._eval_ws[key] = ws
+        return ws
+
+    def _launch_model_eval(self, init_obss, H, gamma, penalized, use_trg, row0, step0, ws_slot=0, verify_images=True):
+        """Enqueue one mobody_model_eval on the current stream; no host synchronisation.  Returns (outputs, counts[H+1])."""
+        dev = self.device
+        B, S = init_obss.shape
+        out = {"returns": torch.empty(B, dtype=torch.float64, device=dev),                  # (the library zeroes them)
+               "discounted_returns": torch.empty(B, dtype=torch.float64, device=dev),
+               "lengths": torch.empty(B, dtype=torch.int32, device=dev)}
+        counts = torch.zeros(H + 1, dtype=torch.int32, device=dev)
+        if B > 0:
+            d = _ffi.ModelEvalDesc()
+            keep = self.dynamics.fill_step_desc(d.step, B, S, dev, policy=self.policy.network, max_action=self.policy.max_action,  # noqa: F841
+                                                use_penalty=penalized, use_trg=use_trg, verify_images=verify_images)
+            ws = self._eval_workspace(B, S, self.config["action_dim"], ws_slot)
+            d.step.obs, d.step.seed, d.step.step, d.step.row0 = _ffi.ptr(init_obss), self.eval_seed, int(step0), int(row0)
+            d.H, d.gamma, d.workspace, d.workspace_bytes = H, float(gamma), _ffi.ptr(ws), ws.numel()
+            d.ret, d.ret_disc = _ffi.ptr(out["returns"]), _ffi.ptr(out["discounted_returns"])
+            d.length, d.counts = _ffi.ptr(out["lengths"]), _ffi.ptr(counts)
+            _ffi.check(_ffi.lib().mobody_model_eval(C.byref(d), _ffi.stream_ptr(dev)))
+        return out, counts
+
+    @torch.no_grad()
+    def evaluate_in_model(self, init_obss, horizon=1000, *, gamma=None, penalized=False, use_trg=True, row0=0, step0=None):
+        """Score the policy without a simulator: one episode per start state in the learned dynamics (the target-domain model
+        with ``use_trg``), driven by the deterministic policy, up to ``horizon`` steps.  An episode's return sums the step
+        rewards up to and including its first terminal step, the quantity eval_policy prints (train_mobody.py:53-205); with
+        ``penalized`` the reward is the rollout's uncertainty-penalized reward.  ONE C-ABI call (mobody_model_eval) runs
+        the whole horizon on the device in memory independent of the horizon.
+
+        Draws: Philox keyed on (eval_seed, step0 + t, row0 + i), so a start state's episode does not depend on how the
+        start states are batched or sharded (give each shard its global ``row0``).  ``step0`` defaults to this object's
+        evaluation counter, advanced by ``horizon`` per call; the training draw counter (dynamics._draw) is never touched,
+        so evaluations interleaved with training change no training result.
+        Returns ({returns, discounted_returns (float64), lengths (int32)}: CUDA tensors [B], info) with info holding
+        ``return_mean``, ``length_mean`` and ``live_per_step`` (live rows entering each step, then the rows still live after
+        the last), read back with one host read."""
+        H = int(horizon)
+        init_obss = _ffi.f32(init_obss, self.device)
+        gamma = self.config["gamma"] if gamma is None else gamma
+        out, counts = self._launch_model_eval(init_obss, H, gamma, penalized, use_trg, row0,
+                                              self._eval_draw if step0 is None else step0)
+        if step0 is None:
+            self._eval_draw += H
+        host = torch.cat([counts.double(), out["returns"].mean()[None], out["lengths"].double().mean()[None]]).cpu()   # the single host read
+        info = {"return_mean": float(host[H + 1]), "length_mean": float(host[H + 2]),
+                "live_per_step": [int(v) for v in host[:H + 1]]}
         return out, info
 
     def _host_slab(self, rows, W):
