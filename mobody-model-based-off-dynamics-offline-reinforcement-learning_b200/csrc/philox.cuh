@@ -2,7 +2,8 @@
 // Replaces torch.normal (mobody_dynamics.py:220), np.random.choice (mobody_module.py:356)
 // and np.random.randint (algo/utils.py:128) with counter-based draws keyed on the
 // *global* row id so results do not depend on how rows are sharded over GPUs.
-// Checked bit-for-bit against oracle/philox.py.
+// Checked bit-for-bit against oracle/philox.py.  Only the low 32 bits of a seed key the generator ((uint32_t)seed):
+// seeds that differ by a multiple of 2^32 give the same draws (pinned by tests/test_gpu_philox_draws.py).
 #pragma once
 #include <stdint.h>
 
@@ -40,12 +41,17 @@ __device__ __forceinline__ void philox_normal4(const Philox4& b, float out[4]) {
   sincosf(t1, &s, &c); out[2] = r1 * c; out[3] = r1 * s;
 }
 
-// one N(0,1): word w (0..3) of the block, same values as philox_normal4()[w]
+// one N(0,1): word w (0..3) of the block, philox_normal4()[w] up to the error of the SFU sine / cosine.
+// The radius takes the precise logf: lg2.approx.f32 has an ABSOLUTE error of about 2^-22 (PTX ISA), the size of ln u
+// itself at the top word (x >> 9 = 2^23 - 1, u = 1 - 2^-24, ln u = -6e-8), where __logf gave r = 0 or NaN instead of
+// 3.45e-4.  With logf (1 ulp) and a correctly rounded sqrtf, r is within 2^-23 r; sin/cos.approx.f32 are within 2^-20.5
+// absolute on t in (0, 2 pi) (PTX ISA); the product adds 2^-24 |n|.  So for every word
+//   |n - r cos t| <= 2^-20.5 r + 2^-22 |n|,   r = sqrt(-2 ln u) <= 5.77,
+// and the tests hold the sample to 2e-6 (1 + |n| + r) of the numpy oracle's, which covers the oracle's own few ulps.
 __device__ __forceinline__ float philox_normal1(const Philox4& b, int w) {
   const float two_pi = 6.283185307179586f;
   const uint32_t xa = (w & 2) ? b.z : b.x, xb = (w & 2) ? b.w : b.y;
-  // SFU forms (lg2/sin/cos.approx): |error| ~1e-6 on the sample, far below the noise it models
-  const float r = sqrtf(-2.0f * __logf(philox_u01(xa))), t = two_pi * philox_u01(xb);
+  const float r = sqrtf(-2.0f * logf(philox_u01(xa))), t = two_pi * philox_u01(xb);
   return (w & 1) ? r * __sinf(t) : r * __cosf(t);
 }
 

@@ -9,6 +9,10 @@ algorithm) keyed on (seed, stream) with the counter holding (global_row, step,
 block) so results do not depend on how rows are sharded.  This file restates
 that published algorithm so the CUDA generator can be checked bit-for-bit.
 
+Only the low 32 bits of a seed key the generator (``seed & 0xFFFFFFFF`` here,
+``(uint32_t)seed`` on the device): seeds that differ by a multiple of 2^32 give
+the same draws.
+
 It also defines ``recipe_fill``: a torch-RNG-independent way to fill weight
 tensors, so golden fixtures can name a recipe instead of storing megabytes.
 """
@@ -91,6 +95,22 @@ def rollout_noise(seed, step, rows, S):
     return n[:, :S].copy()
 
 
+def rollout_radius(seed, step, rows, S):
+    """r[len(rows), S]: the Box-Muller radius sqrt(-2 ln u) of the pair each entry of rollout_noise() belongs to
+    (|noise| <= r; errors of a device sine / cosine scale with r, not with the sample)."""
+    rows = np.asarray(rows, dtype=np.uint64)
+    nb = (S + 3) // 4
+    ctr = np.zeros((len(rows), nb, 4), dtype=np.uint32)
+    ctr[..., 0] = (rows & np.uint64(0xFFFFFFFF)).astype(np.uint32)[:, None]
+    ctr[..., 1] = (rows >> np.uint64(32)).astype(np.uint32)[:, None]
+    ctr[..., 2] = np.uint32(step)
+    ctr[..., 3] = np.arange(nb, dtype=np.uint32)[None, :]
+    key = np.array([seed & 0xFFFFFFFF, STREAM_NOISE], dtype=np.uint32)
+    u = philox_uniform(philox4x32_10(ctr, key)).astype(np.float64)
+    r = np.sqrt(-2.0 * np.log(u[..., [0, 0, 2, 2]]))
+    return r.reshape(len(rows), nb * 4)[:, :S].copy()
+
+
 def rollout_elite_slot(seed, step, rows, n_elites):
     """slot[len(rows)] in [0, n_elites): mulhi(x0, n_elites) (unbiased enough, no modulo)."""
     rows = np.asarray(rows, dtype=np.uint64)
@@ -119,6 +139,39 @@ def buffer_indices(seed, draw, n, size):
     # the 32-bit form: (x0 * size) >> 32, identical to the device code.
     assert size < (1 << 32)
     return ((out[:, 0].astype(np.uint64) * np.uint64(size)) >> np.uint64(32)).astype(np.int64)
+
+
+# ---- noise of the update kernels (mirrors csrc/train.cu and csrc/dynfit.cu) ----
+STREAM_CLSN = 0x636C736E  # 'clsn'
+STREAM_FIT = 0x66697473   # 'fits'
+
+
+def classifier_noise(seed, draw, N, K, k):
+    """randn_like of the classifier inputs: fp32[N, K] for batch rows 0..N-1 of classifier k (0: sas with K = 2S+A,
+    1: sa with K = S+A).  Element (i, j) is word j & 3 of the Box-Muller block of counter (i, k << 16 | j >> 2, draw, 0),
+    key (seed, STREAM_CLSN): the two classifiers never share a counter."""
+    nb = (K + 3) // 4
+    ctr = np.zeros((N, nb, 4), dtype=np.uint32)
+    ctr[..., 0] = np.arange(N, dtype=np.uint32)[:, None]
+    ctr[..., 1] = (np.uint32(k) << np.uint32(16)) | np.arange(nb, dtype=np.uint32)[None, :]
+    ctr[..., 2] = np.uint32(draw)
+    key = np.array([seed & 0xFFFFFFFF, STREAM_CLSN], dtype=np.uint32)
+    return philox_normal_pairs(philox4x32_10(ctr, key)).reshape(N, nb * 4)[:, :K].copy()
+
+
+def fit_noise(seed, draw, stream, n):
+    """fp32[n]: element i of the dynamics-fit noise stream (1: the six reparameterised latents, flattened [6,7,B,16];
+    2: the next-state noise, flattened [7,B,S]).  Element i is word i & 3 of the Box-Muller block of counter
+    (i >> 2 low, i >> 2 high, draw, stream), key (seed, STREAM_FIT)."""
+    nb = (n + 3) // 4
+    blk = np.arange(nb, dtype=np.uint64)
+    ctr = np.zeros((nb, 4), dtype=np.uint32)
+    ctr[:, 0] = (blk & np.uint64(0xFFFFFFFF)).astype(np.uint32)
+    ctr[:, 1] = (blk >> np.uint64(32)).astype(np.uint32)
+    ctr[:, 2] = np.uint32(draw)
+    ctr[:, 3] = np.uint32(stream)
+    key = np.array([seed & 0xFFFFFFFF, STREAM_FIT], dtype=np.uint32)
+    return philox_normal_pairs(philox4x32_10(ctr, key)).reshape(-1)[:n].copy()
 
 
 def recipe_fill(shape, seed, scale):

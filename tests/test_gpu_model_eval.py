@@ -38,8 +38,13 @@ def _term_distance(env, x):
 @pytest.mark.parametrize("prec", ["fp32", "bf16x2"])
 @pytest.mark.parametrize("env,S,A,h0,t3,kind,penalized", CASES, ids=[c[0] for c in CASES])
 def test_returns_match_float64_oracle(env, S, A, h0, t3, kind, penalized, prec):
+    check_against_float64_oracle(env, S, A, h0, t3, kind, penalized, prec, row0=1000, step0=7)
+
+
+def check_against_float64_oracle(env, S, A, h0, t3, kind, penalized, prec, row0, step0, H=24):
+    """Per-start returns, discounted returns and lengths of evaluate_in_model against the float64 reference."""
     ag, p, st = _agent(env, S, A, prec, h0, t3)
-    B, H, row0, step0, gamma = 300, 24, 1000, 7, 0.99                       # 300 rows: the last 128-row tile is ragged
+    B, gamma = 300, 0.99                                                     # 300 rows: the last 128-row tile is ragged
     obs = _starts(env, S, B, h0)
     res, info = ag.evaluate_in_model(torch.from_numpy(obs).cuda(), H, gamma=gamma, penalized=penalized, row0=row0, step0=step0)
     p64 = {k: (v.double() if v.is_floating_point() else v) for k, v in p.items()}
@@ -61,7 +66,7 @@ def test_returns_match_float64_oracle(env, S, A, h0, t3, kind, penalized, prec):
         worst = max(worst, err / 1e-4)
     if kind == 2:
         assert 0 < ref["counts"][H] < B and len(set(ref["lengths"].tolist())) > 5
-    print(f"\n[model eval parity] {env} {prec}: worst err/bound {worst:.3f}, {int(near.sum())}/{B} rows within {MARGIN} of a "
+    print(f"\n[model eval parity] {env} {prec} row0={row0} step0={step0}: worst err/bound {worst:.3f}, {int(near.sum())}/{B} rows within {MARGIN} of a "
           f"termination threshold excluded, lengths {ref['lengths'].min()}..{ref['lengths'].max()}")
 
 
