@@ -45,6 +45,8 @@ extern "C" {
 #define MOBODY_PREC_BF16X2 1  /* tcgen05 bf16 hi+lo split (3 MMAs), ~1e-5 rel: inside the 1e-4 bound */
 #define MOBODY_PREC_BF16 2    /* tcgen05 single-pass bf16: DIAGNOSTIC ONLY, outside the stated bounds (measured 1.6e-2); the Python mirror does not offer it */
 #define MOBODY_PREC_FP16 3    /* tcgen05 single-pass fp16, two tiles per SM, packed-half epilogue; measured <= 4.6e-3, inside the stated looser bound 5e-3; |activations| < 6e4 */
+#define MOBODY_PREC_BF16X2_WIDE 4  /* bf16x2's arithmetic on 64-row tiles for wide observations: MOBODY_TC_WIDE_MIN_S <= S <= MOBODY_TC_WIDE_MAX_S,
+                                      A <= MOBODY_TC_WIDE_MAX_A (Ant's 111 / 8); packed images are bf16x2's */
 /* Shapes of the tensor-core modes: S <= 64, A <= 16, and the [s, a, s'] operand plane of the reward model must fit in
    shared memory next to the other planes: 2S+A <= 96 (bf16x2: hi and lo planes, one row tile per CTA) or 112 (fp16: two
    row tiles per CTA).  mobody_step rejects other shapes with MOBODY_ERR_ARG; the fp32 mode takes S <= 128, A <= 32. */
@@ -52,6 +54,10 @@ extern "C" {
 #define MOBODY_TC_MAX_A 16
 #define MOBODY_TC_BF16X2_MAX_SAS 96
 #define MOBODY_TC_FP16_MAX_SAS 112
+/* Shapes of MOBODY_PREC_BF16X2_WIDE: every shape the fp32 mode takes above MOBODY_TC_MAX_S. */
+#define MOBODY_TC_WIDE_MIN_S 65
+#define MOBODY_TC_WIDE_MAX_S 128
+#define MOBODY_TC_WIDE_MAX_A 32
 
 /* compaction predicates */
 #define MOBODY_KEEP_U8_ZERO 0 /* keep rows with flag == 0      (non-terminal rows, mobody.py:635)   */
@@ -348,7 +354,7 @@ typedef struct mobody_dynfit_desc {
 long long mobody_dynfit_workspace_bytes(int B, int S, int A, int nsplit);
 int mobody_dynfit_step(const mobody_dynfit_desc* d, void* stream);
 
-/* ---- tensor-core weight images (precision MOBODY_PREC_BF16X2 / MOBODY_PREC_FP16) ----
+/* ---- tensor-core weight images (precision MOBODY_PREC_BF16X2 or MOBODY_PREC_BF16X2_WIDE: one format; MOBODY_PREC_FP16) ----
  * The reference keeps weights as fp32 nn.Parameters (mobody_module.py:371-391, mobody.py:35-48); the
  * tcgen05 path consumes them as 16-bit planes in the UMMA shared-memory layout (one launch per image).
  * `state`: NULL -> pack unconditionally.  Otherwise device uint64[4], zero-initialised ONCE by the caller and then

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmobody_b200.so")
-SOURCES = ["api.cu", "step_simt.cu", "buffer.cu", "peer.cu", "tc_selftest.cu", "step_tc.cu", "step_duo.cu", "train.cu", "train_tc.cu", "dynfit.cu"]
+SOURCES = ["api.cu", "step_simt.cu", "buffer.cu", "peer.cu", "tc_selftest.cu", "step_tc.cu", "step_duo.cu", "step_wide.cu", "train.cu", "train_tc.cu", "dynfit.cu"]
 NVCC_FLAGS = (["-DUG_TRACE"] if os.environ.get("UG_TRACE") else []) + ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

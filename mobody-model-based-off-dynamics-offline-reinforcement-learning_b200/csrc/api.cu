@@ -40,6 +40,7 @@ void mb_model_eval_accumulate_launch(const float* reward, const long long* row_i
 const char* mb_tc_dyn_pack(const DynPtrs& dp, int S, int A, int ns, int fp16, unsigned char* blob, unsigned long long* state, cudaStream_t st);
 const char* mb_tc_mlp_pack(const MlpPtrs& mp, int din, int dout, int ns, int fp16, unsigned char* blob, unsigned long long* state, cudaStream_t st);
 const char* mb_tc_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, int ns, cudaStream_t st);
+const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, cudaStream_t st);
 const char* mb_tc_duo_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, int fp16, cudaStream_t st, bool* launched);
 const char* mb_umma_selftest_launch(const float* A, const float* B, int K, int N, int nsplit, float* D, cudaStream_t st);
 void mb_ring_insert_transitions_launch(const float* packed, long long n_cap, const int* n_dev, int S, int A, int rw, long long ptr, long long cap,
@@ -106,6 +107,9 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
     if (d->S > MOBODY_TC_MAX_S || d->A > MOBODY_TC_MAX_A || 2 * d->S + d->A > max_sas)
       return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core modes take S <= 64, A <= 16 and 2S+A <= 96 (bf16x2) / 112 (fp16)");
   }
+  if (d->precision == MOBODY_PREC_BF16X2_WIDE &&
+      (d->S < MOBODY_TC_WIDE_MIN_S || d->S > MOBODY_TC_WIDE_MAX_S || d->A > MOBODY_TC_WIDE_MAX_A))
+    return fail(MOBODY_ERR_ARG, "mobody_step: bf16x2_wide takes 65 <= S <= 128 and A <= 32");
   StepArgs a;
   memset(&a, 0, sizeof(a));
   a.obs = d->obs; a.act = d->policy ? nullptr : d->act; a.eps = d->eps; a.idx = d->idx; a.elites = d->elites;
@@ -147,6 +151,12 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
         err = mb_tc_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr,
                                 d->precision == MOBODY_PREC_BF16X2 ? 2 : 1, (cudaStream_t)stream);
       }
+      break;
+    case MOBODY_PREC_BF16X2_WIDE:
+      if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
+      if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
+      err = mb_tc_wide_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr,
+                                   (cudaStream_t)stream);
       break;
     default: return fail(MOBODY_ERR_UNSUPPORTED, "mobody_step: unknown precision mode");
   }
@@ -475,7 +485,7 @@ int mobody_dara_relabel(float* rows, long long n, int S, int A, int row_width, c
   return check_launch("mobody_dara_relabel");
 }
 
-static int nsplit_of(int precision) { return precision == MOBODY_PREC_BF16X2 ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16) ? 1 : 0; }
+static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16) ? 1 : 0; }
 
 long long mobody_dyn_pack_bytes(int S, int A, int precision) {
   int ns = nsplit_of(precision);

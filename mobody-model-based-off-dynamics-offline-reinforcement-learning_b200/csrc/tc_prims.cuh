@@ -118,6 +118,15 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
       : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
       : "r"(taddr) : "memory");
 }
+// M = 64 accumulators (cta_group::1) hold row i in TMEM lane 32 * (i / 16) + i % 16: a warp's quadrant carries 16 rows.
+// 16x32bx2: threads 0-15 read lanes 0-15 of the quadrant at column taddr, threads 16-31 the same lanes at taddr + 8;
+// each thread gets 8 consecutive columns of its row.
+__device__ __forceinline__ void tmem_ld16x2_8(uint32_t taddr, uint32_t (&r)[8]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.16x32bx2.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8], 8;"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+      : "r"(taddr) : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // ---------------- CTA pair (cta_group::2) variants ----------------

@@ -62,6 +62,8 @@ class StepWorkspace:
 
 def tc_step_supports(S, A, precision):
     """Whether the tensor-core step kernels take observation / action widths (S, A) in ``precision`` (mobody_step's check)."""
+    if precision == "bf16x2_wide":
+        return _ffi.TC_WIDE_MIN_S <= S <= _ffi.TC_WIDE_MAX_S and 1 <= A <= _ffi.TC_WIDE_MAX_A
     return 2 <= S <= _ffi.TC_MAX_S and 1 <= A <= _ffi.TC_MAX_A and 2 * S + A <= _ffi.TC_MAX_SAS[precision]
 
 
@@ -85,13 +87,13 @@ class MOBODYEnsembleDynamics(DynamicsFitting):
         self.cycle_loss_coef = config.get("cycle_loss_coef", 0) if config else 0
         self.encode_trg_diff = getattr(model, "encode_trg_diff", 0)
         # 'auto' (default): the tcgen05 kernel in its fp32-parity mode (bf16 hi+lo split, inside the 1e-4 bound) whenever
-        # it supports the shapes, else the fp32 CUDA-core kernel (any S <= 128)
+        # it supports the shapes, else the fp32 CUDA-core kernel (any S <= 128).  "bf16x2_wide" (S > 64) is opt-in.
         self.precision = precision or (config or {}).get("b200_precision", "auto")
         if self.precision == "auto":
             S_, A_ = getattr(model, "obs_dim", 0), getattr(model, "action_dim", 0)
             self.precision = "bf16x2" if tc_step_supports(S_, A_, "bf16x2") else "fp32"
         if self.precision not in _ffi.PREC:
-            raise ValueError(f"precision {self.precision!r}: choose one of {_ffi.ENABLED_PRECISIONS} (single-pass bf16 is outside "
+            raise ValueError(f"precision {self.precision!r}: choose one of {tuple(_ffi.PREC)} (single-pass bf16 is outside "
                              "the stated error bounds and is not a product mode)")
         self.seed = int(seed)
         self._draw = 0        # Philox step counter for stand-alone step() calls in production mode
