@@ -47,6 +47,8 @@ extern "C" {
 #define MOBODY_PREC_FP16 3    /* tcgen05 single-pass fp16, two tiles per SM, packed-half epilogue; measured <= 4.6e-3, inside the stated looser bound 5e-3; |activations| < 6e4 */
 #define MOBODY_PREC_BF16X2_WIDE 4  /* bf16x2's arithmetic on 64-row tiles for wide observations: MOBODY_TC_WIDE_MIN_S <= S <= MOBODY_TC_WIDE_MAX_S,
                                       A <= MOBODY_TC_WIDE_MAX_A (Ant's 111 / 8); packed images are bf16x2's */
+#define MOBODY_PREC_BF16X2_T64 5   /* bf16x2's arithmetic on the same 64-row tiles for the S <= 64 shapes bf16x2 refuses
+                                      (Adroit's pen 45 / 24, door 39 / 28, relocate 39 / 30, hammer 46 / 26); packed images are bf16x2's */
 /* Shapes of the tensor-core modes: S <= 64, A <= 16, and the [s, a, s'] operand plane of the reward model must fit in
    shared memory next to the other planes: 2S+A <= 96 (bf16x2: hi and lo planes, one row tile per CTA) or 112 (fp16: two
    row tiles per CTA).  mobody_step rejects other shapes with MOBODY_ERR_ARG; the fp32 mode takes S <= 128, A <= 32. */
@@ -58,6 +60,11 @@ extern "C" {
 #define MOBODY_TC_WIDE_MIN_S 65
 #define MOBODY_TC_WIDE_MAX_S 128
 #define MOBODY_TC_WIDE_MAX_A 32
+/* Shapes of MOBODY_PREC_BF16X2_T64: 2 <= S <= MOBODY_TC_T64_MAX_S, 1 <= A <= MOBODY_TC_T64_MAX_A, and A > MOBODY_TC_MAX_A or
+   2S+A > MOBODY_TC_BF16X2_MAX_SAS -- exactly the shapes with S <= 64 that the fp32 mode takes and bf16x2 refuses.  So bf16x2,
+   bf16x2_t64 and bf16x2_wide split the fp32 mode's shapes with no overlap: at most one of them takes a given (S, A). */
+#define MOBODY_TC_T64_MAX_S 64
+#define MOBODY_TC_T64_MAX_A 32
 
 /* compaction predicates */
 #define MOBODY_KEEP_U8_ZERO 0 /* keep rows with flag == 0      (non-terminal rows, mobody.py:635)   */
@@ -354,7 +361,7 @@ typedef struct mobody_dynfit_desc {
 long long mobody_dynfit_workspace_bytes(int B, int S, int A, int nsplit);
 int mobody_dynfit_step(const mobody_dynfit_desc* d, void* stream);
 
-/* ---- tensor-core weight images (precision MOBODY_PREC_BF16X2 or MOBODY_PREC_BF16X2_WIDE: one format; MOBODY_PREC_FP16) ----
+/* ---- tensor-core weight images (precision MOBODY_PREC_BF16X2, MOBODY_PREC_BF16X2_WIDE or MOBODY_PREC_BF16X2_T64: one format; MOBODY_PREC_FP16) ----
  * The reference keeps weights as fp32 nn.Parameters (mobody_module.py:371-391, mobody.py:35-48); the
  * tcgen05 path consumes them as 16-bit planes in the UMMA shared-memory layout (one launch per image).
  * `state`: NULL -> pack unconditionally.  Otherwise device uint64[4], zero-initialised ONCE by the caller and then

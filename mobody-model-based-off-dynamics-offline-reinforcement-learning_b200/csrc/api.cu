@@ -110,6 +110,10 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
   if (d->precision == MOBODY_PREC_BF16X2_WIDE &&
       (d->S < MOBODY_TC_WIDE_MIN_S || d->S > MOBODY_TC_WIDE_MAX_S || d->A > MOBODY_TC_WIDE_MAX_A))
     return fail(MOBODY_ERR_ARG, "mobody_step: bf16x2_wide takes 65 <= S <= 128 and A <= 32");
+  if (d->precision == MOBODY_PREC_BF16X2_T64 &&
+      (d->S > MOBODY_TC_T64_MAX_S || d->A > MOBODY_TC_T64_MAX_A ||
+       (d->A <= MOBODY_TC_MAX_A && 2 * d->S + d->A <= MOBODY_TC_BF16X2_MAX_SAS)))
+    return fail(MOBODY_ERR_ARG, "mobody_step: bf16x2_t64 takes S <= 64, A <= 32 with A > 16 or 2S+A > 96");
   StepArgs a;
   memset(&a, 0, sizeof(a));
   a.obs = d->obs; a.act = d->policy ? nullptr : d->act; a.eps = d->eps; a.idx = d->idx; a.elites = d->elites;
@@ -153,6 +157,7 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
       }
       break;
     case MOBODY_PREC_BF16X2_WIDE:
+    case MOBODY_PREC_BF16X2_T64:
       if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
       if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
       err = mb_tc_wide_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr,
@@ -485,7 +490,7 @@ int mobody_dara_relabel(float* rows, long long n, int S, int A, int row_width, c
   return check_launch("mobody_dara_relabel");
 }
 
-static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16) ? 1 : 0; }
+static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE || precision == MOBODY_PREC_BF16X2_T64) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16) ? 1 : 0; }
 
 long long mobody_dyn_pack_bytes(int S, int A, int precision) {
   int ns = nsplit_of(precision);

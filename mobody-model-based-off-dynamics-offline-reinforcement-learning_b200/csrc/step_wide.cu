@@ -1,4 +1,6 @@
-// Fused one-step model rollout on the tensor cores for wide observations (65 <= S <= 128, 1 <= A <= 32), sm_100a.
+// Fused one-step model rollout on the tensor cores on 64-row tiles (2 <= S <= 128, 1 <= A <= 32), sm_100a.  It serves two
+// modes that differ only in the shapes mobody_step lets through: bf16x2_wide (65 <= S <= 128) and bf16x2_t64 (S <= 64
+// with A > 16 or 2S+A > 96: the shapes the 128-row kernel cannot hold, such as Adroit's pen at 45 / 24).
 //
 // Sibling of step_tc.cu with the same arithmetic (bf16 hi+lo split of both operands, 3 MMAs per K step, inside the 1e-4
 // bound; swish layers pre-scaled by the packer) and the same packed weight images (mobody_dyn_pack / mobody_mlp_pack with
@@ -485,7 +487,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
 const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, cudaStream_t st) {
   if (a.B <= 0) return nullptr;
   const int S = a.S, A = a.A;
-  if (S < 65 || S > 128 || A < 1 || A > 32) return "wide tensor-core step kernel supports 65 <= S <= 128, 1 <= A <= 32";
+  if (S < 2 || S > 128 || A < 1 || A > 32) return "wide tensor-core step kernel supports 2 <= S <= 128, 1 <= A <= 32";
   if (!dynb) return "tensor-core step needs dyn_pack (mobody_dyn_pack)";
   const bool has_policy = polb != nullptr;
   if (has_policy && !a.act_out) return "tensor-core step with a fused policy needs act_out";
