@@ -301,6 +301,24 @@ typedef struct mobody_train_desc {
 long long mobody_train_workspace_bytes(int N, int S, int A, int nsplit);
 int mobody_train_step(const mobody_train_desc* d, void* stream);
 
+/* ---- the same train step with the reference's update-branch flags (mobody.py:210-310, 533-573) ----
+ * advantage=1: first a value step -- adv = min(Q'1(s,a), Q'2(s,a)) - V(s) with the target critics before this step's
+ *   Polyak update, v_loss = mean(|0.7 - 1[adv<0]| adv^2), Adam on `value` (lr = critic_lr, moments value_m / value_v);
+ *   then the TD target r + nd * gamma * V(s') with the updated V, and BC weights exp(3 (min Q(s_t,a_t) - V(s_t))).
+ * scale_q=0: p_w = 1 instead of weight / mean|q(s,pi(s))| (update_policy_1).   q_weighted=0: BC weights 1 (plain BC).
+ * Flags 0/0/1/1 (advantage, scale_q, q_weighted = 0, 1, 1) are mobody_train_step, bit for bit.  The workspace must hold
+ * mobody_train_ex_workspace_bytes(...).  scalars_out keeps slots [0..10]; with advantage=1 it adds [11] v_loss
+ * [12] mean adv of the value step [13] mean V(s) before the step, and with any non-default flag [14] mean min Q(s,a)
+ * after the critic step (all rows).  Other slots are not written. */
+typedef struct mobody_train_ex_desc {
+  mobody_train_desc base;
+  int advantage, scale_q, q_weighted;          /* config flags, 0/1 */
+  mobody_mlp_state value, value_m, value_v;    /* ValueFunc + Adam moments; required iff advantage */
+  int t_v;                                     /* value optimiser step count AFTER this step (1-based) when advantage */
+} mobody_train_ex_desc;
+long long mobody_train_ex_workspace_bytes(int N, int S, int A, int nsplit);
+int mobody_train_step_ex(const mobody_train_ex_desc* d, void* stream);
+
 /* ---- DARA domain classifier (SURVEY.md section 8f rank 1) ----
  * mobody_classifier_step replaces the forward / double-softmax cross-entropy / backward / Adam of
  * MOBODY.update_classifier (algo/offline_offline/mobody.py:146-181) for Classifier (:11-33): `rows` [N,row_width]

@@ -101,6 +101,13 @@ class TrainDesc(C.Structure):
     ]
 
 
+class TrainExDesc(C.Structure):
+    _fields_ = [
+        ("base", TrainDesc), ("advantage", C.c_int), ("scale_q", C.c_int), ("q_weighted", C.c_int),
+        ("value", MlpState), ("value_m", MlpState), ("value_v", MlpState), ("t_v", C.c_int),
+    ]
+
+
 class ClassifierDesc(C.Structure):
     _fields_ = [
         ("rows", C.c_void_p), ("N", C.c_int), ("S", C.c_int), ("A", C.c_int), ("row_width", C.c_int),
@@ -186,6 +193,9 @@ def lib():
         L.mobody_train_workspace_bytes.restype = C.c_longlong
         L.mobody_train_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int]
         L.mobody_train_step.argtypes = [C.POINTER(TrainDesc), C.c_void_p]
+        L.mobody_train_ex_workspace_bytes.restype = C.c_longlong
+        L.mobody_train_ex_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int]
+        L.mobody_train_step_ex.argtypes = [C.POINTER(TrainExDesc), C.c_void_p]
         L.mobody_classifier_workspace_bytes.restype = C.c_longlong
         L.mobody_classifier_workspace_bytes.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int]
         L.mobody_classifier_step.argtypes = [C.POINTER(ClassifierDesc), C.c_void_p]

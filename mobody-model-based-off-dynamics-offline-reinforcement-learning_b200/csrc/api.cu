@@ -58,7 +58,8 @@ const char* mb_gemm_selftest_launch(const float* A, const float* B, int M, int N
                                     float* C, cudaStream_t st);
 void mb_tc_set_trace(long long* buf);
 long long mb_train_workspace_bytes(int N, int S, int A, int nsplit);
-const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st);
+long long mb_train_ex_workspace_bytes(int N, int S, int A, int nsplit);
+const char* mb_train_step_launch(const mobody_train_ex_desc& d, cudaStream_t st);
 
 long long mb_classifier_workspace_bytes(int N, int S, int A, int nsplit);
 const char* mb_classifier_step_launch(const mobody_classifier_desc& d, cudaStream_t st);
@@ -429,18 +430,53 @@ long long mobody_train_workspace_bytes(int N, int S, int A, int nsplit) {
   return mb_train_workspace_bytes(N, S, A, nsplit);
 }
 
-int mobody_train_step(const mobody_train_desc* d, void* stream) {
-  if (!d || !d->rows) return fail(MOBODY_ERR_ARG, "mobody_train_step: null descriptor / rows");
-  if (d->row_width != mobody_row_width(d->S, d->A)) return fail(MOBODY_ERR_ARG, "mobody_train_step: row_width does not match (S, A)");
+static int fail_in(const char* fn, const char* msg) {
+  snprintf(g_err, sizeof(g_err), "%s: %s", fn, msg);
+  return MOBODY_ERR_ARG;
+}
+static bool mlp_state_null(const mobody_mlp_state& s) {
+  for (int j = 0; j < 3; ++j)
+    if (!s.w[j] || !s.b[j]) return true;
+  return false;
+}
+
+// shared by mobody_train_step (default flags) and mobody_train_step_ex; `fn` names the entry point in messages
+static int train_step(const mobody_train_ex_desc& x, void* stream, const char* fn) {
+  const mobody_train_desc* d = &x.base;
+  if (!d->rows) return fail_in(fn, "null descriptor / rows");
+  if (d->row_width != mobody_row_width(d->S, d->A)) return fail_in(fn, "row_width does not match (S, A)");
   const mobody_mlp_state* all[11] = {&d->policy, &d->q1, &d->q2, &d->q1_target, &d->q2_target, &d->policy_m, &d->policy_v,
                                      &d->q1_m, &d->q1_v, &d->q2_m, &d->q2_v};
   for (int i = 0; i < 11; ++i)
-    for (int j = 0; j < 3; ++j)
-      if (!all[i]->w[j] || !all[i]->b[j]) return fail(MOBODY_ERR_ARG, "mobody_train_step: null parameter / moment pointer");
-  if (d->t_q < 1 || d->t_pi < 1) return fail(MOBODY_ERR_ARG, "mobody_train_step: optimiser step counts are 1-based");
-  const char* err = mb_train_step_launch(*d, (cudaStream_t)stream);
+    if (mlp_state_null(*all[i])) return fail_in(fn, "null parameter / moment pointer");
+  if (d->t_q < 1 || d->t_pi < 1) return fail_in(fn, "optimiser step counts are 1-based");
+  const char* err = mb_train_step_launch(x, (cudaStream_t)stream);
   if (err) return fail(MOBODY_ERR_UNSUPPORTED, err);
-  return check_launch("mobody_train_step");
+  return check_launch(fn);
+}
+
+int mobody_train_step(const mobody_train_desc* d, void* stream) {
+  if (!d) return fail(MOBODY_ERR_ARG, "mobody_train_step: null descriptor / rows");
+  mobody_train_ex_desc x{};
+  x.base = *d; x.advantage = 0; x.scale_q = 1; x.q_weighted = 1;
+  return train_step(x, stream, "mobody_train_step");
+}
+
+long long mobody_train_ex_workspace_bytes(int N, int S, int A, int nsplit) {
+  if (N < 1 || S < 1 || A < 1 || nsplit < 1) return 0;
+  return mb_train_ex_workspace_bytes(N, S, A, nsplit);
+}
+
+int mobody_train_step_ex(const mobody_train_ex_desc* d, void* stream) {
+  if (!d) return fail(MOBODY_ERR_ARG, "mobody_train_step_ex: null descriptor / rows");
+  for (int f : {d->advantage, d->scale_q, d->q_weighted})
+    if (f != 0 && f != 1) return fail(MOBODY_ERR_ARG, "mobody_train_step_ex: advantage / scale_q / q_weighted must be 0 or 1");
+  if (d->advantage) {
+    if (mlp_state_null(d->value) || mlp_state_null(d->value_m) || mlp_state_null(d->value_v))
+      return fail(MOBODY_ERR_ARG, "mobody_train_step_ex: advantage=1 needs the value function and its Adam moments");
+    if (d->t_v < 1) return fail(MOBODY_ERR_ARG, "mobody_train_step_ex: the value optimiser step count is 1-based");
+  }
+  return train_step(*d, stream, "mobody_train_step_ex");
 }
 
 long long mobody_dynfit_workspace_bytes(int B, int S, int A, int nsplit) {

@@ -7,6 +7,10 @@
 //   update_policy + bc_loss + pi backward     :314-345, 246-276, 571-573
 //   torch.optim.Adam (lr, betas .9/.999, eps 1e-8) :127-131
 // Math: SURVEY.md Appendix A.3.  All networks are MLPNetwork (Linear-ReLU-Linear-ReLU-Linear, :35-48).
+// The reference's other update branches select phases and loss terms of the same chain (mobody_train_step_ex):
+//   advantage=1: the value step first (update_v_function, :210-242: expectile loss on min Q'(s, a) - V(s), Adam on
+//                ValueFunc), TD target r + nd gamma V(s') with the updated V, BC weights exp(3 (min Q(s_t, a_t) - V(s_t)))
+//   scale_Q=0:   p_w = 1 (update_policy_1, :278-310)         q_weighted=0: BC weights 1 (:262-263)
 //
 // A CTA owns a tile of 64 rows; hidden activations stay in shared memory for the whole
 // forward + backward-data chain of that tile (simt_layers.cuh).  Only what the weight-gradient
@@ -37,6 +41,9 @@ struct CriticArgs {
   float* part;         // [n_tiles][4]: sum (q1-y)^2, sum (q2-y)^2, sum q1, sum q2
   float* Hp[2];        // relu activations of pi(s), [N][256]      (phase 1 role 3: the actor's forward does not depend on
   float* api;          // pi(s), [N][A]                             the critic update, so it rides along with it)
+  // advantage=1 only (vn == nullptr otherwise): the UPDATED value function replaces pi(s') and the target critics --
+  // phase 1 role 0 = V(s') (the TD target), role 4 = V(s_t) on the n_true true rows (the actor's advantage weights)
+  MlpPtrs v; float* vn; float* vh; int n_true;
 };
 
 struct ActorArgs {
@@ -53,6 +60,9 @@ struct ActorArgs {
   float weight;
   float* out;          // scalars [16]
   int* counter;        // zeroed by the critic's Adam launch of the same update
+  // update branches: scale_q = 0 -> p_w = 1; branch = 1 (any non-default flag) -> q_hat on all n_qh = N rows and out[14];
+  // part_v (advantage=1): the value step's tile partials [ntiles_c][4] -> out[11..13]
+  int scale_q, branch, n_qh; const float* part_v;
 };
 
 template <int TMv>
@@ -107,15 +117,21 @@ __global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) critic_fwd_kernel(Critic
   const int S = a.S, A = a.A, ldi = rup16(S + A);
   float* X0 = sm; float* X1 = X0 + TM * H; float* in_s = X1 + TM * H; float* qa = in_s + TM * ldi;
   const int tid = threadIdx.x, row0 = blockIdx.x * TM, rows = min(TM, a.N - row0), role = blockIdx.y;
+  if (role == 4 && row0 >= a.n_true) return;
   for (int i = tid; i < TM * ldi; i += NT) {
     const int r = i / ldi, j = i - r * ldi;
     const float* x = a.X + (size_t)(row0 + r) * a.rw;
-    in_s[i] = role == 0 ? ((r < rows && j < S) ? x[S + A + j] : 0.f)        // [s', 0]
-            : role == 3 ? ((r < rows && j < S) ? x[j] : 0.f)                 // [s, 0]
-                        : ((r < rows && j < S + A) ? x[j] : 0.f);            // [s, a, 0]
+    in_s[i] = role == 0 ? ((r < rows && j < S) ? x[S + A + j] : 0.f)                  // [s', 0]
+            : (role == 3 || role == 4) ? ((r < rows && j < S) ? x[j] : 0.f)            // [s, 0]
+                                       : ((r < rows && j < S + A) ? x[j] : 0.f);       // [s, a, 0]
   }
   __syncthreads();
-  if (role == 3) {
+  if (a.vn && (role == 0 || role == 4)) {                     // V(s') / V(s_t) through the updated value function
+    big_layer_mma<true, RPT>(in_s, ldi, S, a.v.w[0], a.v.b[0], X0, ACT_RELU);
+    big_layer_mma<true, RPT, true>(X0, H, H, a.v.w[1], a.v.b[1], X1, ACT_RELU);
+    q_head<TM>(X1, a.v.w[2], a.v.b[2], qa);
+    if (tid < rows && (role == 0 || row0 + tid < a.n_true)) (role == 0 ? a.vn : a.vh)[row0 + tid] = qa[tid];
+  } else if (role == 3) {
     big_layer_mma<true, RPT>(in_s, ldi, S, a.pi.w[0], a.pi.b[0], X0, ACT_RELU);
     store_tile<TM>(X0, a.Hp[0], row0, rows);
     big_layer_mma<true, RPT, true>(X0, H, H, a.pi.w[1], a.pi.b[1], X1, ACT_RELU);
@@ -179,7 +195,8 @@ __global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) critic_bwd_kernel(Critic
     float d = 0.f, q = 0.f;
     if (tid < rows) {
       const float* x = a.X + (size_t)(row0 + tid) * a.rw;
-      const float y = x[2 * S + A] + x[2 * S + A + 1] * a.gamma * fminf(a.qtk[0][row0 + tid], a.qtk[1][row0 + tid]);
+      const float boot = a.vn ? a.vn[row0 + tid] : fminf(a.qtk[0][row0 + tid], a.qtk[1][row0 + tid]);
+      const float y = x[2 * S + A] + x[2 * S + A + 1] * a.gamma * boot;
       q = a.qk[k][row0 + tid];
       d = q - y;
       a.d3[k][row0 + tid] = 2.0f * d / (float)a.N;
@@ -255,7 +272,19 @@ __device__ void actor_reduce(const ActorArgs& a, float* sh) {
   l = block_sum(l, sh); q1s = block_sum(q1s, sh);
   if (threadIdx.x == 0) {
     a.out[0] = l / (float)a.N; a.out[1] = q1s / (float)a.N;                 // mse(q1,y) + mse(q2,y) (:207)
-    a.out[4] = mean_q; a.out[5] = mean_abs; a.out[9] = a.weight / mean_abs; a.out[10] = mean_h;
+    a.out[4] = mean_q; a.out[5] = mean_abs; a.out[9] = a.scale_q ? a.weight / mean_abs : 1.0f; a.out[10] = mean_h;
+  }
+  if (a.branch) {                                                           // train/q_behavior: mean min Q(s, a), all rows
+    float s_b = 0.f;
+    for (int i = threadIdx.x; i < a.N; i += blockDim.x) s_b += fminf(__ldcg(a.qh[0] + i), __ldcg(a.qh[1] + i));
+    s_b = block_sum(s_b, sh);
+    if (threadIdx.x == 0) a.out[14] = s_b / (float)a.N;
+  }
+  if (a.part_v) {                                                           // value step: v_loss, mean adv, mean V(s)
+    float lv = 0.f, sa = 0.f, sv = 0.f;
+    for (int t = threadIdx.x; t < a.ntiles_c; t += blockDim.x) { lv += a.part_v[t * 4]; sa += a.part_v[t * 4 + 1]; sv += a.part_v[t * 4 + 2]; }
+    lv = block_sum(lv, sh); sa = block_sum(sa, sh); sv = block_sum(sv, sh);
+    if (threadIdx.x == 0) { a.out[11] = lv / (float)a.N; a.out[12] = sa / (float)a.N; a.out[13] = sv / (float)a.N; }
   }
 }
 __device__ void actor_finish(const ActorArgs& a, float* sh) {
@@ -281,7 +310,7 @@ __global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) actor_q_kernel(ActorArgs
   float* qa = sap_s + TM * ldi; float* ones = qa + TM; float* gk = ones + TM;      // gk [TM][A]
   const int tid = threadIdx.x, row0 = blockIdx.x * TM, rows = min(TM, a.N - row0), k = blockIdx.y & 1;
   const bool qhat = blockIdx.y >= 2;
-  if (qhat && row0 >= a.n_true) { actor_finish(a, sm); return; }
+  if (qhat && row0 >= a.n_qh) { actor_finish(a, sm); return; }
   for (int i = tid; i < TM * ldi; i += NT) {
     const int r = i / ldi, j = i - r * ldi;
     float v = 0.f;
@@ -297,7 +326,7 @@ __global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) actor_q_kernel(ActorArgs
     big_layer_mma<true, RPT>(sap_s, ldi, S + A, a.q[k].w[0], a.q[k].b[0], X0, ACT_RELU);
     big_layer_mma<true, RPT, true>(X0, H, H, a.q[k].w[1], a.q[k].b[1], X1, ACT_RELU);
     q_head<TM>(X1, a.q[k].w[2], a.q[k].b[2], qa);
-    if (tid < rows && row0 + tid < a.n_true) a.qh[k][row0 + tid] = qa[tid];
+    if (tid < rows && row0 + tid < a.n_qh) a.qh[k][row0 + tid] = qa[tid];
     actor_finish(a, sm);
     return;
   }
@@ -326,7 +355,15 @@ struct PolicyBwdArgs {
   float* part;         // [ntiles][4]: sum w, min w, max w, sum w * |pi(s) - a|^2
   float* out;          // scalars [16]; [9] = p_w and [10] = mean|q_hat| were written by actor_q_kernel
   int* counter;
+  const float* vh;     // advantage=1: V(s_t) of the updated value function, [n_true]; nullptr: q_hat / mean|q_hat|
+  int q_weighted;      // 0: plain BC (weights 1)
 };
+// exp-advantage weight of true row r (:252-263)
+__device__ __forceinline__ float bc_weight(const PolicyBwdArgs& a, int r, float mean_h) {
+  if (!a.q_weighted) return 1.0f;
+  const float qb = fminf(a.qh[0][r], a.qh[1][r]);
+  return fminf(expf(3.0f * (a.vh ? qb - a.vh[r] : qb / mean_h)), 100.0f);
+}
 template <int RPT>
 __global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) policy_bwd_kernel(PolicyBwdArgs a) {
   mb_pdl_begin();
@@ -344,7 +381,7 @@ __global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) policy_bwd_kernel(Policy
     const int r = row0 + tid;
     float w = 0.f;
     if (tid < rows && r < a.n_true) {
-      w = fminf(expf(3.0f * (fminf(a.qh[0][r], a.qh[1][r]) / mean_h)), 100.0f);           // :252-258
+      w = bc_weight(a, r, mean_h);                                                         // :252-263
       const float* x = a.X + (size_t)r * a.rw + a.S;
       float e = 0.f;
       for (int j = 0; j < a.A; ++j) { const float d = a.api[(size_t)r * a.A + j] - x[j]; e += d * d; }
@@ -790,7 +827,8 @@ __global__ void __launch_bounds__(NT, 1) dara_relabel_kernel(RelabelArgs a) {
 // Element-wise glue between the GEMMs (everything else of the math lives in GEMM epilogues).
 
 // TD target, MSE gradient and the logging partials (mobody.py:189-207): one thread per row, 256-row blocks
-struct TdArgs { const float* X; int N, S, A, rw; float gamma; const float* qk[2]; const float* qtk[2]; float* d3[2]; float* part; };
+struct TdArgs { const float* X; int N, S, A, rw; float gamma; const float* qk[2]; const float* qtk[2]; float* d3[2]; float* part;
+                const float* vn; };   // vn: V(s') (advantage=1) replaces min Q'(s', pi(s'))
 __global__ void __launch_bounds__(256) td_kernel(const TdArgs a) {
   mb_pdl_begin();
   __shared__ float sh[40];
@@ -798,7 +836,8 @@ __global__ void __launch_bounds__(256) td_kernel(const TdArgs a) {
   float e0 = 0.f, e1 = 0.f, s0 = 0.f, s1 = 0.f;
   if (r < a.N) {
     const float* x = a.X + (size_t)r * a.rw;
-    const float y = x[2 * a.S + a.A] + x[2 * a.S + a.A + 1] * a.gamma * fminf(a.qtk[0][r], a.qtk[1][r]);
+    const float boot = a.vn ? a.vn[r] : fminf(a.qtk[0][r], a.qtk[1][r]);
+    const float y = x[2 * a.S + a.A] + x[2 * a.S + a.A + 1] * a.gamma * boot;
     const float q0 = a.qk[0][r], q1 = a.qk[1][r], d0 = q0 - y, d1 = q1 - y;
     a.d3[0][r] = 2.0f * d0 / (float)a.N; a.d3[1][r] = 2.0f * d1 / (float)a.N;
     e0 = d0 * d0; e1 = d1 * d1; s0 = q0; s1 = q1;
@@ -881,7 +920,7 @@ __global__ void __launch_bounds__(128) policy_grad_kernel(const PolicyBwdArgs a)
   float w = 0.f, w_s = 0.f, w_mn = 3.4e38f, w_mx = -3.4e38f, w_e = 0.f;
   if (r < a.N) {
     if (r < a.n_true) {
-      w = fminf(expf(3.0f * (fminf(a.qh[0][r], a.qh[1][r]) / mean_h)), 100.0f);                 // :252-258
+      w = bc_weight(a, r, mean_h);                                                               // :252-263
       const float* x = a.X + (size_t)r * a.rw + a.S;
       float e = 0.f;
       for (int j = 0; j < a.A; ++j) { const float d = a.api[(size_t)r * a.A + j] - x[j]; e += d * d; }
@@ -920,6 +959,101 @@ __global__ void __launch_bounds__(128) policy_grad_kernel(const PolicyBwdArgs a)
   }
 }
 
+// ================= value step (advantage=1, mobody.py:210-242), first in the update =================
+// adv = min(Q'1(s, a), Q'2(s, a)) - V(s) with the target critics before this update's Polyak step, all N rows;
+// v_loss = mean(|0.7 - 1[adv < 0]| adv^2) (asymmetric_l2_loss, :85-86).  d v_loss / d V(s) of a row; loss / adv / V partials.
+__device__ __forceinline__ float expectile_grad(float qt0, float qt1, float v, int N, float& loss, float& adv) {
+  adv = fminf(qt0, qt1) - v;
+  const float wt = fabsf(0.7f - (adv < 0.f ? 1.0f : 0.0f));
+  loss = wt * adv * adv;
+  return -2.0f * wt * adv / (float)N;
+}
+struct ValueArgs {
+  const float* X; int N, S, A, rw;
+  MlpPtrs v, qt[2];
+  float* qts[2];       // Q'_k(s, a), [N]
+  float* vs;           // V(s), [N]
+  float* Hv[2];        // relu activations of V(s), [N][256]
+  float* Dv[2];        // dLoss/d(pre-activation), [N][256]
+  float* d3;           // dLoss/dV(s), [N]
+  float* part;         // [n_tiles][4]: sum loss, sum adv, sum V(s), 0
+};
+
+// roles 0, 1 = Q'_k(s, a) (no grad), role 2 = V(s) with stored activations
+template <int RPT>
+__global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) value_fwd_kernel(ValueArgs a) {
+  mb_pdl_begin();
+  constexpr int TM = 8 * RPT;
+  extern __shared__ __align__(16) float sm[];
+  const int S = a.S, A = a.A, ldi = rup16(S + A);
+  float* X0 = sm; float* X1 = X0 + TM * H; float* in_s = X1 + TM * H; float* qa = in_s + TM * ldi;
+  const int tid = threadIdx.x, row0 = blockIdx.x * TM, rows = min(TM, a.N - row0), role = blockIdx.y;
+  const int K = role == 2 ? S : S + A;
+  for (int i = tid; i < TM * ldi; i += NT) {
+    const int r = i / ldi, j = i - r * ldi;
+    in_s[i] = (r < rows && j < K) ? a.X[(size_t)(row0 + r) * a.rw + j] : 0.f;       // [s, 0] or [s, a, 0]
+  }
+  __syncthreads();
+  if (role == 2) {
+    big_layer_mma<true, RPT>(in_s, ldi, S, a.v.w[0], a.v.b[0], X0, ACT_RELU);
+    store_tile<TM>(X0, a.Hv[0], row0, rows);
+    big_layer_mma<true, RPT, true>(X0, H, H, a.v.w[1], a.v.b[1], X1, ACT_RELU);
+    store_tile<TM>(X1, a.Hv[1], row0, rows);
+    q_head<TM>(X1, a.v.w[2], a.v.b[2], qa);
+    if (tid < rows) a.vs[row0 + tid] = qa[tid];
+  } else {
+    big_layer_mma<true, RPT>(in_s, ldi, S + A, a.qt[role].w[0], a.qt[role].b[0], X0, ACT_RELU);
+    big_layer_mma<true, RPT, true>(X0, H, H, a.qt[role].w[1], a.qt[role].b[1], X1, ACT_RELU);
+    q_head<TM>(X1, a.qt[role].w[2], a.qt[role].b[2], qa);
+    if (tid < rows) a.qts[role][row0 + tid] = qa[tid];
+  }
+}
+
+// expectile gradient and V's backward to the pre-activations
+template <int RPT>
+__global__ void __launch_bounds__(NT, RPT == 4 ? 2 : 1) value_bwd_kernel(ValueArgs a) {
+  mb_pdl_begin();
+  constexpr int TM = 8 * RPT;
+  extern __shared__ __align__(16) float sm[];
+  __shared__ float red[40];
+  float* X0 = sm; float* X1 = X0 + TM * H; float* g3 = X1 + TM * H;
+  const int tid = threadIdx.x, row0 = blockIdx.x * TM, rows = min(TM, a.N - row0);
+  load_tile<TM>(X0, a.Hv[0], row0, rows);
+  load_tile<TM>(X1, a.Hv[1], row0, rows);
+  float l = 0.f, ad = 0.f, vv = 0.f;
+  if (tid < TM) {
+    float g = 0.f;
+    if (tid < rows) {
+      const int r = row0 + tid;
+      vv = a.vs[r];
+      g = expectile_grad(a.qts[0][r], a.qts[1][r], vv, a.N, l, ad);
+      a.d3[r] = g;
+    }
+    g3[tid] = g;
+  }
+  __syncthreads();
+  head_backward<TM>(X1, a.v.w[2], g3);
+  store_tile<TM>(X1, a.Dv[1], row0, rows);
+  big_layer_mma<false, RPT, true>(X1, H, H, a.v.w[1], nullptr, X0, ACT_MASK);
+  store_tile<TM>(X0, a.Dv[0], row0, rows);
+  l = block_sum(l, red); ad = block_sum(ad, red); vv = block_sum(vv, red);
+  if (tid == 0) { float* p = a.part + (size_t)blockIdx.x * 4; p[0] = l; p[1] = ad; p[2] = vv; p[3] = 0.f; }
+}
+
+// large-batch path: the same row math between the GEMMs, 256-row blocks (one partial per block)
+__global__ void __launch_bounds__(256) value_loss_kernel(const ValueArgs a) {
+  mb_pdl_begin();
+  __shared__ float sh[40];
+  const int r = blockIdx.x * 256 + threadIdx.x;
+  float l = 0.f, ad = 0.f, vv = 0.f;
+  if (r < a.N) {
+    vv = a.vs[r];
+    a.d3[r] = expectile_grad(a.qts[0][r], a.qts[1][r], vv, a.N, l, ad);
+  }
+  l = block_sum(l, sh); ad = block_sum(ad, sh); vv = block_sum(vv, sh);
+  if (threadIdx.x == 0) { float* p = a.part + (size_t)blockIdx.x * 4; p[0] = l; p[1] = ad; p[2] = vv; p[3] = 0.f; }
+}
+
 }  // namespace trn
 
 // ---------------- host launchers ----------------
@@ -946,9 +1080,21 @@ const char* mb_train_critic_launch(const trn::CriticArgs& a, cudaStream_t st) {
   if (const char* e = set_smem(k1, bytes)) return e;
   if (const char* e = set_smem(k2, bytes)) return e;
   if (const char* e = set_smem(k3, bytes)) return e;
-  mb_launch(k1, dim3(ntiles, 4), dim3(simt::NT), bytes, st, a);
-  mb_launch(k2, dim3(ntiles, 2), dim3(simt::NT), bytes, st, a);
+  mb_launch(k1, dim3(ntiles, a.vn ? 5 : 4), dim3(simt::NT), bytes, st, a);
+  if (!a.vn) mb_launch(k2, dim3(ntiles, 2), dim3(simt::NT), bytes, st, a);     // advantage=1: the TD target is V(s')
   mb_launch(k3, dim3(ntiles, 2), dim3(simt::NT), bytes, st, a);
+  return nullptr;
+}
+const char* mb_train_value_launch(const trn::ValueArgs& a, cudaStream_t st) {
+  constexpr int tm = TRAIN_TM;
+  const int ntiles = (a.N + tm - 1) / tm;
+  const size_t bytes = (2 * (size_t)tm * simt::H + (size_t)tm * simt::rup16(a.S + a.A) + 2 * tm + 8) * sizeof(float);
+  auto k1 = trn::value_fwd_kernel<tm / 8>;
+  auto k2 = trn::value_bwd_kernel<tm / 8>;
+  if (const char* e = set_smem(k1, bytes)) return e;
+  if (const char* e = set_smem(k2, bytes)) return e;
+  mb_launch(k1, dim3(ntiles, 3), dim3(simt::NT), bytes, st, a);
+  mb_launch(k2, dim3(ntiles), dim3(simt::NT), bytes, st, a);
   return nullptr;
 }
 const char* mb_train_actor_launch(const trn::ActorArgs& a, cudaStream_t st) {
@@ -992,6 +1138,10 @@ const char* mb_train_adam_launch(const trn::AdamArgs& a, cudaStream_t st) {
 // ---------------- whole train step (C ABI: mobody_train_step) ----------------
 struct TrainWs {   // float offsets into the workspace
   size_t Hq[2][2], Dq[2][2], d3[2], part, Hp[2], Dp[2], api, a2, qk[2], qtk[2], qv[2], qh[2], gak[2], d3p, scal, part2, cnt, gq[2][6], gp[6], T[2], img[17], total;
+  // advantage=1, past `total` (mobody_train_ex_workspace_bytes): V(s), V(s'), V(s_t), dLoss/dV, value partials, V's
+  // weight-gradient partials and weight images.  V's activations use Hp / Dp, which the value step finishes with before
+  // the critic phase writes pi(s) there.
+  size_t vs, vn, vh, d3v, partv, gv[6], img_v[3], total_ex;
   int ntiles;
 };
 static TrainWs train_ws(int N, int S, int A, int nsplit) {
@@ -1017,11 +1167,49 @@ static TrainWs train_ws(int N, int S, int A, int nsplit) {
     for (int i = 0; i < 17; ++i) w.img[i] = take(ug::packed_floats(ik[i], inp[i]));
   }
   w.total = o;
+  w.vs = take(N); w.vn = take(N); w.vh = take(N); w.d3v = take(N); w.partv = take((size_t)w.ntiles * 4);
+  const size_t vn6[6] = {(size_t)256 * S, 256, 256 * 256, 256, 256, 1};
+  for (int t = 0; t < 6; ++t) w.gv[t] = take(vn6[t] * nsplit);
+  w.img_v[0] = take(ug::packed_floats(S, 256)); w.img_v[1] = take(ug::packed_floats(256, 256)); w.img_v[2] = take(ug::packed_floats(256, 256));
+  w.total_ex = o;
   return w;
 }
 long long mb_train_workspace_bytes(int N, int S, int A, int nsplit) { return (long long)train_ws(N, S, A, nsplit).total * 4; }
+long long mb_train_ex_workspace_bytes(int N, int S, int A, int nsplit) { return (long long)train_ws(N, S, A, nsplit).total_ex * 4; }
 
 static MlpPtrs as_ptrs(const mobody_mlp_state& s) { MlpPtrs p; for (int i = 0; i < 3; ++i) { p.w[i] = s.w[i]; p.b[i] = s.b[i]; } return p; }
+
+// Adam on ValueFunc (lr = critic_lr, :132) from the row-split partials of its weight gradients
+static const char* value_adam(const mobody_train_ex_desc& x, const TrainWs& w, float* ws, cudaStream_t st) {
+  const int S = x.base.S;
+  trn::AdamArgs av{}; av.nsplit = x.base.nsplit; av.b1 = 0.9f; av.b2 = 0.999f; av.eps = 1e-8f; av.tau = 0.f; av.njobs = 6;
+  const double bc1 = 1.0 - pow(0.9, (double)x.t_v), bc2 = 1.0 - pow(0.999, (double)x.t_v);
+  av.lr_over_bc1 = (float)(x.base.critic_lr / bc1); av.inv_sqrt_bc2 = (float)(1.0 / sqrt(bc2));
+  const int vn6[6] = {256 * S, 256, 256 * 256, 256, 256, 1};
+  for (int t = 0; t < 6; ++t) {
+    const int li = t >> 1; const bool isw = (t & 1) == 0;
+    av.job[t] = {isw ? x.value.w[li] : x.value.b[li], ws + w.gv[t], isw ? x.value_m.w[li] : x.value_m.b[li],
+                 isw ? x.value_v.w[li] : x.value_v.b[li], nullptr, vn6[t]};
+  }
+  return mb_train_adam_launch(av, st);
+}
+static trn::ValueArgs value_args(const mobody_train_ex_desc& x, const TrainWs& w, float* ws) {
+  const mobody_train_desc& d = x.base;
+  trn::ValueArgs v{};
+  v.X = d.rows; v.N = d.N; v.S = d.S; v.A = d.A; v.rw = d.row_width;
+  v.v = as_ptrs(x.value); v.qt[0] = as_ptrs(d.q1_target); v.qt[1] = as_ptrs(d.q2_target);
+  v.qts[0] = ws + w.qtk[0]; v.qts[1] = ws + w.qtk[1]; v.vs = ws + w.vs;     // (qtk is free: the TD target is V(s'))
+  for (int l = 0; l < 2; ++l) { v.Hv[l] = ws + w.Hp[l]; v.Dv[l] = ws + w.Dp[l]; }
+  v.d3 = ws + w.d3v; v.part = ws + w.partv;
+  return v;
+}
+// scalars_out: slots [0..10] always, [11..13] with the value step, [14] (q_behavior) with any non-default flag
+static void copy_scalars(const mobody_train_ex_desc& x, const float* scal, cudaStream_t st) {
+  float* out = x.base.scalars_out;
+  if (!out) return;
+  cudaMemcpyAsync(out, scal, (x.advantage ? 15 : 11) * sizeof(float), cudaMemcpyDeviceToDevice, st);
+  if (!x.advantage && (!x.scale_q || !x.q_weighted)) cudaMemcpyAsync(out + 14, scal + 14, sizeof(float), cudaMemcpyDeviceToDevice, st);
+}
 
 // ---------------- large-batch update on tcgen05 (rows >= MOBODY_TC_TRAIN_MIN_ROWS: the GEMMs are throughput bound) ----------------
 const char* mb_gemm_launch(const ug::Args& a, cudaStream_t st);     // train_tc.cu
@@ -1053,12 +1241,14 @@ const char* mb_pack_b_launch(const ug::PackArgs& a, cudaStream_t st);     // tra
 static ug::PackJob pack_job(const float* src, int ld, int mode, int N, int K, int NP, float* dst) {
   return ug::PackJob{src, ld, mode, N, K, NP, reinterpret_cast<uint32_t*>(dst)};
 }
-template <typename... J> static const char* run_gemms(cudaStream_t st, int nsplit, J... jobs) {
-  ug::Args a{}; a.nsplit = nsplit;
-  const ug::Job list[] = {jobs...};
-  a.njobs = (int)sizeof...(jobs);
-  for (int i = 0; i < a.njobs; ++i) a.job[i] = list[i];
+static const char* run_gemm_list(cudaStream_t st, int nsplit, const ug::Job* list, int n) {
+  ug::Args a{}; a.nsplit = nsplit; a.njobs = n;
+  for (int i = 0; i < n; ++i) a.job[i] = list[i];
   return mb_gemm_launch(a, st);
+}
+template <typename... J> static const char* run_gemms(cudaStream_t st, int nsplit, J... jobs) {
+  const ug::Job list[] = {jobs...};
+  return run_gemm_list(st, nsplit, list, (int)sizeof...(jobs));
 }
 
 // Launches of the large-batch update that do not depend on each other run on a side stream (fork by event, join by event):
@@ -1082,7 +1272,9 @@ static TrainSide& train_side() {
   return ss;
 }
 
-static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const TrainWs& w, cudaStream_t st) {
+static const char* mb_train_step_tc_launch(const mobody_train_ex_desc& x, const TrainWs& w, cudaStream_t st) {
+  const mobody_train_desc& d = x.base;
+  const bool adv = x.advantage, branch = adv || !x.scale_q || !x.q_weighted;
   TrainSide& side = train_side();
   // fork(i): the side stream continues after everything enqueued on `st` so far; join(i): `st` waits for the side stream
   auto fork = [&](int i) -> cudaStream_t {
@@ -1133,22 +1325,68 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
     pack_q(pa, false);
     if ((e = mb_pack_b_launch(pa, st))) return e;
   }
-  // ---- critic forward.  layer 1 of pi(s'), Q1(s,a), Q2(s,a), pi(s) side by side; then layer 2 (+ Q heads); then the policy tails ----
-  if ((e = run_gemms(st, 1, P(fwd_job(X + SA, rw, N, S, pi.w[0], pi.b[0], 256, T[0]), 0), P(fwd_job(X, rw, N, SA, q[0].w[0], q[0].b[0], 256, Hq[0][0]), 3),
-                     P(fwd_job(X, rw, N, SA, q[1].w[0], q[1].b[0], 256, Hq[1][0]), 4), P(fwd_job(X, rw, N, S, pi.w[0], pi.b[0], 256, Hp[0]), 0)))) return e;
+  // ---- advantage=1: value step.  Q'_k(s, a) and V(s) (V's activations in Hp / Dp), expectile gradient, V's backward,
+  //      weight gradients, Adam, and V's images again for V(s') / V(s_t) below.  Images: V W1, W2 forward, W2 backward ----
+  const MlpPtrs vf = as_ptrs(x.value);
+  float* img_v[3] = {ws + w.img_v[0], ws + w.img_v[1], ws + w.img_v[2]};
+  auto PV = [&](ug::Job j, int slot) { j.B = img_v[slot]; j.b_src = ug::SRC_PACKED; return j; };
+  auto pack_v = [&](int n) {
+    ug::PackArgs pa{};
+    pa.job[pa.njobs++] = pack_job(vf.w[0], S, ug::SRC_KCONTIG, 256, S, 256, img_v[0]);
+    pa.job[pa.njobs++] = pack_job(vf.w[1], 256, ug::SRC_KCONTIG, 256, 256, 256, img_v[1]);
+    if (n == 3) pa.job[pa.njobs++] = pack_job(vf.w[1], 256, ug::SRC_RCONTIG, 256, 256, 256, img_v[2]);
+    return mb_pack_b_launch(pa, st);
+  };
+  if (adv) {
+    const trn::ValueArgs v = value_args(x, w, ws);
+    if ((e = pack_v(3))) return e;
+    if ((e = run_gemms(st, 1, P(fwd_job(X, rw, N, SA, qt[0].w[0], qt[0].b[0], 256, T[0]), 7), P(fwd_job(X, rw, N, SA, qt[1].w[0], qt[1].b[0], 256, T[1]), 8),
+                       PV(fwd_job(X, rw, N, S, vf.w[0], vf.b[0], 256, v.Hv[0]), 0)))) return e;
+    ug::Job h[3] = {fwd_job(T[0], 256, N, 256, qt[0].w[1], qt[0].b[1], 256, nullptr), fwd_job(T[1], 256, N, 256, qt[1].w[1], qt[1].b[1], 256, nullptr),
+                    fwd_job(v.Hv[0], 256, N, 256, vf.w[1], vf.b[1], 256, v.Hv[1])};
+    const MlpPtrs* hn[3] = {&qt[0], &qt[1], &vf};
+    float* ho[3] = {v.qts[0], v.qts[1], v.vs};
+    for (int i = 0; i < 3; ++i) { h[i].epi = ug::EPI_HEAD; h[i].w3 = hn[i]->w[2]; h[i].b3 = hn[i]->b[2]; h[i].out1 = ho[i]; }
+    if ((e = run_gemms(st, 1, P(h[0], 9), P(h[1], 10), PV(h[2], 1)))) return e;
+    mb_launch(trn::value_loss_kernel, dim3((N + 255) / 256), dim3(256), 0, st, v);
+    trn::HeadBwdArgs hb{{v.Hv[1], nullptr}, {v.d3, nullptr}, {vf.w[2], nullptr}, {v.Dv[1], nullptr}, N};
+    mb_launch(trn::head_bwd_kernel, dim3(296, 1), dim3(256), 0, st, hb);
+    if ((e = run_gemms(st, 1, PV(bwd_job(v.Dv[1], 256, N, 256, vf.w[1], 256, 256, v.Hv[0], v.Dv[0]), 2)))) return e;
+    if ((e = run_gemms(st, ns, wgrad_job(v.Dv[0], 256, 256, X, rw, S, N, ws + w.gv[0], ws + w.gv[1]),
+                       wgrad_job(v.Dv[1], 256, 256, v.Hv[0], 256, 256, N, ws + w.gv[2], ws + w.gv[3]),
+                       wgrad_job(v.d3, 1, 1, v.Hv[1], 256, 256, N, ws + w.gv[4], ws + w.gv[5])))) return e;
+    if ((e = value_adam(x, w, ws, st))) return e;
+    if ((e = pack_v(2))) return e;
+  }
+  // ---- critic forward.  layer 1 of pi(s') (advantage=1: V(s') and V(s_t) instead), Q1(s,a), Q2(s,a), pi(s) side by side;
+  //      then layer 2 (+ Q / V heads); then the policy tails ----
+  float* vn = ws + w.vn; float* vh = ws + w.vh;
+  {
+    ug::Job l1[5] = {adv ? PV(fwd_job(X + SA, rw, N, S, vf.w[0], vf.b[0], 256, T[0]), 0) : P(fwd_job(X + SA, rw, N, S, pi.w[0], pi.b[0], 256, T[0]), 0),
+                     P(fwd_job(X, rw, N, SA, q[0].w[0], q[0].b[0], 256, Hq[0][0]), 3), P(fwd_job(X, rw, N, SA, q[1].w[0], q[1].b[0], 256, Hq[1][0]), 4),
+                     P(fwd_job(X, rw, N, S, pi.w[0], pi.b[0], 256, Hp[0]), 0), PV(fwd_job(X, rw, nt, S, vf.w[0], vf.b[0], 256, T[1]), 0)};
+    if ((e = run_gemm_list(st, 1, l1, adv ? 5 : 4))) return e;
+  }
   {
     ug::Job j1 = fwd_job(Hq[0][0], 256, N, 256, q[0].w[1], q[0].b[1], 256, Hq[0][1]), j2 = fwd_job(Hq[1][0], 256, N, 256, q[1].w[1], q[1].b[1], 256, Hq[1][1]);
     j1.epi = j2.epi = ug::EPI_HEAD; j1.w3 = q[0].w[2]; j1.b3 = q[0].b[2]; j1.out1 = qk[0]; j2.w3 = q[1].w[2]; j2.b3 = q[1].b[2]; j2.out1 = qk[1];
-    if ((e = run_gemms(st, 1, P(fwd_job(T[0], 256, N, 256, pi.w[1], pi.b[1], 256, T[1]), 1), P(j1, 5), P(j2, 6),
-                       P(fwd_job(Hp[0], 256, N, 256, pi.w[1], pi.b[1], 256, Hp[1]), 1)))) return e;
+    ug::Job l2[5] = {P(fwd_job(T[0], 256, N, 256, pi.w[1], pi.b[1], 256, T[1]), 1), P(j1, 5), P(j2, 6),
+                     P(fwd_job(Hp[0], 256, N, 256, pi.w[1], pi.b[1], 256, Hp[1]), 1), {}};
+    if (adv) {   // V(s') -> vn, V(s_t) -> vh: heads only, no activations stored
+      ug::Job hv[2] = {fwd_job(T[0], 256, N, 256, vf.w[1], vf.b[1], 256, nullptr), fwd_job(T[1], 256, nt, 256, vf.w[1], vf.b[1], 256, nullptr)};
+      for (int i = 0; i < 2; ++i) { hv[i].epi = ug::EPI_HEAD; hv[i].w3 = vf.w[2]; hv[i].b3 = vf.b[2]; hv[i].out1 = i ? vh : vn; }
+      l2[0] = PV(hv[0], 1); l2[4] = PV(hv[1], 1);
+    }
+    if ((e = run_gemm_list(st, 1, l2, adv ? 5 : 4))) return e;
   }
   {
     trn::RowDotArgs rd{}; rd.njobs = 2; rd.A = A; rd.scale = d.max_action; rd.tanh_act = 1;
     rd.job[0] = {T[1], pi.w[2], 256, 0, pi.b[2], a2, N}; rd.job[1] = {Hp[1], pi.w[2], 256, 0, pi.b[2], api, N};
-    mb_launch(trn::rowdot_kernel, dim3(296, 2), dim3(256), (size_t)A * 256 * sizeof(float), st, rd);
+    if (adv) { rd.job[0] = rd.job[1]; rd.njobs = 1; }                  // no pi(s'): only pi(s)
+    mb_launch(trn::rowdot_kernel, dim3(296, rd.njobs), dim3(256), (size_t)A * 256 * sizeof(float), st, rd);
   }
   // ---- target critics on (s', pi(s')): the input is [s' | a2], read from two sources ----
-  {
+  if (!adv) {
     ug::Job j1 = fwd_job(X + SA, rw, N, SA, qt[0].w[0], qt[0].b[0], 256, T[0]), j2 = fwd_job(X + SA, rw, N, SA, qt[1].w[0], qt[1].b[0], 256, T[1]);
     j1.A2 = j2.A2 = a2; j1.lda2 = j2.lda2 = A; j1.ksplit = j2.ksplit = S;
     if ((e = run_gemms(st, 1, P(j1, 7), P(j2, 8)))) return e;
@@ -1159,7 +1397,7 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
   }
   // ---- TD target + MSE gradient, head backward, backward-data ----
   {
-    trn::TdArgs t{X, N, S, A, rw, d.gamma, {qk[0], qk[1]}, {qtk[0], qtk[1]}, {d3[0], d3[1]}, ws + w.part};
+    trn::TdArgs t{X, N, S, A, rw, d.gamma, {qk[0], qk[1]}, {qtk[0], qtk[1]}, {d3[0], d3[1]}, ws + w.part, adv ? vn : nullptr};
     mb_launch(trn::td_kernel, dim3((N + 255) / 256), dim3(256), 0, st, t);
     trn::HeadBwdArgs hb{{Hq[0][1], Hq[1][1]}, {d3[0], d3[1]}, {q[0].w[2], q[1].w[2]}, {Dq[0][1], Dq[1][1]}, N};
     mb_launch(trn::head_bwd_kernel, dim3(296, 2), dim3(256), 0, st, hb);
@@ -1199,14 +1437,16 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
     pack_q(pa, true);
     if ((e = mb_pack_b_launch(pa, st))) return e;
   }
-  // ---- actor: Q_k(s, pi(s)) with the UPDATED, frozen critics (activations kept for the backward), q_hat_k on the true rows ----
+  // ---- actor: Q_k(s, pi(s)) with the UPDATED, frozen critics (activations kept for the backward), q_hat_k on the true rows
+  //      (any non-default flag: on all rows, for q_behavior) ----
+  const int nq = branch ? N : nt;
   {
     ug::Job j1 = fwd_job(X, rw, N, SA, q[0].w[0], q[0].b[0], 256, Hq[0][0]), j2 = fwd_job(X, rw, N, SA, q[1].w[0], q[1].b[0], 256, Hq[1][0]);
     j1.A2 = j2.A2 = api; j1.lda2 = j2.lda2 = A; j1.ksplit = j2.ksplit = S;
-    if ((e = run_gemms(st, 1, P(j1, 3), P(j2, 4), P(fwd_job(X, rw, nt, SA, q[0].w[0], q[0].b[0], 256, T[0]), 3),
-                       P(fwd_job(X, rw, nt, SA, q[1].w[0], q[1].b[0], 256, T[1]), 4)))) return e;
+    if ((e = run_gemms(st, 1, P(j1, 3), P(j2, 4), P(fwd_job(X, rw, nq, SA, q[0].w[0], q[0].b[0], 256, T[0]), 3),
+                       P(fwd_job(X, rw, nq, SA, q[1].w[0], q[1].b[0], 256, T[1]), 4)))) return e;
     ug::Job h[4] = {fwd_job(Hq[0][0], 256, N, 256, q[0].w[1], q[0].b[1], 256, Hq[0][1]), fwd_job(Hq[1][0], 256, N, 256, q[1].w[1], q[1].b[1], 256, Hq[1][1]),
-                    fwd_job(T[0], 256, nt, 256, q[0].w[1], q[0].b[1], 256, nullptr), fwd_job(T[1], 256, nt, 256, q[1].w[1], q[1].b[1], 256, nullptr)};
+                    fwd_job(T[0], 256, nq, 256, q[0].w[1], q[0].b[1], 256, nullptr), fwd_job(T[1], 256, nq, 256, q[1].w[1], q[1].b[1], 256, nullptr)};
     for (int i = 0; i < 4; ++i) { h[i].epi = ug::EPI_HEAD; h[i].w3 = q[i & 1].w[2]; h[i].b3 = q[i & 1].b[2]; h[i].out1 = i < 2 ? qv[i] : qh[i - 2]; }
     if ((e = run_gemms(st, 1, P(h[0], 5), P(h[1], 6), P(h[2], 5), P(h[3], 6)))) return e;
   }
@@ -1215,6 +1455,7 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
   for (int k = 0; k < 2; ++k) { ac.qv[k] = qv[k]; ac.qh[k] = qh[k]; ac.gak[k] = gak[k]; }
   ac.part = ws + w.part; ac.ntiles_c = (N + 255) / 256; ac.weight = d.weight; ac.out = ws + w.scal;
   ac.counter = reinterpret_cast<int*>(ws + w.cnt);
+  ac.scale_q = x.scale_q; ac.branch = branch; ac.n_qh = nq; ac.part_v = adv ? ws + w.partv : nullptr;
   mb_launch(trn::actor_scalar_kernel, dim3(1), dim3(1024), 0, fork(1), ac);      // single CTA: beside the dQ/da chain below
   {   // dQ_k / d action: head backward with unit gradient, backward-data through layers 2 and 1 (action columns of W1 only)
     trn::HeadBwdArgs hb{{Hq[0][1], Hq[1][1]}, {nullptr, nullptr}, {q[0].w[2], q[1].w[2]}, {Dq[0][1], Dq[1][1]}, N};
@@ -1230,6 +1471,7 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
   for (int k = 0; k < 2; ++k) { pb.gak[k] = gak[k]; pb.qv[k] = qv[k]; pb.qh[k] = qh[k]; }
   pb.api = api; pb.X = X; pb.bc_coef = d.bc_coef; pb.max_action = d.max_action;
   pb.d3p = d3p; pb.part = ws + w.part2; pb.out = ws + w.scal; pb.counter = reinterpret_cast<int*>(ws + w.cnt) + 1;
+  pb.vh = adv ? vh : nullptr; pb.q_weighted = x.q_weighted;
   join(1);
   mb_launch(trn::policy_grad_kernel, dim3((N + 127) / 128), dim3(128), 0, st, pb);
   // ---- policy backward-data: dH2 = (d3 W3) * 1[H2 > 0], dH1 = (dH2 W2) * 1[H1 > 0]; weight gradients; Adam ----
@@ -1255,19 +1497,32 @@ static const char* mb_train_step_tc_launch(const mobody_train_desc& d, const Tra
     }
   }
   if ((e = mb_train_adam_launch(ap, st))) return e;
-  if (d.scalars_out) cudaMemcpyAsync(d.scalars_out, ws + w.scal, 16 * sizeof(float), cudaMemcpyDeviceToDevice, st);
+  copy_scalars(x, ws + w.scal, st);
   return nullptr;
 }
 
-const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st) {
+const char* mb_train_step_launch(const mobody_train_ex_desc& x, cudaStream_t st) {
+  const mobody_train_desc& d = x.base;
   const int N = d.N, S = d.S, A = d.A, ns = d.nsplit;
   if (N < 1 || d.n_true < 1 || d.n_true > N || S < 1 || S > 128 || A < 1 || A > 32 || ns < 1 || ns > 64) return "train step: bad N/n_true/S/A/nsplit";
   const TrainWs w = train_ws(N, S, A, ns);
-  if (!d.workspace || d.workspace_bytes < (long long)w.total * 4) return "train step: workspace too small";
+  if (!d.workspace || d.workspace_bytes < (long long)(x.advantage ? w.total_ex : w.total) * 4) return "train step: workspace too small";
   // large batches: every contraction as tcgen05 GEMM tiles.  Cross-over measured on the tuned tiles (S17/A6, updates/s tcgen05
   // vs mma.sync): 640 rows 4 540 vs 6 435, 1 280 rows 4 350 vs 4 220, 1 920 rows 3 920 vs 3 340, 2 560 rows 4 180 vs 3 600
-  if (N >= MOBODY_TC_TRAIN_MIN_ROWS) return mb_train_step_tc_launch(d, w, st);
+  if (N >= MOBODY_TC_TRAIN_MIN_ROWS) return mb_train_step_tc_launch(x, w, st);
   float* ws = (float*)d.workspace;
+  const bool branch = x.advantage || !x.scale_q || !x.q_weighted;
+  // ---- advantage=1: value step (forward, expectile gradient, backward, weight gradients, Adam) ----
+  if (x.advantage) {
+    const trn::ValueArgs v = value_args(x, w, ws);
+    if (const char* e = mb_train_value_launch(v, st)) return e;
+    trn::WgradArgs g{}; g.N = N; g.nsplit = ns; g.njobs = 3;
+    g.job[0] = {v.Dv[0], 256, d.rows, d.row_width, ws + w.gv[0], ws + w.gv[1], 256, S};
+    g.job[1] = {v.Dv[1], 256, v.Hv[0], 256, ws + w.gv[2], ws + w.gv[3], 256, 256};
+    g.job[2] = {v.d3, 1, v.Hv[1], 256, ws + w.gv[4], ws + w.gv[5], 1, 256};
+    if (const char* e = mb_train_wgrad_launch(g, st)) return e;
+    if (const char* e = value_adam(x, w, ws, st)) return e;
+  }
   const mobody_mlp_state* qs[2] = {&d.q1, &d.q2};
   const mobody_mlp_state* qts[2] = {&d.q1_target, &d.q2_target};
   const mobody_mlp_state* qm[2] = {&d.q1_m, &d.q2_m};
@@ -1283,6 +1538,7 @@ const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st) {
   c.gamma = d.gamma; c.max_action = d.max_action; c.part = ws + w.part; c.a2 = ws + w.a2;
   c.Hp[0] = ws + w.Hp[0]; c.Hp[1] = ws + w.Hp[1]; c.api = ws + w.api;
   for (int k = 0; k < 2; ++k) { c.qk[k] = ws + w.qk[k]; c.qtk[k] = ws + w.qtk[k]; }
+  if (x.advantage) { c.v = as_ptrs(x.value); c.vn = ws + w.vn; c.vh = ws + w.vh; c.n_true = d.n_true; }
   if (const char* e = mb_train_critic_launch(c, st)) return e;
   // ---- critic weight gradients + Adam + Polyak ----
   trn::WgradArgs g{}; g.N = N; g.nsplit = ns; g.njobs = 6;
@@ -1314,12 +1570,14 @@ const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st) {
   for (int k = 0; k < 2; ++k) { ac.qv[k] = ws + w.qv[k]; ac.qh[k] = ws + w.qh[k]; ac.gak[k] = ws + w.gak[k]; }
   ac.part = ws + w.part; ac.ntiles_c = (N + TRAIN_TM - 1) / TRAIN_TM; ac.weight = d.weight; ac.out = ws + w.scal;
   ac.counter = reinterpret_cast<int*>(ws + w.cnt);
+  ac.scale_q = x.scale_q; ac.branch = branch; ac.n_qh = branch ? N : d.n_true; ac.part_v = x.advantage ? ws + w.partv : nullptr;
   if (const char* e = mb_train_actor_launch(ac, st)) return e;
   trn::PolicyBwdArgs pb{}; pb.N = N; pb.n_true = d.n_true; pb.S = S; pb.A = A; pb.rw = d.row_width; pb.pi = ac.pi;
   pb.Hp[0] = ac.Hp[0]; pb.Hp[1] = ac.Hp[1]; pb.Dp[0] = ws + w.Dp[0]; pb.Dp[1] = ws + w.Dp[1];
   for (int k = 0; k < 2; ++k) { pb.gak[k] = ac.gak[k]; pb.qv[k] = ac.qv[k]; pb.qh[k] = ac.qh[k]; }
   pb.api = ac.api; pb.X = d.rows; pb.bc_coef = d.bc_coef; pb.max_action = d.max_action;
   pb.d3p = ws + w.d3p; pb.part = ws + w.part2; pb.out = ws + w.scal; pb.counter = reinterpret_cast<int*>(ws + w.cnt) + 1;
+  pb.vh = x.advantage ? ws + w.vh : nullptr; pb.q_weighted = x.q_weighted;
   if (const char* e = mb_train_policy_bwd_launch(pb, st)) return e;
   trn::WgradArgs gp{}; gp.N = N; gp.nsplit = ns; gp.njobs = 3;
   gp.job[0] = {pb.Dp[0], 256, d.rows, d.row_width, ws + w.gp[0], ws + w.gp[1], 256, S};
@@ -1338,7 +1596,7 @@ const char* mb_train_step_launch(const mobody_train_desc& d, cudaStream_t st) {
     }
   }
   if (const char* e = mb_train_adam_launch(ap, st)) return e;
-  if (d.scalars_out) cudaMemcpyAsync(d.scalars_out, ws + w.scal, 16 * sizeof(float), cudaMemcpyDeviceToDevice, st);
+  copy_scalars(x, ws + w.scal, st);
   return nullptr;
 }
 

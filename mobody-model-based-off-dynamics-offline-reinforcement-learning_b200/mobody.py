@@ -54,7 +54,7 @@ class Policy(nn.Module):                                       # mobody.py:60-72
         return out
 
     def forward_autograd(self, x):
-        """Same function through torch ops (differentiable): used only by the non-default update branches."""
+        """Same function through torch ops (differentiable): used only by the torch reference update (_train_torch_path)."""
         return torch.tanh(self.network(x)) * self.max_action
 
 
@@ -64,7 +64,7 @@ class DoubleQFunc(nn.Module):                                  # mobody.py:74-83
         self.network1 = MLPNetwork(state_dim + action_dim, 1, hidden_size)
         self.network2 = MLPNetwork(state_dim + action_dim, 1, hidden_size)
 
-    def forward(self, state, action):                          # torch ops: non-default update branches only
+    def forward(self, state, action):                          # torch ops: the torch reference update only
         x = torch.cat((state, action), dim=1)
         return self.network1(x), self.network2(x)
 
@@ -172,7 +172,7 @@ class MOBODY(object):
                       "v": _adam(self.v_func.parameters(), config["critic_lr"]),
                       "pi": _adam(self.policy.parameters(), config["actor_lr"]),
                       "cls": _adam(self.classifier.parameters(), config["actor_lr"])}
-        self._t_q = self._t_pi = self._t_cls = 0                 # steps taken by the fused kernels (host counters) ...
+        self._t_q = self._t_pi = self._t_cls = self._t_v = 0     # steps taken by the fused kernels (host counters) ...
         self._steps_dirty = set()                                # ... flushed into the optimizers' ``step`` tensors on access
         self._moment_cache = {}
         self._cls_ws, self._cls_scalars = None, torch.zeros(2, dtype=torch.float32, device=self.device)
@@ -192,7 +192,7 @@ class MOBODY(object):
         self._wave = sm * 128
 
     # ------------------------------------------------------------------ optimizers (mobody.py:127-135)
-    _OPT_COUNTER = {"q": "_t_q", "pi": "_t_pi", "cls": "_t_cls"}
+    _OPT_COUNTER = {"q": "_t_q", "v": "_t_v", "pi": "_t_pi", "cls": "_t_cls"}
 
     def _optimizer(self, name):
         """The torch optimizer ``name`` with its ``step`` tensors brought up to date with the fused kernels' counters."""
@@ -621,12 +621,13 @@ class MOBODY(object):
     def train_on_rows(self, rows, n_true, *, nsplit=None):
         """One fused critic + Polyak + actor update on packed batch rows [N, RW] (device, rows ordered
         src, tar, fake; the first ``n_true`` rows are the src+tar rows of the BC term).  Asynchronous:
-        losses land in ``self._scalars`` (device).  mobody.py:541-573.
+        losses land in ``self._scalars`` (device).  mobody.py:533-573.  The config flags select the update's branches:
+        ``advantage`` (value step first, V(s') TD target, V(s_t) advantage weights), ``scale_Q`` and ``q_weighted``;
+        the default flags take mobody_train_step, every other combination mobody_train_step_ex.
         ``nsplit`` overrides the row-split count of the weight-gradient GEMMs (1..64; tests)."""
         cfg = self.config
-        if not self._fused_update_ok():
-            raise RuntimeError("train_on_rows is the fused default update (advantage=0, scale_Q=1, q_weighted=1); "
-                               "train() routes the other branches through the torch path")
+        default = self._default_update()
+        advantage = bool(cfg.get("advantage", 0))
         S, A = cfg["state_dim"], cfg["action_dim"]
         N = rows.shape[0]
         if nsplit is None:
@@ -637,12 +638,13 @@ class MOBODY(object):
             else:
                 nsplit = _wgrad_splits(N, (2 * (8 + 2 * ((S + A + 63) // 64)), 8 + 2 * ((S + 63) // 64)), self.device)
         lib = _ffi.lib()
-        need = int(lib.mobody_train_workspace_bytes(N, S, A, nsplit))
+        need = int(lib.mobody_train_workspace_bytes(N, S, A, nsplit) if default else lib.mobody_train_ex_workspace_bytes(N, S, A, nsplit))
         if self._train_ws is None or self._train_ws.numel() < need:
             self._train_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         self._t_q += 1; self._t_pi += 1
         self._steps_dirty.update(("q", "pi"))
-        d = _ffi.TrainDesc()
+        x = _ffi.TrainExDesc()
+        d = x.base
         d.rows, d.N, d.n_true, d.S, d.A, d.row_width = _ffi.ptr(rows), N, int(n_true), S, A, rows.shape[1]
         qt = self.target_q_funcs
         d.policy = _ffi.mlp_state(_ffi.mlp_tensors(self.policy.network))
@@ -659,18 +661,32 @@ class MOBODY(object):
         d.weight, d.bc_coef, d.max_action = float(cfg["weight"]), float(cfg.get("bc_coef", 1.0)), float(cfg["max_action"])
         d.nsplit, d.workspace, d.workspace_bytes = nsplit, _ffi.ptr(self._train_ws), self._train_ws.numel()
         d.scalars_out = _ffi.ptr(self._scalars)
-        _ffi.check(lib.mobody_train_step(C.byref(d), _ffi.stream_ptr(self.device)))
+        if default:
+            _ffi.check(lib.mobody_train_step(C.byref(d), _ffi.stream_ptr(self.device)))
+            return self._scalars
+        x.advantage, x.scale_q, x.q_weighted = int(advantage), int(bool(cfg.get("scale_Q", 1))), int(bool(cfg.get("q_weighted", 1)))
+        if advantage:
+            self._t_v += 1
+            self._steps_dirty.add("v")
+            ((v_m, v_v),) = self._moments("v", (self.v_func.network,))
+            x.value = _ffi.mlp_state(_ffi.mlp_tensors(self.v_func.network))
+            x.value_m, x.value_v, x.t_v = _ffi.mlp_state(v_m), _ffi.mlp_state(v_v), self._t_v
+        _ffi.check(lib.mobody_train_step_ex(C.byref(x), _ffi.stream_ptr(self.device)))
         # (parameters were updated in place behind autograd's version counters; the packed tensor-core image of the
         # policy follows them through the library's device-side checksum, dynamics._packed_image)
         return self._scalars
 
     def loss_scalars(self):
-        """Host copy of the last step's diagnostics (one D2H sync; call sparingly)."""
+        """Host copy of the last step's diagnostics (one D2H sync; call sparingly).  With advantage=1 it adds the value
+        step's loss, mean advantage and mean V(s)."""
         v = self._scalars.cpu().tolist()
-        return dict(q_loss=v[0], q1_mean=v[1], pi_loss=v[2], bc_loss=v[3], q_policy=v[4], q_abs_mean=v[5],
-                    w_mean=v[6], w_min=v[7], w_max=v[8], p_w=v[9])
+        out = dict(q_loss=v[0], q1_mean=v[1], pi_loss=v[2], bc_loss=v[3], q_policy=v[4], q_abs_mean=v[5],
+                   w_mean=v[6], w_min=v[7], w_max=v[8], p_w=v[9])
+        if self.config.get("advantage", 0):
+            out.update(v_loss=v[11], adv_mean=v[12], v_mean=v[13])
+        return out
 
-    def _fused_update_ok(self):
+    def _default_update(self):
         cfg = self.config
         return not cfg.get("advantage", 0) and bool(cfg.get("scale_Q", 1)) and bool(cfg.get("q_weighted", 1))
 
@@ -736,18 +752,15 @@ class MOBODY(object):
                 self.refresh_fake_buffer(src_replay_buffer, tar_replay_buffer, inj, batch_size)
             if n_fake:
                 self.fake_replay_buffer.sample_rows(n_fake, inj.get("fake"), out=rows[n_src + n_tar:])   # :524
-        if self._fused_update_ok():
-            self.train_on_rows(rows, n_src + n_tar)
-            self._train_side_effects(writer, wandbrun)
-        else:
-            self._train_torch_path(rows, n_src + n_tar, writer, wandbrun)
+        self.train_on_rows(rows, n_src + n_tar)
+        self._train_side_effects(writer, wandbrun)
 
     def _train_torch_path(self, rows, n_true, writer, wandbrun):
-        """The update branches the fused kernels do not cover -- ``advantage=1`` (value-function baseline, mobody.py:210-242,
-        533-539), ``scale_Q=0`` (update_policy_1, :278-310) and ``q_weighted=0`` (:262-263) -- run through torch autograd on
-        the same device-resident batch rows and the same torch.optim.Adam objects (whose moments the fused kernels share),
-        as SURVEY section 2 #4 asks ("must keep working via the unchanged PyTorch path").  Off by default in every shipped
-        config; not a performance path."""
+        """The reference update as torch autograd, every branch -- ``advantage=1`` (value-function baseline, mobody.py:210-242,
+        533-539), ``scale_Q=0`` (update_policy_1, :278-310), ``q_weighted=0`` (:262-263) and the default flags -- on the same
+        device-resident batch rows and the same torch.optim.Adam objects (whose moments the fused kernels share).  train()
+        runs the fused kernels for every flag combination; this path is the reference the tests compare them against.  Not a
+        performance path."""
         cfg = self.config
         S, A = cfg["state_dim"], cfg["action_dim"]
         state, action, next_state = rows[:, :S], rows[:, S:S + A], rows[:, S + A:2 * S + A]
@@ -765,6 +778,7 @@ class MOBODY(object):
                 writer.add_scalar("train/value", v.mean(), self.total_it)
             v_loss = torch.mean(torch.abs(0.7 - (adv < 0).float()) * adv ** 2)                        # asymmetric_l2_loss(adv, 0.7), :85-86
             self.v_optimizer.zero_grad(); v_loss.backward(); self.v_optimizer.step()
+            self._pull_steps("v")
         with torch.no_grad():                                                                         # :189-195 / :210-216
             if cfg.get("advantage", 0):
                 q_target = self.v_func(next_state)
@@ -820,7 +834,9 @@ class MOBODY(object):
         if self.total_it % 1000 == 0 and cfg.get("q_weighted", 1):                                    # :269-270
             v = self.loss_scalars()
             print(v["w_mean"], v["w_min"], v["w_max"])
-        if writer is not None and self.total_it % 5000 == 0:                                          # :203-205, 272-274, 332-344
+        if not self._default_update():
+            self._branch_side_effects(writer, wandbrun)
+        elif writer is not None and self.total_it % 5000 == 0:                                        # :203-205, 272-274, 332-344
             v = self.loss_scalars()
             writer.add_scalar("train/q1", v["q1_mean"], self.total_it)
             writer.add_scalar("train/exp_adv", v["w_mean"], self.total_it)
@@ -830,6 +846,27 @@ class MOBODY(object):
             if wandbrun is not None:
                 wandbrun.log({"train/q1": v["q1_mean"], "train/q_policy": v["q_policy"], "train/policy_loss": v["pi_loss"]},
                              step=self.total_it)
+
+    def _branch_side_effects(self, writer, wandbrun):
+        """The writer / wandb keys of the update branches, in _train_torch_path's order (:217-218, 203-205, 272-274, 332-344)."""
+        if writer is None or self.total_it % 5000 != 0:
+            return
+        cfg, it = self.config, self.total_it
+        v = self.loss_scalars()
+        q_beh = float(self._scalars[14])
+        if cfg.get("advantage", 0):
+            writer.add_scalar("train/adv", v["adv_mean"], it)
+            writer.add_scalar("train/value", v["v_mean"], it)
+        writer.add_scalar("train/q1", v["q1_mean"], it)
+        if wandbrun is not None:
+            wandbrun.log({"train/q1": v["q1_mean"]}, step=it, commit=False)
+        writer.add_scalar("train/exp_adv", v["w_mean"] if cfg.get("q_weighted", 1) else 1.0, it)
+        writer.add_scalar("train/bc_loss", v["bc_loss"], it)
+        writer.add_scalar("train/q_behavior", q_beh, it)
+        writer.add_scalar("train/q_policy", v["q_policy"], it)
+        writer.add_scalar("train/policy_loss", v["pi_loss"], it)
+        if wandbrun is not None:
+            wandbrun.log({"train/q_behavior": q_beh, "train/q_policy": v["q_policy"], "train/policy_loss": v["pi_loss"]}, step=it)
 
     def refresh_fake_buffer(self, src_buf, tar_buf, inj=None, batch_size=128):
         """Synthetic-data refresh (mobody.py:441-475): two policy rollouts through the learned target dynamics and one
