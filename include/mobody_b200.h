@@ -49,6 +49,9 @@ extern "C" {
                                       A <= MOBODY_TC_WIDE_MAX_A (Ant's 111 / 8); packed images are bf16x2's */
 #define MOBODY_PREC_BF16X2_T64 5   /* bf16x2's arithmetic on the same 64-row tiles for the S <= 64 shapes bf16x2 refuses
                                       (Adroit's pen 45 / 24, door 39 / 28, relocate 39 / 30, hammer 46 / 26); packed images are bf16x2's */
+#define MOBODY_PREC_FP16_T64 6     /* fp16's arithmetic (single pass, packed-half epilogue, the stated looser bound 5e-3,
+                                      |activations| < 6e4) on the same 64-row tiles for the shapes fp16 refuses (Ant's 111 / 8,
+                                      Adroit); packed images are fp16's */
 /* Shapes of the tensor-core modes: S <= 64, A <= 16, and the [s, a, s'] operand plane of the reward model must fit in
    shared memory next to the other planes: 2S+A <= 96 (bf16x2: hi and lo planes, one row tile per CTA) or 112 (fp16: two
    row tiles per CTA).  mobody_step rejects other shapes with MOBODY_ERR_ARG; the fp32 mode takes S <= 128, A <= 32. */
@@ -65,6 +68,9 @@ extern "C" {
    bf16x2_t64 and bf16x2_wide split the fp32 mode's shapes with no overlap: at most one of them takes a given (S, A). */
 #define MOBODY_TC_T64_MAX_S 64
 #define MOBODY_TC_T64_MAX_A 32
+/* Shapes of MOBODY_PREC_FP16_T64: 2 <= S <= MOBODY_TC_WIDE_MAX_S, 1 <= A <= MOBODY_TC_WIDE_MAX_A, and not (S <= MOBODY_TC_MAX_S,
+   A <= MOBODY_TC_MAX_A and 2S+A <= MOBODY_TC_FP16_MAX_SAS) -- exactly the shapes the fp32 mode takes and fp16 refuses.  So fp16
+   and fp16_t64 split the fp32 mode's shapes with no overlap. */
 
 /* compaction predicates */
 #define MOBODY_KEEP_U8_ZERO 0 /* keep rows with flag == 0      (non-terminal rows, mobody.py:635)   */
@@ -379,7 +385,8 @@ typedef struct mobody_dynfit_desc {
 long long mobody_dynfit_workspace_bytes(int B, int S, int A, int nsplit);
 int mobody_dynfit_step(const mobody_dynfit_desc* d, void* stream);
 
-/* ---- tensor-core weight images (precision MOBODY_PREC_BF16X2, MOBODY_PREC_BF16X2_WIDE or MOBODY_PREC_BF16X2_T64: one format; MOBODY_PREC_FP16) ----
+/* ---- tensor-core weight images (precision MOBODY_PREC_BF16X2, MOBODY_PREC_BF16X2_WIDE or MOBODY_PREC_BF16X2_T64: one format;
+ *      MOBODY_PREC_FP16 or MOBODY_PREC_FP16_T64: another) ----
  * The reference keeps weights as fp32 nn.Parameters (mobody_module.py:371-391, mobody.py:35-48); the
  * tcgen05 path consumes them as 16-bit planes in the UMMA shared-memory layout (one launch per image).
  * `state`: NULL -> pack unconditionally.  Otherwise device uint64[4], zero-initialised ONCE by the caller and then

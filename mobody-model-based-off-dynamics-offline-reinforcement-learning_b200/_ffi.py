@@ -18,16 +18,17 @@ DYN_LAYER_NAMES = ("zs1", "zs2", "zs3", "za_src1", "za_src2", "za_trg1", "za_trg
                    "reward_model1", "reward_model2", "reward_model3")
 # fp32: CUDA-core kernel; bf16x2: tcgen05 hi+lo split, inside the 1e-4 bound (default); fp16: tcgen05 single pass, inside the
 # stated looser bound 5e-3; bf16x2_wide: bf16x2's arithmetic on 64-row tiles for 65 <= S <= 128; bf16x2_t64: the same 64-row
-# kernel for the S <= 64 shapes bf16x2 refuses (A > 16 or 2S+A > 96: Adroit).  Both are opt-in: "auto" keeps fp32 for the
-# shapes bf16x2 refuses.  The library's single-pass bf16 mode (code 2, measured 1.6e-2) is outside every stated bound: it is a
-# kernel-development diagnostic and is not offered here.
-PREC = {"fp32": 0, "bf16x2": 1, "fp16": 3, "bf16x2_wide": 4, "bf16x2_t64": 5}
-# the general modes, which take the small shapes every test and the benchmark sweep; bf16x2_wide and bf16x2_t64 do not
+# kernel for the S <= 64 shapes bf16x2 refuses (A > 16 or 2S+A > 96: Adroit); fp16_t64: fp16's arithmetic on the same
+# 64-row kernel for the shapes fp16 refuses (S > 64, A > 16 or 2S+A > 112), inside fp16's bound 5e-3.  All three are opt-in:
+# "auto" keeps fp32 for the shapes bf16x2 refuses.  The library's single-pass bf16 mode (code 2, measured 1.6e-2) is
+# outside every stated bound: it is a kernel-development diagnostic and is not offered here.
+PREC = {"fp32": 0, "bf16x2": 1, "fp16": 3, "bf16x2_wide": 4, "bf16x2_t64": 5, "fp16_t64": 6}
+# the general modes, which take the small shapes every test and the benchmark sweep; the 64-row modes do not
 ENABLED_PRECISIONS = ("fp32", "bf16x2", "fp16")
 # shapes the tensor-core modes take (MOBODY_TC_* in include/mobody_b200.h): S <= 64, A <= 16, 2S+A <= the mode's limit
 TC_MAX_S, TC_MAX_A, TC_MAX_SAS = 64, 16, {"bf16x2": 96, "fp16": 112}
 # shapes of bf16x2_wide (MOBODY_TC_WIDE_*): TC_WIDE_MIN_S <= S <= TC_WIDE_MAX_S, A <= TC_WIDE_MAX_A
-TC_WIDE_MIN_S, TC_WIDE_MAX_S, TC_WIDE_MAX_A = 65, 128, 32
+TC_WIDE_MIN_S, TC_WIDE_MAX_S, TC_WIDE_MAX_A = 65, 128, 32   # fp16_t64: 2 <= S <= TC_WIDE_MAX_S, A <= TC_WIDE_MAX_A, not fp16's
 # shapes of bf16x2_t64 (MOBODY_TC_T64_*): 2 <= S <= TC_T64_MAX_S, A <= TC_T64_MAX_A, and a shape bf16x2 refuses
 TC_T64_MAX_S, TC_T64_MAX_A = 64, 32
 ABI_VERSION = 2

@@ -40,7 +40,7 @@ void mb_model_eval_accumulate_launch(const float* reward, const long long* row_i
 const char* mb_tc_dyn_pack(const DynPtrs& dp, int S, int A, int ns, int fp16, unsigned char* blob, unsigned long long* state, cudaStream_t st);
 const char* mb_tc_mlp_pack(const MlpPtrs& mp, int din, int dout, int ns, int fp16, unsigned char* blob, unsigned long long* state, cudaStream_t st);
 const char* mb_tc_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, int ns, cudaStream_t st);
-const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, cudaStream_t st);
+const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, int fp16, cudaStream_t st);
 const char* mb_tc_duo_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, int fp16, cudaStream_t st, bool* launched);
 const char* mb_umma_selftest_launch(const float* A, const float* B, int K, int N, int nsplit, float* D, cudaStream_t st);
 void mb_ring_insert_transitions_launch(const float* packed, long long n_cap, const int* n_dev, int S, int A, int rw, long long ptr, long long cap,
@@ -115,6 +115,10 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
       (d->S > MOBODY_TC_T64_MAX_S || d->A > MOBODY_TC_T64_MAX_A ||
        (d->A <= MOBODY_TC_MAX_A && 2 * d->S + d->A <= MOBODY_TC_BF16X2_MAX_SAS)))
     return fail(MOBODY_ERR_ARG, "mobody_step: bf16x2_t64 takes S <= 64, A <= 32 with A > 16 or 2S+A > 96");
+  if (d->precision == MOBODY_PREC_FP16_T64 &&
+      (d->S > MOBODY_TC_WIDE_MAX_S || d->A > MOBODY_TC_WIDE_MAX_A ||
+       (d->S <= MOBODY_TC_MAX_S && d->A <= MOBODY_TC_MAX_A && 2 * d->S + d->A <= MOBODY_TC_FP16_MAX_SAS)))
+    return fail(MOBODY_ERR_ARG, "mobody_step: fp16_t64 takes S <= 128, A <= 32 outside fp16's S <= 64, A <= 16, 2S+A <= 112");
   StepArgs a;
   memset(&a, 0, sizeof(a));
   a.obs = d->obs; a.act = d->policy ? nullptr : d->act; a.eps = d->eps; a.idx = d->idx; a.elites = d->elites;
@@ -159,10 +163,11 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
       break;
     case MOBODY_PREC_BF16X2_WIDE:
     case MOBODY_PREC_BF16X2_T64:
+    case MOBODY_PREC_FP16_T64:
       if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
       if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
       err = mb_tc_wide_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr,
-                                   (cudaStream_t)stream);
+                                   d->precision == MOBODY_PREC_FP16_T64, (cudaStream_t)stream);
       break;
     default: return fail(MOBODY_ERR_UNSUPPORTED, "mobody_step: unknown precision mode");
   }
@@ -526,7 +531,9 @@ int mobody_dara_relabel(float* rows, long long n, int S, int A, int row_width, c
   return check_launch("mobody_dara_relabel");
 }
 
-static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE || precision == MOBODY_PREC_BF16X2_T64) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16) ? 1 : 0; }
+static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE || precision == MOBODY_PREC_BF16X2_T64) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16 || precision == MOBODY_PREC_FP16_T64) ? 1 : 0; }
+// the single fp16 plane of the fp16 modes (one image format for MOBODY_PREC_FP16 and MOBODY_PREC_FP16_T64)
+static int is_fp16(int precision) { return precision == MOBODY_PREC_FP16 || precision == MOBODY_PREC_FP16_T64; }
 
 long long mobody_dyn_pack_bytes(int S, int A, int precision) {
   int ns = nsplit_of(precision);
@@ -540,7 +547,7 @@ int mobody_dyn_pack(const mobody_dyn_params* dyn, int S, int A, int precision, v
   DynPtrs dp; memcpy(&dp, dyn, sizeof(dp));
   for (int i = 0; i < L_COUNT; ++i)
     if (!dp.w[i] || !dp.b[i]) return fail(MOBODY_ERR_ARG, "mobody_dyn_pack: null parameter pointer");
-  const char* err = mb_tc_dyn_pack(dp, S, A, ns, precision == MOBODY_PREC_FP16, (unsigned char*)blob, state, (cudaStream_t)stream);
+  const char* err = mb_tc_dyn_pack(dp, S, A, ns, is_fp16(precision), (unsigned char*)blob, state, (cudaStream_t)stream);
   if (err) return fail(MOBODY_ERR_ARG, err);
   return check_launch("mobody_dyn_pack");
 }
@@ -555,7 +562,7 @@ int mobody_mlp_pack(const mobody_mlp_params* mlp, int din, int dout, int precisi
   int ns = nsplit_of(precision);
   if (!ns || !mlp || !blob || din < 1 || dout < 1) return fail(MOBODY_ERR_ARG, "mobody_mlp_pack: bad arguments");
   MlpPtrs mp; memcpy(&mp, mlp, sizeof(mp));
-  const char* err = mb_tc_mlp_pack(mp, din, dout, ns, precision == MOBODY_PREC_FP16, (unsigned char*)blob, state, (cudaStream_t)stream);
+  const char* err = mb_tc_mlp_pack(mp, din, dout, ns, is_fp16(precision), (unsigned char*)blob, state, (cudaStream_t)stream);
   if (err) return fail(MOBODY_ERR_ARG, err);
   return check_launch("mobody_mlp_pack");
 }

@@ -1,16 +1,21 @@
-// Fused one-step model rollout on the tensor cores on 64-row tiles (2 <= S <= 128, 1 <= A <= 32), sm_100a.  It serves two
-// modes that differ only in the shapes mobody_step lets through: bf16x2_wide (65 <= S <= 128) and bf16x2_t64 (S <= 64
-// with A > 16 or 2S+A > 96: the shapes the 128-row kernel cannot hold, such as Adroit's pen at 45 / 24).
+// Fused one-step model rollout on the tensor cores on 64-row tiles (2 <= S <= 128, 1 <= A <= 32), sm_100a.  The kernel is a
+// template over its arithmetic:
+//  * F16 = false: bf16x2's arithmetic (bf16 hi+lo split of both operands, 3 MMAs per K step, inside the 1e-4 bound) on the
+//    two-plane images of mobody_dyn_pack / mobody_mlp_pack.  It serves bf16x2_wide (65 <= S <= 128) and bf16x2_t64 (S <= 64
+//    with A > 16 or 2S+A > 96: the shapes the 128-row kernel cannot hold, such as Adroit's pen at 45 / 24).
+//  * F16 = true: the fp16 mode's arithmetic (step_duo.cu): one fp16 plane per operand, one MMA per K step and the
+//    packed-half epilogue of tc_epi.cuh, inside the stated looser bound 5e-3.  It serves fp16_t64: the shapes of the fp32
+//    mode that the fp16 mode's 128-row kernel refuses.
+// Swish layers arrive pre-scaled by the packer for the mode's plane count.  What differs from step_tc.cu is the row tile:
+// one CTA owns 64 rows (UMMA M = 64), so every operand plane is half the size of step_tc.cu's and the planes of S <= 128,
+// A <= 32 (the [s | a | s'] plane of the reward model reaches K = 288) fit in shared memory next to a weight ring of at
+// least 4 stages (DESIGN.md 4.1c, 4.1e).  Everything after the last GEMM of a chain (transition3's means, the ensemble
+// statistics, noise, pick, penalty, termination, the mean of the reward heads) is the same fp32 code in both.
 //
-// Sibling of step_tc.cu with the same arithmetic (bf16 hi+lo split of both operands, 3 MMAs per K step, inside the 1e-4
-// bound; swish layers pre-scaled by the packer) and the same packed weight images (mobody_dyn_pack / mobody_mlp_pack with
-// two planes).  What changes is the row tile: one CTA owns 64 rows (UMMA M = 64), so every operand plane is half the size
-// of step_tc.cu's and the planes of S <= 128, A <= 32 (the [s | a | s'] plane of the reward model reaches K = 288) fit in
-// shared memory next to a weight ring of at least 4 stages (DESIGN.md 4.1c).
-//
-//  * producer warp: per layer, its bias (ring of NB slots) and one K step of both weight planes per stage (1-D TMA bulk
-//    copies, mbarrier complete_tx);
-//  * MMA warp: one elected thread issues tcgen05.mma 64 x N x 16 into TMEM (two 256-column accumulators, ping-pong);
+//  * producer warp: per layer, its bias (ring of NB slots) and the weight K steps through the ring (1-D TMA bulk copies,
+//    mbarrier complete_tx): bf16x2, one K step of both planes per stage; fp16, up to F16_KPS K steps of its plane;
+//  * MMA warp: one elected thread issues tcgen05.mma 64 x N x 16 into TMEM (two 256-column accumulators, ping-pong); in
+//    fp16 it waits and commits once per ring stage, since one MMA is shorter than the issuing thread's wait and commit;
 //  * 16 epilogue warps (4 groups x 4 TMEM lane quadrants).  An M = 64 accumulator puts row i in TMEM lane
 //    32 * (i / 16) + i % 16, so quadrant q holds rows 16q .. 16q+15 in its first 16 lanes.  tcgen05.ld 16x32bx2 gives
 //    thread `lane` row 16q + lane % 16 and, per 64-column chunk, the 8 columns group * 16 + (lane / 16) * 8: one K group
@@ -27,12 +32,12 @@ namespace tcw {
 using namespace tce;
 
 constexpr int TM = 64;                   // rows per CTA (UMMA M)
-constexpr int NS = 2;                    // bf16 hi + lo planes
 constexpr int NG = 4;                    // epilogue groups of 4 warps (one warp per TMEM lane quadrant)
 constexpr int SLOTS = 2 * NG;            // epilogue threads per row
 constexpr int CHUNK = 64;                // accumulator columns per announced chunk
-constexpr uint32_t KG = TM * 16;         // bytes of one 8-wide K group of one plane (64 rows x 8 x bf16)
-constexpr uint32_t MAIN_PLANE = 32 * KG; // 64 rows x 256 k x bf16
+constexpr uint32_t KG = TM * 16;         // bytes of one 8-wide K group of one plane (64 rows x 8 x 16 bits)
+constexpr uint32_t MAIN_PLANE = 32 * KG; // 64 rows x 256 k x 16 bits
+constexpr int F16_KPS = 4;               // fp16: K steps of a 256-wide layer per ring stage (one 64-column chunk)
 constexpr int MAX_NST = 12;
 constexpr int NB = 4;                    // bias ring slots (one layer's bias each)
 constexpr int BSLOT = 528;               // floats per slot: 256 bias + reward_model3 vector (272) behind reward_model2's bias
@@ -50,9 +55,12 @@ struct Bars {
   uint32_t tmem_slot, pad;
 };
 
+// F16: one fp16 plane per operand and the packed-half epilogue instead of the bf16 hi + lo planes and fp32 epilogue math
+template <bool F16>
 __global__ void __launch_bounds__(32 * (4 * NG + 2), 1)
 step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const unsigned char* __restrict__ polb,
                  const __grid_constant__ TcSched sched, const Cfg cfg) {
+  constexpr int NS = F16 ? 1 : 2;          // operand planes: fp16, or bf16 hi + lo
   constexpr int EPI_WARPS = 4 * NG, PROD_WARP = EPI_WARPS, MMA_WARP = EPI_WARPS + 1;
   extern __shared__ __align__(128) unsigned char smem[];
   const int S = a.S, A = a.A, B = a.B;
@@ -98,11 +106,22 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
           tc::mbar_arrive_expect_tx(&bars->b_full[slot], bb);
           tc::bulk_g2s(bias_s + slot * BSLOT, bsrc, bb, &bars->b_full[slot]);
         }
-        for (int s = 0; s < L.ksteps; ++s) {
-          tc::mbar_wait(&bars->w_empty[stage], phase ^ 1u);
-          tc::mbar_arrive_expect_tx(&bars->w_full[stage], bytes);
-          tc::bulk_g2s(wst + (size_t)stage * cfg.stage_bytes, src + (size_t)s * bytes, bytes, &bars->w_full[stage]);
-          if (++stage == cfg.nst) { stage = 0; phase ^= 1u; }
+        if constexpr (F16) {   // as many K steps per stage as fit (F16_KPS of a 256-wide layer, all of a narrow one): one copy
+          const int kps = max(1, min((int)L.ksteps, (int)(cfg.stage_bytes / bytes)));
+          for (int s = 0; s < L.ksteps; s += kps) {
+            const uint32_t nb = (uint32_t)min(kps, (int)L.ksteps - s) * bytes;
+            tc::mbar_wait(&bars->w_empty[stage], phase ^ 1u);
+            tc::mbar_arrive_expect_tx(&bars->w_full[stage], nb);
+            tc::bulk_g2s(wst + (size_t)stage * cfg.stage_bytes, src + (size_t)s * bytes, nb, &bars->w_full[stage]);
+            if (++stage == cfg.nst) { stage = 0; phase ^= 1u; }
+          }
+        } else {
+          for (int s = 0; s < L.ksteps; ++s) {
+            tc::mbar_wait(&bars->w_empty[stage], phase ^ 1u);
+            tc::mbar_arrive_expect_tx(&bars->w_full[stage], bytes);
+            tc::bulk_g2s(wst + (size_t)stage * cfg.stage_bytes, src + (size_t)s * bytes, bytes, &bars->w_full[stage]);
+            if (++stage == cfg.nst) { stage = 0; phase ^= 1u; }
+          }
         }
       }
     }
@@ -120,24 +139,47 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
         uint32_t abase, aplane;
         if (L.a_region == REG_MAIN) { abase = main0; aplane = MAIN_PLANE; }
         else { aplane = cfg.small_plane; abase = small0 + (L.a_region == REG_SA ? cfg.sa_off : 0u); }
-        const uint32_t idesc = tc::make_idesc_bf16(TM, L.n);
         const uint32_t bplane = (uint32_t)L.n * 32u, blbo = (uint32_t)L.n * 16u;
-        for (int s = 0; s < L.ksteps; ++s) {
-          if ((s & 3) == 0 && (s >> 2) < L.a_wait) {     // a chunk is 64 columns = 4 K steps
-            const int c = s >> 2;
-            tc::mbar_wait(&bars->a_ready[c], (aph >> c) & 1u); aph ^= (1u << c);
+        if constexpr (F16) {
+          // one wait and one commit per ring stage (the producer's K-step grouping); operand chunks are awaited per K step
+          const uint32_t idesc = tc::make_idesc_f16(TM, L.n);
+          const int kps = max(1, min((int)L.ksteps, (int)(cfg.stage_bytes / bplane)));
+          for (int s0 = 0; s0 < L.ksteps; s0 += kps) {
+            tc::mbar_wait(&bars->w_full[stage], wphase);
             tc::tc_fence_after();
+            const int ne = min(kps, (int)L.ksteps - s0);
+            for (int j = 0; j < ne; ++j) {
+              const int s = s0 + j;
+              if ((s & 3) == 0 && (s >> 2) < L.a_wait) {   // a chunk is 64 columns = 4 K steps
+                const int c = s >> 2;
+                tc::mbar_wait(&bars->a_ready[c], (aph >> c) & 1u); aph ^= (1u << c);
+                tc::tc_fence_after();
+              }
+              const uint32_t ao = abase + (uint32_t)s * 2u * KG, bo = wst0 + (uint32_t)stage * cfg.stage_bytes + (uint32_t)j * bplane;
+              tc::umma_bf16(dcol, tc::make_smem_desc(ao, KG, 128), tc::make_smem_desc(bo, blbo, 128), idesc, s > 0 ? 1u : 0u);
+            }
+            tc::umma_commit(&bars->w_empty[stage]);
+            if (++stage == cfg.nst) { stage = 0; wphase ^= 1u; }
           }
-          tc::mbar_wait(&bars->w_full[stage], wphase);
-          tc::tc_fence_after();
-          const uint32_t ao = abase + (uint32_t)s * 2u * KG, bo = wst0 + (uint32_t)stage * cfg.stage_bytes;
-          const uint64_t ah = tc::make_smem_desc(ao, KG, 128), bh = tc::make_smem_desc(bo, blbo, 128);
-          const uint64_t al = tc::make_smem_desc(ao + aplane, KG, 128), bl = tc::make_smem_desc(bo + bplane, blbo, 128);
-          tc::umma_bf16(dcol, ah, bh, idesc, s > 0 ? 1u : 0u);
-          tc::umma_bf16(dcol, al, bh, idesc, 1u);
-          tc::umma_bf16(dcol, ah, bl, idesc, 1u);
-          tc::umma_commit(&bars->w_empty[stage]);
-          if (++stage == cfg.nst) { stage = 0; wphase ^= 1u; }
+        } else {
+          const uint32_t idesc = tc::make_idesc_bf16(TM, L.n);
+          for (int s = 0; s < L.ksteps; ++s) {
+            if ((s & 3) == 0 && (s >> 2) < L.a_wait) {     // a chunk is 64 columns = 4 K steps
+              const int c = s >> 2;
+              tc::mbar_wait(&bars->a_ready[c], (aph >> c) & 1u); aph ^= (1u << c);
+              tc::tc_fence_after();
+            }
+            tc::mbar_wait(&bars->w_full[stage], wphase);
+            tc::tc_fence_after();
+            const uint32_t ao = abase + (uint32_t)s * 2u * KG, bo = wst0 + (uint32_t)stage * cfg.stage_bytes;
+            const uint64_t ah = tc::make_smem_desc(ao, KG, 128), bh = tc::make_smem_desc(bo, blbo, 128);
+            const uint64_t al = tc::make_smem_desc(ao + aplane, KG, 128), bl = tc::make_smem_desc(bo + bplane, blbo, 128);
+            tc::umma_bf16(dcol, ah, bh, idesc, s > 0 ? 1u : 0u);
+            tc::umma_bf16(dcol, al, bh, idesc, 1u);
+            tc::umma_bf16(dcol, ah, bl, idesc, 1u);
+            tc::umma_commit(&bars->w_empty[stage]);
+            if (++stage == cfg.nst) { stage = 0; wphase ^= 1u; }
+          }
         }
         tc::umma_commit(&bars->d_full[buf]);
       }
@@ -175,6 +217,10 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
       const float4 t0 = *reinterpret_cast<const float4*>(b), t1 = *(reinterpret_cast<const float4*>(b) + 1);
       bv[0] = t0.x; bv[1] = t0.y; bv[2] = t0.z; bv[3] = t0.w; bv[4] = t1.x; bv[5] = t1.y; bv[6] = t1.z; bv[7] = t1.w;
     };
+    // 8 fp32 values -> this thread's K group of row r in an operand plane (fp16: saturating at +-65504)
+    auto put8 = [&](unsigned char* base, uint32_t plane, uint32_t off, const float (&v)[8]) {
+      if constexpr (F16) store8_f16(base, off, v); else store8<NS>(base, plane, off, v);
+    };
     // the accumulator columns [c * 64 + col0, +8) of layer l, this thread's row
     auto ld_acc = [&](int l, int c, uint32_t (&x)[8]) { tc::tmem_ld16x2_8(lane_addr + (uint32_t)(l & 1) * 256u + (uint32_t)(c * CHUNK), x); };
 
@@ -184,10 +230,18 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
       wait_d(l);
       uint32_t xa[8], xb[8];
       auto chunk = [&](int c, const uint32_t (&x)[8]) {
-        float bv[8], v[8];
+        float bv[8];
         ld8(bias + c * CHUNK, bv);
-        act8<NS>(x, bv, v, relu);
-        store8<NS>(A_main, MAIN_PLANE, (uint32_t)((c * CHUNK + col0) / 8) * KG + roff, v);
+        const uint32_t off = (uint32_t)((c * CHUNK + col0) / 8) * KG + roff;
+        if constexpr (F16) {
+          uint32_t o[4];
+          act8_f16(x, bv, o, relu);
+          *reinterpret_cast<uint4*>(A_main + off) = make_uint4(o[0], o[1], o[2], o[3]);
+        } else {
+          float v[8];
+          act8<NS>(x, bv, v, relu);
+          store8<NS>(A_main, MAIN_PLANE, off, v);
+        }
         signal_a(c);
       };
       ld_acc(l, 0, xa);
@@ -204,21 +258,21 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
       bias_done(l);
     };
 
-    // ---------------- prologue: obs (and given actions) -> bf16 operand planes ----------------
+    // ---------------- prologue: obs (and given actions) -> operand planes ----------------
     {
       const float* orow = a.obs + grow * a.obs_ld;
       for (int kg = slot; kg < (int)cfg.obs_kp / 8; kg += SLOTS) {
         float v[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) { int j = kg * 8 + i; v[i] = (valid && j < S) ? __ldg(orow + j) : 0.f; }
-        store8<NS>(A_small, sp, (uint32_t)kg * KG + roff, v);
+        put8(A_small, sp, (uint32_t)kg * KG + roff, v);
       }
       if (!cfg.has_policy && 2 + slot < (int)cfg.sa_kp / 8) {   // [zs | a]: K groups 2 .. sa_kp/8 - 1 hold a, zero-padded
         const float* arow = a.act + grow * a.act_ld;
         float v[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) { int j = slot * 8 + i; v[i] = (valid && j < A) ? __ldg(arow + j) : 0.f; }
-        store8<NS>(A_small, sp, cfg.sa_off + (uint32_t)(2 + slot) * KG + roff, v);
+        put8(A_small, sp, cfg.sa_off + (uint32_t)(2 + slot) * KG + roff, v);
       }
       signal_a(0);
     }
@@ -243,7 +297,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
             v[i] = (j < A) ? tanhf(__uint_as_float(x[i]) + bias[j]) * a.max_action : 0.f;
             if (valid && j < A && a.act_out) a.act_out[grow * A + j] = v[i];
           }
-          store8<NS>(A_small, sp, cfg.sa_off + (uint32_t)(2 + slot) * KG + roff, v);
+          put8(A_small, sp, cfg.sa_off + (uint32_t)(2 + slot) * KG + roff, v);
         }
         release_d(l);
         bias_done(l);
@@ -265,7 +319,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
           tc::tmem_ld_wait();
 #pragma unroll
           for (int j = 0; j < 8; ++j) zs[j] = __uint_as_float(x[j]) + bias[col0 + j];
-          store8<NS>(A_small, sp, cfg.sa_off + (uint32_t)slot * KG + roff, zs);
+          put8(A_small, sp, cfg.sa_off + (uint32_t)slot * KG + roff, zs);
         }
         signal_a(0);
         release_d(l);
@@ -279,10 +333,16 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
           uint32_t x[8];
           ld_acc(l, 0, x);
           tc::tmem_ld_wait();
-          float v[8];
+          if constexpr (F16) {
+            uint32_t o[4];
+            act8_f16(x, bias + col0, o, false);
+            *reinterpret_cast<uint4*>(A_main + (uint32_t)slot * KG + roff) = make_uint4(o[0], o[1], o[2], o[3]);
+          } else {
+            float v[8];
 #pragma unroll
-          for (int i = 0; i < 8; ++i) v[i] = swish_ns<NS>(__uint_as_float(x[i]) + bias[col0 + i]);
-          store8<NS>(A_main, MAIN_PLANE, (uint32_t)slot * KG + roff, v);
+            for (int i = 0; i < 8; ++i) v[i] = swish_ns<NS>(__uint_as_float(x[i]) + bias[col0 + i]);
+            store8<NS>(A_main, MAIN_PLANE, (uint32_t)slot * KG + roff, v);
+          }
         }
         signal_a(0);
         release_d(l);
@@ -299,7 +359,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
           float v[8];
 #pragma unroll
           for (int i = 0; i < 8; ++i) v[i] = zs[i] + (__uint_as_float(x[i]) + bias[col0 + i]);
-          store8<NS>(A_main, MAIN_PLANE, (uint32_t)slot * KG + roff, v);
+          put8(A_main, MAIN_PLANE, (uint32_t)slot * KG + roff, v);
         }
         signal_a(0);
         release_d(l);
@@ -330,7 +390,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
     // As in step_tc.cu: element-wise over the tile's contiguous [64 x S] block of every member, all epilogue threads in
     // flight; per-row sums of squared deviations go through shared memory in member batches, added in a fixed order.
     // Every dynamics MMA has completed, so both operand regions (A_main and the small planes behind it, contiguous) serve
-    // as fp32 scratch: at S = 128 that holds 3 members' squared deviations per batch.
+    // as fp32 scratch: at S = 128 that holds 3 members' squared deviations per batch in bf16x2 and 1 in fp16 (one plane).
     constexpr int NEPI = 32 * EPI_WARPS;
     const int n_el = TM * S;
     float* nobs_s = reinterpret_cast<float*>(A_main);                 // [64*S]    next_obs of the tile
@@ -422,7 +482,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
           }
           v[i] = t;
         }
-        store8<NS>(A_small, sp, (uint32_t)kg * KG + roff, v);
+        put8(A_small, sp, (uint32_t)kg * KG + roff, v);
       }
       tc::fence_proxy_async_smem();
     }
@@ -448,8 +508,18 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
           float bv[8], wv[8];
           ld8(bslot + c * CHUNK + col0, bv);
           ld8(w3 + c * CHUNK + col0, wv);
+          if constexpr (F16) {   // the packed-half swish, unpacked for the fp32 dot
+            uint32_t o[4];
+            float v[8];
+            act8_f16(x, bv, o, false);
 #pragma unroll
-          for (int i = 0; i < 8; ++i) part = fmaf(swish_ns<NS>(__uint_as_float(x[i]) + bv[i]), wv[i], part);
+            for (int i = 0; i < 4; ++i) unpack_f16x2(o[i], v[2 * i], v[2 * i + 1]);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) part = fmaf(v[i], wv[i], part);
+          } else {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) part = fmaf(swish_ns<NS>(__uint_as_float(x[i]) + bv[i]), wv[i], part);
+          }
           if (c + 1 < 4) {
             tc::tmem_ld_wait();
 #pragma unroll
@@ -484,14 +554,15 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
 
 }  // namespace tcw
 
-const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, cudaStream_t st) {
+// fp16 = 1: the single-plane fp16 image and arithmetic (fp16_t64); 0: bf16x2's (bf16x2_wide, bf16x2_t64)
+const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb, const unsigned char* polb, int fp16, cudaStream_t st) {
   if (a.B <= 0) return nullptr;
   const int S = a.S, A = a.A;
   if (S < 2 || S > 128 || A < 1 || A > 32) return "wide tensor-core step kernel supports 2 <= S <= 128, 1 <= A <= 32";
   if (!dynb) return "tensor-core step needs dyn_pack (mobody_dyn_pack)";
   const bool has_policy = polb != nullptr;
   if (has_policy && !a.act_out) return "tensor-core step with a fused policy needs act_out";
-  constexpr int ns = tcw::NS;
+  const int ns = fp16 ? 1 : 2;
   const TcDynLayout DL = tc_dyn_layout(S, A, ns);
   TcSched sc{}; int n = 0;
   auto add = [&](size_t w_off, uint32_t b_off, const TcGeom& g, int region, int a_wait, int kind, int blob) {
@@ -533,18 +604,23 @@ const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb,
   cfg.sa_off = (cfg.obs_kp / 8) * tcw::KG;
   const uint32_t small = cfg.sa_off + (cfg.sa_kp / 8) * tcw::KG, sasb = (cfg.sas_kp / 8) * tcw::KG;
   cfg.small_plane = small > sasb ? small : sasb;
-  cfg.stage_bytes = (uint32_t)ns * 256u * 32u;
+  cfg.stage_bytes = (fp16 ? (uint32_t)tcw::F16_KPS : 1u) * (uint32_t)ns * 256u * 32u;   // 32 KB (fp16) / 16 KB (bf16x2)
   cfg.dyn_bias_base = (uint32_t)DL.bias_base;
   cfg.has_policy = has_policy ? 1 : 0;
   const size_t fixed = (size_t)ns * tcw::MAIN_PLANE + (size_t)ns * cfg.small_plane + (2 * tcw::SLOTS * tcw::TM + tcw::NB * tcw::BSLOT) * sizeof(float) +
                        sizeof(tcw::Bars) + 128;
   const size_t budget = 227 * 1024;
   if (fixed + 4 * cfg.stage_bytes > budget) return "wide tensor-core step kernel: shared memory budget exceeded for this (S, A)";
+  // the statistics phase keeps the tile's next states, member picks and at least one member's squared deviations in the
+  // operand planes (in fp16 at S = 128 that is one member per batch)
+  if ((size_t)ns * (tcw::MAIN_PLANE + cfg.small_plane) / 4 < (size_t)2 * (tcw::TM * S + tcw::TM))
+    return "wide tensor-core step kernel: operand planes too small for the statistics scratch at this (S, A)";
   int nst = (int)((budget - fixed) / cfg.stage_bytes);
   if (nst > tcw::MAX_NST) nst = tcw::MAX_NST;
   cfg.nst = nst;
   const size_t bytes = fixed + (size_t)nst * cfg.stage_bytes;
-  if (cudaFuncSetAttribute(tcw::step_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
+  auto kern = fp16 ? tcw::step_wide_kernel<true> : tcw::step_wide_kernel<false>;
+  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
     return "cudaFuncSetAttribute(step_wide_kernel) failed";
   // every tile streams the whole weight image from L2 (9.2 MB at obs 111 / act 8): keep it persisting, as step_tc.cu does
   static thread_local int limit_dev = -1;
@@ -561,6 +637,6 @@ const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb,
   lc.gridDim = dim3((a.B + tcw::TM - 1) / tcw::TM); lc.blockDim = dim3(32 * (4 * tcw::NG + 2)); lc.dynamicSmemBytes = bytes; lc.stream = st;
   lc.attrs = at; lc.numAttrs = 1;
   const unsigned char* polp = polb ? polb : dynb;
-  if (cudaLaunchKernelEx(&lc, tcw::step_wide_kernel, a, dynb, polp, sc, cfg) != cudaSuccess) return "step_wide_kernel launch failed";
+  if (cudaLaunchKernelEx(&lc, kern, a, dynb, polp, sc, cfg) != cudaSuccess) return "step_wide_kernel launch failed";
   return nullptr;
 }

@@ -66,6 +66,8 @@ def tc_step_supports(S, A, precision):
         return _ffi.TC_WIDE_MIN_S <= S <= _ffi.TC_WIDE_MAX_S and 1 <= A <= _ffi.TC_WIDE_MAX_A
     if precision == "bf16x2_t64":
         return (2 <= S <= _ffi.TC_T64_MAX_S and 1 <= A <= _ffi.TC_T64_MAX_A) and not tc_step_supports(S, A, "bf16x2")
+    if precision == "fp16_t64":
+        return (2 <= S <= _ffi.TC_WIDE_MAX_S and 1 <= A <= _ffi.TC_WIDE_MAX_A) and not tc_step_supports(S, A, "fp16")
     return 2 <= S <= _ffi.TC_MAX_S and 1 <= A <= _ffi.TC_MAX_A and 2 * S + A <= _ffi.TC_MAX_SAS[precision]
 
 
@@ -89,8 +91,8 @@ class MOBODYEnsembleDynamics(DynamicsFitting):
         self.cycle_loss_coef = config.get("cycle_loss_coef", 0) if config else 0
         self.encode_trg_diff = getattr(model, "encode_trg_diff", 0)
         # 'auto' (default): the tcgen05 kernel in its fp32-parity mode (bf16 hi+lo split, inside the 1e-4 bound) whenever
-        # it supports the shapes, else the fp32 CUDA-core kernel (any S <= 128).  "bf16x2_wide" (S > 64) and
-        # "bf16x2_t64" (the S <= 64 shapes bf16x2 refuses) are opt-in.
+        # it supports the shapes, else the fp32 CUDA-core kernel (any S <= 128).  "bf16x2_wide" (S > 64),
+        # "bf16x2_t64" (the S <= 64 shapes bf16x2 refuses) and "fp16_t64" (the shapes fp16 refuses) are opt-in.
         self.precision = precision or (config or {}).get("b200_precision", "auto")
         if self.precision == "auto":
             S_, A_ = getattr(model, "obs_dim", 0), getattr(model, "action_dim", 0)

@@ -1,20 +1,22 @@
 #!/usr/bin/env python
-"""Benchmark of the 64-row tensor-core step mode for Adroit's shapes (bf16x2_t64) against the fp32 CUDA-core kernel;
-prints one JSON line.
+"""Benchmark of the 64-row tensor-core step modes at Adroit's shapes (bf16x2_t64, and fp16_t64: fp16's arithmetic on the
+same tiles) against the fp32 CUDA-core kernel; prints one JSON line.  Speedups are against fp32, and fp16_t64's also
+against bf16x2_t64.
 
   rollout:    pen S45/A24, door S39/A28, relocate S39/A30 and hammer S46/A26, 100 000 start states, T = 1 rollouts
-              (MOBODY.rollout_device: one mobody_rollout call, policy fused), fp32 and bf16x2_t64 alternated in the same
-              run.  pen uses its predicate (part of the rows terminate); door's predicate never fires, and relocate and
+              (MOBODY.rollout_device: one mobody_rollout call, policy fused), fp32, bf16x2_t64 and fp16_t64 alternated in
+              the same run.  pen uses its predicate (part of the rows terminate); door's predicate never fires, and relocate and
               hammer have none in the reference, so they run with the never-firing one.  The start states rotate over a
               pool of buffers larger than the 126 MB L2, so every rollout reads them from HBM; every shape is warmed up first.
   kernel:     the step kernel alone (MOBODYEnsembleDynamics.launch_step, policy fused, CUDA events around many launches,
               same input rotation) and its algorithmic rate, 2 [7 (dyn + rew) + policy] FLOP per transition (SURVEY.md 8d):
               3 861 504 at pen.
-  outputs:    the two modes' T = 1 rollouts of the same seeded start states and Philox key, compared element-wise.
+  outputs:    each tensor-core mode's T = 1 rollout of the same seeded start states and Philox key against fp32's,
+              compared element-wise.
   model_eval: at pen, MOBODY.evaluate_in_model, 100 000 start states, H = 1 000, a predicate that never fires (every step
-              runs at full width), both modes.
+              runs at full width), every mode.
   train:      at pen, MOBODY.train updates/s at batch 128 with penalty_type="par" (one 128-row dynamics step inside every
-              update), both modes alternated.
+              update), every mode alternated.
 The card's name and power limit are read in the same run.
 """
 import argparse
@@ -35,7 +37,8 @@ from helpers import AGENT_CFG, rel_err, rel_err_strict  # noqa: E402
 
 SHAPES = {"pen": (45, 24, "pen-human-v0"), "door": (39, 28, "door-human-v0"), "relocate": (39, 30, "door-human-v0"),
           "hammer": (46, 26, "door-human-v0")}
-MODES = ("fp32", "bf16x2_t64")
+MODES = ("fp32", "bf16x2_t64", "fp16_t64")
+PAIRS = (("bf16x2_t64", "fp32"), ("fp16_t64", "fp32"), ("fp16_t64", "bf16x2_t64"))
 CFG = dict(AGENT_CFG, env_filter=1e9)
 PEN_X = 0.16   # transition3's bias puts the pen's object height (column 26) here: part of the rows fall below 0.075
 
@@ -47,7 +50,7 @@ def flop_per_transition(S, A, H=256, E=7):
 
 
 def make_agent(mb, prec, S, A, task, dev, seed=3, **cfg):
-    """Agent with the reference module's random initialiser (seeded: both modes get the same weights)."""
+    """Agent with the reference module's random initialiser (seeded: every mode gets the same weights)."""
     torch.manual_seed(seed)
     model = mb.MOBODYModule(S, A, 256, 7, 5, device=dev, config={"mopo": 0, "latent_reward": 0})
     with torch.no_grad():
@@ -106,7 +109,7 @@ def bench_shape(mb, env, a, dev):
         ag = ags[p]
         ag.dynamics.launch_step(nxt(), None, wss[p], policy=ag.policy.network, step=0, verify_images=False)
 
-    for p in MODES:                                              # warm-up of every shape and both paths
+    for p in MODES:                                              # warm-up of every shape and every path
         for _ in range(3):
             rollout(p)
         ags[p].dynamics.launch_step(pool[0], None, wss[p], policy=ags[p].policy.network, step=0)
@@ -125,20 +128,24 @@ def bench_shape(mb, env, a, dev):
         res[p] = {"rollout_T1_ms": [round(1e3 * t, 3) for t in ro[p]], "rollout_transitions_per_s": round(B / r, 0),
                   "kernel_ms": [round(1e3 * t, 3) for t in kt[p]], "kernel_transitions_per_s": round(B / k, 0),
                   "kernel_tflops": round(fpt * B / k * 1e-12, 2)}
-    res["speedup_rollout"] = round(res["bf16x2_t64"]["rollout_transitions_per_s"] / res["fp32"]["rollout_transitions_per_s"], 2)
-    res["speedup_kernel"] = round(res["bf16x2_t64"]["kernel_transitions_per_s"] / res["fp32"]["kernel_transitions_per_s"], 2)
-    # the same seeded start states and Philox key through both modes: outputs side by side
+    for p, base in PAIRS:
+        res[f"speedup_rollout_{p}_vs_{base}"] = round(res[p]["rollout_transitions_per_s"] / res[base]["rollout_transitions_per_s"], 2)
+        res[f"speedup_kernel_{p}_vs_{base}"] = round(res[p]["kernel_transitions_per_s"] / res[base]["kernel_transitions_per_s"], 2)
+    # the same seeded start states and Philox key through every mode: outputs side by side
     got = {}
     for p in MODES:
         _, info = ags[p].rollout_device(pool[0], 1, step0=0)
         ws = ags[p]._rollout_workspace(1, B, S, A, 0)
         got[p] = {"next_obs": ws["nexts"][0].cpu().numpy(), "reward": ws["rews"][0].cpu().numpy(),
                   "terminal": ws["terms"][0].cpu().numpy(), "kept": info["kept"]}
-    w, f = got["bf16x2_t64"], got["fp32"]
-    res["outputs"] = {k: {"rel_err": rel_err(w[k], f[k]), "rel_err_strict": rel_err_strict(w[k], f[k])} for k in ("next_obs", "reward")}
-    res["outputs"]["terminal_mismatches"] = int((w["terminal"] != f["terminal"]).sum())
-    res["outputs"]["terminal_rows"] = int(f["terminal"].sum())
-    res["outputs"]["kept"] = [w["kept"], f["kept"]]
+    f = got["fp32"]
+    res["outputs"] = {"terminal_rows_fp32": int(f["terminal"].sum()), "kept_fp32": f["kept"]}
+    for p in MODES[1:]:
+        w = got[p]
+        o = {k: {"rel_err": rel_err(w[k], f[k]), "rel_err_strict": rel_err_strict(w[k], f[k])} for k in ("next_obs", "reward")}
+        o["terminal_mismatches"] = int((w["terminal"] != f["terminal"]).sum())
+        o["kept"] = w["kept"]
+        res["outputs"][f"{p}_vs_fp32"] = o
     del pool, ags, wss
     torch.cuda.empty_cache()
     return res
@@ -154,7 +161,8 @@ def bench_model_eval(mb, a, dev):
         ag.evaluate_in_model(x0, 8, step0=0)
         ts = [timed(lambda: ag.evaluate_in_model(x0, a.horizon, step0=0), 1) for _ in range(2)]
         ev[p] = {"total_s": [round(t, 3) for t in ts], "transitions_per_s": round(B * a.horizon / min(ts), 0)}
-    ev["speedup"] = round(ev["bf16x2_t64"]["transitions_per_s"] / ev["fp32"]["transitions_per_s"], 2)
+    for p, base in PAIRS:
+        ev[f"speedup_{p}_vs_{base}"] = round(ev[p]["transitions_per_s"] / ev[base]["transitions_per_s"], 2)
     ev["workload"] = f"S{S}/A{A}, {B} start states, H={a.horizon}, predicate never fires"
     return ev
 
@@ -181,6 +189,8 @@ def bench_train(mb, a, dev):
         for p in MODES:
             tt[p].append(timed(lambda: ags[p].train(src, tar, 128, None, None), a.train_steps))
     tr = {p: {"updates_per_s": [round(1.0 / t, 0) for t in tt[p]]} for p in MODES}
+    for p, base in PAIRS:
+        tr[f"speedup_{p}_vs_{base}"] = round(float(np.median(tt[base]) / np.median(tt[p])), 2)
     tr["workload"] = f"S{S}/A{A}, batch 128, penalty_type='par' (a 128-row dynamics step in every update)"
     return tr
 

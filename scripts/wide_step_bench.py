@@ -1,15 +1,17 @@
 #!/usr/bin/env python
-"""Benchmark of the wide tensor-core step mode (bf16x2_wide) against the fp32 CUDA-core kernel at Ant's shape; prints one
-JSON line.
+"""Benchmark of the 64-row tensor-core step modes at Ant's shape (bf16x2_wide, and fp16_t64: fp16's arithmetic on the same
+tiles) against the fp32 CUDA-core kernel; prints one JSON line.
 
   rollout:    S111/A8, ant termination, 100 000 start states, T = 1 rollouts (MOBODY.rollout_device: one mobody_rollout
-              call, policy fused), fp32 and bf16x2_wide alternated in the same run.  The start states rotate over a pool
+              call, policy fused), fp32, bf16x2_wide and fp16_t64 alternated in the same run.  Speedups are against fp32,
+              and fp16_t64's also against bf16x2_wide.  The start states rotate over a pool
               of buffers larger than the 126 MB L2, so every rollout reads them from HBM; every shape is warmed up first.
   kernel:     the step kernel alone (MOBODYEnsembleDynamics.launch_step, policy fused, CUDA events around many launches,
               same input rotation) and its algorithmic rate: 4 768 768 FLOP per transition at S111/A8 (SURVEY.md 8d).
   model_eval: MOBODY.evaluate_in_model, 100 000 start states, H = 1 000, a predicate that never fires (every step runs at
-              full width), both modes.
-  outputs:    the two modes' T = 1 rollouts of the same seeded start states and Philox key, compared element-wise.
+              full width), every mode.
+  outputs:    each tensor-core mode's T = 1 rollout of the same seeded start states and Philox key against fp32's,
+              compared element-wise.
 The card's name and power limit are read in the same run.
 """
 import argparse
@@ -27,13 +29,13 @@ import torch  # noqa: E402
 
 S, A = 111, 8
 FLOP_PER_TRANSITION = 4_768_768
-MODES = ("fp32", "bf16x2_wide")
+MODES = ("fp32", "bf16x2_wide", "fp16_t64")
 CFG = dict(max_action=1.0, hidden_sizes=256, gamma=0.99, tau=0.005, actor_lr=3e-4, critic_lr=3e-4, weight=2.5,
            bc_coef=1.0, penalty_type="none", filter_bad_rollout=1, env_filter=1e9)
 
 
 def make_agent(mb, prec, task, dev, seed=3):
-    """Agent with the reference module's random initialiser (seeded: both modes get the same weights); transition3's
+    """Agent with the reference module's random initialiser (seeded: every mode gets the same weights); transition3's
     bias puts x0 at 0.6, inside Ant's healthy range, so part of the rows terminate."""
     torch.manual_seed(seed)
     model = mb.MOBODYModule(S, A, 256, 7, 5, device=dev, config={"mopo": 0, "latent_reward": 0})
@@ -102,7 +104,7 @@ def main():
         ag = ags[p]
         ag.dynamics.launch_step(nxt(), None, wss[p], policy=ag.policy.network, step=0, verify_images=False)
 
-    for p in MODES:                                              # warm-up of every shape and both paths
+    for p in MODES:                                              # warm-up of every shape and every path
         for _ in range(3):
             rollout(p)
         ags[p].dynamics.launch_step(pool[0], None, wss[p], policy=ags[p].policy.network, step=0)
@@ -120,11 +122,12 @@ def main():
         res[p] = {"rollout_T1_ms": [round(1e3 * t, 3) for t in ro[p]], "rollout_transitions_per_s": round(B / r, 0),
                   "kernel_ms": [round(1e3 * t, 3) for t in kt[p]], "kernel_transitions_per_s": round(B / k, 0),
                   "kernel_tflops": round(FLOP_PER_TRANSITION * B / k * 1e-12, 2)}
-    res["speedup_rollout"] = round(res["bf16x2_wide"]["rollout_transitions_per_s"] / res["fp32"]["rollout_transitions_per_s"], 2)
-    res["speedup_kernel"] = round(res["bf16x2_wide"]["kernel_transitions_per_s"] / res["fp32"]["kernel_transitions_per_s"], 2)
+    for p, base in (("bf16x2_wide", "fp32"), ("fp16_t64", "fp32"), ("fp16_t64", "bf16x2_wide")):
+        res[f"speedup_rollout_{p}_vs_{base}"] = round(res[p]["rollout_transitions_per_s"] / res[base]["rollout_transitions_per_s"], 2)
+        res[f"speedup_kernel_{p}_vs_{base}"] = round(res[p]["kernel_transitions_per_s"] / res[base]["kernel_transitions_per_s"], 2)
     out["rollout"] = res
 
-    # ---- the same seeded start states and Philox key through both modes: outputs side by side ----
+    # ---- the same seeded start states and Philox key through every mode: outputs side by side ----
     from helpers import rel_err, rel_err_strict
     got = {}
     for p in MODES:
@@ -132,11 +135,14 @@ def main():
         ws = ags[p]._rollout_workspace(1, B, S, A, 0)
         got[p] = {"next_obs": ws["nexts"][0].cpu().numpy(), "reward": ws["rews"][0].cpu().numpy(),
                   "terminal": ws["terms"][0].cpu().numpy(), "kept": info["kept"]}
-    w, f = got["bf16x2_wide"], got["fp32"]
-    out["outputs"] = {k: {"rel_err": rel_err(w[k], f[k]), "rel_err_strict": rel_err_strict(w[k], f[k])} for k in ("next_obs", "reward")}
-    out["outputs"]["terminal_mismatches"] = int((w["terminal"] != f["terminal"]).sum())
-    out["outputs"]["terminal_rows"] = int(f["terminal"].sum())
-    out["outputs"]["kept"] = [w["kept"], f["kept"]]
+    f = got["fp32"]
+    out["outputs"] = {"terminal_rows_fp32": int(f["terminal"].sum()), "kept_fp32": f["kept"]}
+    for p in MODES[1:]:
+        w = got[p]
+        o = {k: {"rel_err": rel_err(w[k], f[k]), "rel_err_strict": rel_err_strict(w[k], f[k])} for k in ("next_obs", "reward")}
+        o["terminal_mismatches"] = int((w["terminal"] != f["terminal"]).sum())
+        o["kept"] = w["kept"]
+        out["outputs"][f"{p}_vs_fp32"] = o
 
     # ---- evaluate_in_model, H = 1000, every row live throughout ----
     ev = {}
@@ -145,7 +151,8 @@ def main():
         ag.evaluate_in_model(pool[0], 8, step0=0)
         ts = [timed(lambda: ag.evaluate_in_model(pool[0], a.horizon, step0=0), 1) for _ in range(2)]
         ev[p] = {"total_s": [round(t, 3) for t in ts], "transitions_per_s": round(B * a.horizon / min(ts), 0)}
-    ev["speedup"] = round(ev["bf16x2_wide"]["transitions_per_s"] / ev["fp32"]["transitions_per_s"], 2)
+    for p, base in (("bf16x2_wide", "fp32"), ("fp16_t64", "fp32"), ("fp16_t64", "bf16x2_wide")):
+        ev[f"speedup_{p}_vs_{base}"] = round(ev[p]["transitions_per_s"] / ev[base]["transitions_per_s"], 2)
     out["model_eval"] = dict(ev, workload=f"S{S}/A{A}, {B} start states, H={a.horizon}, predicate never fires")
     print(json.dumps(out))
 
