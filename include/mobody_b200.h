@@ -44,6 +44,8 @@ extern "C" {
 #define MOBODY_PREC_FP32 0    /* CUDA-core fp32 FMA; bit-faithful op order per row                  */
 #define MOBODY_PREC_BF16X2 1  /* tcgen05 bf16 hi+lo split (3 MMAs), ~1e-5 rel: inside the 1e-4 bound */
 #define MOBODY_PREC_BF16 2    /* tcgen05 single-pass bf16: DIAGNOSTIC ONLY, outside the stated bounds (measured 1.6e-2); the Python mirror does not offer it */
+                              /* takes S <= 63 where two row tiles do not fit (2S+A > 112): the one-tile fallback has no
+                                 statistics scratch at S = 64 and reports MOBODY_ERR_UNSUPPORTED */
 #define MOBODY_PREC_FP16 3    /* tcgen05 single-pass fp16, two tiles per SM, packed-half epilogue; measured <= 4.6e-3, inside the stated looser bound 5e-3; |activations| < 6e4 */
 #define MOBODY_PREC_BF16X2_WIDE 4  /* bf16x2's arithmetic on 64-row tiles for wide observations: MOBODY_TC_WIDE_MIN_S <= S <= MOBODY_TC_WIDE_MAX_S,
                                       A <= MOBODY_TC_WIDE_MAX_A (Ant's 111 / 8); packed images are bf16x2's */

@@ -88,6 +88,11 @@ static_assert(sizeof(mobody_dyn_params) == sizeof(DynPtrs), "DynPtrs layout");
 static_assert(sizeof(mobody_mlp_params) == sizeof(MlpPtrs), "MlpPtrs layout");
 static_assert(MOBODY_N_DYN_LAYERS == L_COUNT, "layer count");
 
+// operand planes of a precision mode's packed images: 2 (bf16 hi + lo), 1 (bf16 or fp16), 0 for fp32 (no image)
+static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE || precision == MOBODY_PREC_BF16X2_T64) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16 || precision == MOBODY_PREC_FP16_T64) ? 1 : 0; }
+// the single fp16 plane of the fp16 modes (one image format for MOBODY_PREC_FP16 and MOBODY_PREC_FP16_T64)
+static int is_fp16(int precision) { return precision == MOBODY_PREC_FP16 || precision == MOBODY_PREC_FP16_T64; }
+
 extern "C" {
 
 int mobody_abi_version(void) { return MOBODY_ABI_VERSION; }
@@ -134,12 +139,14 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
     if (!dp.w[i] || !dp.b[i]) return fail(MOBODY_ERR_ARG, "mobody_step: null dynamics parameter pointer");
   MlpPtrs pol; const MlpPtrs* polp = nullptr;
   if (d->policy) { memcpy(&pol, d->policy, sizeof(pol)); polp = &pol; }
+  if (nsplit_of(d->precision)) {   // every tensor-core mode runs on the packed images
+    if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
+    if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
+  }
   const char* err = nullptr;
   switch (d->precision) {
     case MOBODY_PREC_FP32: err = mb_simt_step_launch(a, dp, polp, (cudaStream_t)stream); break;
     case MOBODY_PREC_FP16: {
-      if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
-      if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
       bool launched = false;
       err = mb_tc_duo_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr, 1,
                                   (cudaStream_t)stream, &launched);
@@ -147,8 +154,6 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
     } break;
     case MOBODY_PREC_BF16X2:
     case MOBODY_PREC_BF16:
-      if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
-      if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
       {   // one CTA per 128-row tile; the single bf16 plane (diagnostic mode) fits two row tiles per SM -> two-tiles-in-flight kernel
         if (d->precision == MOBODY_PREC_BF16) {
           bool launched = false;
@@ -164,8 +169,6 @@ int mobody_step(const mobody_step_desc* d, void* stream) {
     case MOBODY_PREC_BF16X2_WIDE:
     case MOBODY_PREC_BF16X2_T64:
     case MOBODY_PREC_FP16_T64:
-      if (!d->dyn_pack) return fail(MOBODY_ERR_ARG, "mobody_step: tensor-core precision needs dyn_pack (mobody_dyn_pack)");
-      if (d->policy && !d->policy_pack) return fail(MOBODY_ERR_ARG, "mobody_step: fused policy needs policy_pack (mobody_mlp_pack)");
       err = mb_tc_wide_step_launch(a, (const unsigned char*)d->dyn_pack, d->policy ? (const unsigned char*)d->policy_pack : nullptr,
                                    d->precision == MOBODY_PREC_FP16_T64, (cudaStream_t)stream);
       break;
@@ -530,10 +533,6 @@ int mobody_dara_relabel(float* rows, long long n, int S, int A, int row_width, c
   if (err) return fail(MOBODY_ERR_UNSUPPORTED, err);
   return check_launch("mobody_dara_relabel");
 }
-
-static int nsplit_of(int precision) { return (precision == MOBODY_PREC_BF16X2 || precision == MOBODY_PREC_BF16X2_WIDE || precision == MOBODY_PREC_BF16X2_T64) ? 2 : (precision == MOBODY_PREC_BF16 || precision == MOBODY_PREC_FP16 || precision == MOBODY_PREC_FP16_T64) ? 1 : 0; }
-// the single fp16 plane of the fp16 modes (one image format for MOBODY_PREC_FP16 and MOBODY_PREC_FP16_T64)
-static int is_fp16(int precision) { return precision == MOBODY_PREC_FP16 || precision == MOBODY_PREC_FP16_T64; }
 
 long long mobody_dyn_pack_bytes(int S, int A, int precision) {
   int ns = nsplit_of(precision);

@@ -10,23 +10,18 @@
 // cluster), so the hand-offs cost what they cost in step_tc.cu.  The bf16 hi+lo mode does not fit (2 x 128 KB of A).
 //
 // Units are processed in (layer, tile) order by the producer warp (weights: one K step per ring stage, streamed once
-// per unit; biases: once per layer), the MMA warp and the 16 epilogue warps.
-#include "common.cuh"
-#include "philox.cuh"
-#include "term.cuh"
-#include "tc_prims.cuh"
-#include "tc_layout.h"
-#include "tc_epi.cuh"
+// per unit; biases: once per layer), the MMA warp and the 16 epilogue warps.  The layer schedule, the bias staging and each
+// tile's statistics phase (ensemble statistics, noise, pick, penalty, termination, the reward head's operand) and final
+// write are the code of tc_step.cuh, shared with step_tc.cu and step_wide.cu.
+#include "tc_step.cuh"
 #include <stdlib.h>
 
 namespace tcd {
-using namespace tce;
+using namespace tst;
 
 constexpr int TM = 128;
 constexpr uint32_t MAIN_PLANE = 65536;     // 128 rows x 256 k x bf16
 constexpr int MAX_NST = 12;
-constexpr int NB = 4;                      // bias ring slots (one layer's bias each, shared by both tiles)
-constexpr int BSLOT = 528;                 // 256 bias + reward_model3 vector (272)
 constexpr int EPI_WARPS = 16, PROD_WARP = 16, MMA_WARP = 17, NTHREADS = 32 * 18;
 constexpr int NS = 1;                      // single bf16 plane
 
@@ -88,14 +83,7 @@ step_duo_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const 
         const TcLayer L = sched.L[li];
         const unsigned char* src = (L.blob ? polb : dynb) + L.w_off;
         const uint32_t bytes = (uint32_t)L.n * 32u;
-        {
-          const int slot = li & (NB - 1);
-          const float* bsrc = reinterpret_cast<const float*>(L.blob ? polb + cfg.pol_bias_base : dynb + cfg.dyn_bias_base) + L.b_off;
-          const uint32_t bb = (L.kind == EPI_REWARD ? (uint32_t)BSLOT : (uint32_t)L.n) * 4u;
-          tc::mbar_wait(&bars->b_empty[slot], (uint32_t)(((li / NB) & 1) ^ 1));
-          tc::mbar_arrive_expect_tx(&bars->b_full[slot], bb);
-          tc::bulk_g2s(bias_s + slot * BSLOT, bsrc, bb, &bars->b_full[slot]);
-        }
+        tc_stage_bias(li, L, dynb, polb, cfg.dyn_bias_base, cfg.pol_bias_base, bias_s, bars->b_full, bars->b_empty);
         // a unit's MMAs wait for the tile's whole previous epilogue, so nothing hides the ring's load -> MMA -> commit ->
         // reload round trip here: narrow layers put as many K steps as fit into one stage (one copy, one round trip)
         const int kps = max(1, min((int)L.ksteps, (int)(cfg.stage_bytes / bytes)));
@@ -254,106 +242,18 @@ step_duo_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const 
       signal_a(u);
     }
 
-    // ---------------- ensemble statistics, noise, pick, penalty, termination, reward-head operand (tile u) ----------------
+    // ---------------- ensemble statistics, noise, pick, penalty, termination, reward-head operand (tile u; tc_step.cuh) ----------------
+    // The tile's A_main serves as fp32 scratch (every dynamics MMA of the tile has completed); [s | a | s'] aliases its
+    // obs / sa planes.
     auto stats = [&](int u) {
-      constexpr int NEPI = 32 * EPI_WARPS;
-      const size_t g0 = row0_of(u);
-      const int n_el = TM * S;
-      float* nobs_s = reinterpret_cast<float*>(main_of(u));              // [128*S]  next_obs of the tile
-      int* member_s = reinterpret_cast<int*>(nobs_s + n_el);             // [128]    picked member per row
-      float* dsq_s = reinterpret_cast<float*>(member_s + TM) + TM;       // [batch][128*S] squared deviations
-      const int scratch_floats = (int)(MAIN_PLANE / 4) - n_el - 2 * TM;
-      const int mbatch = min(MB_E, scratch_floats / n_el);
-      float* redu = red + u * 4 * TM;
-      const size_t grow = g0 + r;
+      float* nobs_s = reinterpret_cast<float*>(main_of(u));
+      const size_t grow = row0_of(u) + r;
       const bool valid = grow < (size_t)live;
-      if (tid < TM) {
-        int mem = 0;
-        if (g0 + tid < (size_t)live) {
-          const size_t gr = g0 + tid;
-          const unsigned long long gid = a.row_ids ? (unsigned long long)a.row_ids[gr] : a.row0 + gr;
-          mem = a.idx ? (int)a.idx[gr] : (int)a.elites[philox_elite_slot(a.seed, a.step, gid, a.n_elites)];
-        }
-        member_s[tid] = mem;
-      }
-      epi_bar<EPI_WARPS>();   // every mean column of this tile has been written; member_s is visible
-      float row_pmax = 0.f;
-      for (int e0 = 0; e0 < MB_E; e0 += mbatch) {
-#pragma unroll 1   // one code path for every element: a row's result must not depend on its position in the tile
-        for (int i = tid; i < n_el; i += NEPI) {
-          const int rr = i / S, j = i - rr * S;
-          const size_t gr = g0 + rr;
-          if (gr < (size_t)live) {
-            float mv[MB_E], sum = 0.f;
-#pragma unroll
-            for (int e = 0; e < MB_E; ++e) { mv[e] = a.mean[((size_t)e * B + g0) * S + i]; sum += mv[e]; }
-            const float mbar = sum / (float)MB_E;
-            const int member = member_s[rr];
-            float ss = 0.f, mk = 0.f;
-#pragma unroll
-            for (int e = 0; e < MB_E; ++e) {
-              const float d = mv[e] - mbar, dd = __fmul_rn(d, d);    // explicit roundings (no contraction choices)
-              ss = __fadd_rn(ss, dd);
-              if (e >= e0 && e < e0 + mbatch) dsq_s[(e - e0) * n_el + i] = (j < S - 1) ? dd : 0.f;   // quirk: last dim excluded (:246)
-              if (e == member) mk = mv[e];
-            }
-            if (e0 == 0) {
-              const float sd = sqrtf(ss / (float)(MB_E - 1));
-              float ep;
-              if (a.eps) ep = a.eps[((size_t)member * B + gr) * S + j];
-              else {
-                const unsigned long long gid = a.row_ids ? (unsigned long long)a.row_ids[gr] : a.row0 + gr;
-                ep = philox_normal1(philox_noise_block(a.seed, a.step, gid, (unsigned)(j >> 2)), j & 3);
-              }
-              const float nv = __fmaf_rn(ep, sd, mk);
-              a.next_obs[g0 * S + i] = nv;
-              nobs_s[i] = nv;
-            }
-          }
-        }
-        epi_bar<EPI_WARPS>();
-        if (valid) {   // (row, member) sums in a fixed order; group g takes members g, g + 4, ... of its row
-          for (int e = group; e < mbatch && e0 + e < MB_E; e += 4) {
-            const float* p = dsq_s + e * n_el + r * S;
-            float v0 = 0.f, v1 = 0.f;
-            int j = 0;
-            for (; j + 2 <= S - 1; j += 2) { v0 += p[j]; v1 += p[j + 1]; }
-            if (j < S - 1) v0 += p[j];
-            row_pmax = fmaxf(row_pmax, sqrtf(v0 + v1));
-          }
-        }
-        if (e0 + mbatch < MB_E) epi_bar<EPI_WARPS>();   // dsq_s is rewritten by the next batch
-      }
-      redu[group * TM + r] = row_pmax;
-      if (group == 0 && valid) a.terminal[grow] = (unsigned char)mb_terminal(a.term_kind, nobs_s + r * S, S);
-      epi_bar<EPI_WARPS>();
-      if (group == 0 && valid) {
-        float pm = 0.f;
-#pragma unroll
-        for (int g2 = 0; g2 < 4; ++g2) pm = fmaxf(pm, redu[g2 * TM + r]);
-        pen[u] = pm;
-      }
-      {   // sas = [obs, act, next_obs, 0-pad] operand of the reward head (mobody_module.py:296); aliases obs/sa planes
-        const float* actp = cfg.has_policy ? a.act_out : a.act;
-        const int act_ld = cfg.has_policy ? A : a.act_ld;
-        unsigned char* As = small_of(u);
-        for (int kg = group; kg < (int)cfg.sas_kp / 8; kg += 4) {
-          float v[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int k = kg * 8 + i;
-            float t = 0.f;
-            if (valid) {
-              if (k < S) t = __ldg(a.obs + grow * a.obs_ld + k);
-              else if (k < S + A) t = actp[grow * act_ld + (k - S)];
-              else if (k < 2 * S + A) t = nobs_s[r * S + (k - S - A)];
-            }
-            v[i] = t;
-          }
-          put8(As, (uint32_t)kg * 2048u + (uint32_t)r * 16u, v);
-        }
-        tc::fence_proxy_async_smem();
-      }
+      const float row_pmax = tc_stats<TM, EPI_WARPS, 4>(a, S, B, row0_of(u), live, r, group, valid, nobs_s, MAIN_PLANE, [](int) {});
+      pen[u] = tc_penalty_terminal<TM, EPI_WARPS, 4>(a, S, row_pmax, red + u * 4 * TM, r, group, valid, grow, nobs_s, [](int) {});
+      unsigned char* As = small_of(u);
+      tc_sas_operand<4>(a, S, A, cfg.has_policy, (int)cfg.sas_kp, r, group, valid, grow, nobs_s,
+                        [&](int kg, const float (&v)[8]) { put8(As, (uint32_t)kg * 2048u + (uint32_t)r * 16u, v); });
       epi_bar<EPI_WARPS>();   // every sas plane is written (and nobs_s is no longer needed) before the operand is announced
       __syncwarp();
       if (lane == 0) tc::mbar_arrive(&bars->a_ready[u]);
@@ -498,12 +398,7 @@ step_duo_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const 
     if (group == 0) {
       for (int u = 0; u < 2; ++u) {
         const size_t grow = row0_of(u) + r;
-        if (grow < (size_t)live) {
-          const float raw = racc[u] / (float)MB_E;
-          if (a.raw_reward) a.raw_reward[grow] = raw;
-          a.penalty[grow] = pen[u];
-          a.reward[grow] = (a.coef != 0.f && a.use_penalty) ? raw - a.coef * pen[u] : raw;     // :261-263
-        }
+        if (grow < (size_t)live) tc_write_reward(a, grow, racc[u], pen[u]);
       }
     }
   }
@@ -526,49 +421,17 @@ const char* mb_tc_duo_step_launch(const StepArgs& a, const unsigned char* dynb, 
   if (!dynb) return "tensor-core step needs dyn_pack (mobody_dyn_pack)";
   const bool has_policy = polb != nullptr;
   if (has_policy && !a.act_out) return "tensor-core step with a fused policy needs act_out";
-  const TcDynLayout DL = tc_dyn_layout(S, A, ns);
-  TcSched sc{}; int n = 0;
-  auto add = [&](size_t w_off, uint32_t b_off, const TcGeom& g, int region, int a_wait, int kind, int blob) {
-    TcLayer& L = sc.L[n++];
-    L.w_off = (uint32_t)w_off; L.b_off = b_off; L.ksteps = (uint16_t)(g.Kp / 16); L.n = (uint16_t)g.Np;
-    L.a_region = (uint8_t)region; L.a_wait = (uint8_t)a_wait; L.kind = (uint8_t)kind; L.blob = (uint8_t)blob;
-  };
   tcd::Cfg cfg{};
-  // a_wait = 1: the layer's A operand is announced by the preceding epilogue / prologue / statistics phase of the tile
-  if (has_policy) {
-    const TcMlpLayout PL = tc_mlp_layout(S, A, ns);
-    add(PL.w_off[0], PL.b_off[0], PL.g[0], REG_OBS, 1, EPI_RELU256, 1);
-    add(PL.w_off[1], PL.b_off[1], PL.g[1], REG_MAIN, 1, EPI_RELU256, 1);
-    add(PL.w_off[2], PL.b_off[2], PL.g[2], REG_MAIN, 1, EPI_ACTION, 1);
-    cfg.pol_bias_base = (uint32_t)PL.bias_base;
-  }
-  sc.first_dyn = n; cfg.first_dyn = n;
-  const int za1 = a.use_trg ? PK_ZATRG1 : PK_ZASRC1, za2 = a.use_trg ? PK_ZATRG2 : PK_ZASRC2;
-  const int sas_kp = tc_rup16(2 * S + A);
-  for (int e = 0; e < MB_E; ++e) {
-    const size_t wb = (size_t)e * DL.member_w_bytes; const uint32_t bb = (uint32_t)e * DL.member_b_floats;
-    auto lay = [&](int pk, int region, int a_wait, int kind) { add(wb + DL.w_off[pk], bb + DL.b_off[pk], tc_dyn_geom(pk, S, A), region, a_wait, kind, 0); };
-    lay(PK_ZS1, REG_OBS, (e == 0 && !has_policy) ? 1 : 0, EPI_SWISH256);
-    lay(PK_ZS2, REG_MAIN, 1, EPI_SWISH256);
-    lay(PK_ZS3, REG_MAIN, 1, EPI_ZS);
-    lay(za1, REG_SA, 1, EPI_G);
-    lay(za2, REG_MAIN, 1, EPI_Z);
-    lay(PK_T1, REG_MAIN, 1, EPI_SWISH256);
-    lay(PK_T2, REG_MAIN, 1, EPI_SWISH256);
-    lay(PK_T3, REG_MAIN, 1, EPI_MEAN);
-  }
-  for (int e = 0; e < MB_E; ++e) {
-    const size_t wb = (size_t)e * DL.member_w_bytes; const uint32_t bb = (uint32_t)e * DL.member_b_floats;
-    add(wb + DL.w_off[PK_R1], bb + DL.b_off[PK_R1], tc_dyn_geom(PK_R1, S, A), REG_SAS, e == 0 ? 1 : 0, EPI_SWISH256, 0);
-    add(wb + DL.w_off[PK_R2], bb + DL.b_off[PK_R2], tc_dyn_geom(PK_R2, S, A), REG_MAIN, 1, EPI_REWARD, 0);
-  }
-  sc.n_layers = n;
-  cfg.obs_kp = (uint32_t)tc_rup16(S); cfg.sas_kp = (uint32_t)sas_kp;
+  // a_wait = 1: a layer's whole A operand is announced at once, by the tile's preceding epilogue / prologue / statistics phase
+  const TcSched sc = tst::tc_step_sched(a, ns, has_policy, 256, &cfg.pol_bias_base);
+  const TcDynLayout DL = tc_dyn_layout(S, A, ns);
+  cfg.obs_kp = (uint32_t)tc_rup16(S); cfg.sas_kp = (uint32_t)tc_rup16(2 * S + A);
   cfg.sa_off = (cfg.obs_kp / 8) * 2048u;
   uint32_t small = cfg.sa_off + 4 * 2048u, sasb = (cfg.sas_kp / 8) * 2048u;
   cfg.small_plane = small > sasb ? small : sasb;
   cfg.dyn_bias_base = (uint32_t)DL.bias_base;
   cfg.has_policy = has_policy ? 1 : 0;
+  cfg.first_dyn = sc.first_dyn;
   cfg.trace = mb_tc_get_trace();
   const size_t fixed = 2 * ((size_t)tcd::MAIN_PLANE + (size_t)cfg.small_plane) +
                        (2 * 4 * tcd::TM + tcd::NB * tcd::BSLOT) * sizeof(float) + sizeof(tcd::Bars) + 128;

@@ -17,36 +17,31 @@
 //    place in SMEM.  All groups work on the same 32-column chunk (8 columns per warp), so chunks are
 //    announced in order (one mbarrier per chunk) and the next layer's MMAs trail the epilogue by one chunk:
 //    tensor pipe and epilogue overlap inside a single row tile.
-//  Sibling: step_duo.cu (two tiles in flight per CTA; the single-pass fp16 mode runs there).  The CTA-pair experiment of
-//  round 1 (cta_group::2; correct, 3x slower) lives in scripts/experimental/ and is not part of the library; DESIGN.md 4.1.
+//  Siblings: step_duo.cu (two tiles in flight per CTA; the single-pass fp16 mode runs there) and step_wide.cu (64-row
+//  tiles).  The three share tc_step.cuh: the layer schedule, the launch, the bias staging and everything after the last
+//  dynamics GEMM (ensemble statistics, noise, pick, penalty, termination, the reward head's operand, the final write).
+//  The CTA-pair experiment of round 1 (cta_group::2; correct, 3x slower) lives in scripts/experimental/ and is not part of
+//  the library; DESIGN.md 4.1.
 //
 // Precision: NS = 2 -> bf16 hi+lo split of both operands, 3 MMAs per K step (hi*hi + lo*hi + hi*lo), ~2^-16 per
 // product: inside the 1e-4 bound (the default mode).  NS = 1 -> single bf16 pass (bound 2e-2; used when the two-tile
 // kernel does not fit).  Biases come from a shared-memory ring staged by the producer warp; swish
 // layers are packed pre-scaled (tc_layout.h: tc_swish_scales) so the epilogue needs no multiply before the SFU op.
-#include "common.cuh"
-#include "philox.cuh"
-#include "term.cuh"
-#include "tc_prims.cuh"
-#include "tc_layout.h"
-#include "tc_epi.cuh"
+#include "tc_step.cuh"
 #include <cuda_fp16.h>
 
 namespace tcs {
-using namespace tce;
-
+using namespace tst;
 
 constexpr int TM = 128;
 constexpr int NG = 4;                    // epilogue groups of 4 warps (one warp per TMEM lane quadrant)
 constexpr uint32_t MAIN_PLANE = 65536;   // 128 rows x 256 k x bf16
 constexpr int MAX_NST = 12;
-constexpr int NB = 4;                    // bias ring slots (one layer's bias each)
-constexpr int BSLOT = 528;               // floats per slot: 256 bias + reward_model3 vector (272) behind reward_model2's bias
 
 struct Cfg {
   int nst;
   uint32_t stage_bytes, small_plane, sa_off, obs_kp, sas_kp;
-  uint32_t dyn_bias_base, pol_bias_base, member_b_floats, r3_b_off;
+  uint32_t dyn_bias_base, pol_bias_base;
   int has_policy;
   long long* trace;     // debug: per-layer clock64 timestamps of CTA 0 ([layer][8]); nullptr in production
 };
@@ -101,14 +96,7 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
         const TcLayer L = sched.L[li];
         const unsigned char* src = (L.blob ? polb : dynb) + L.w_off;
         const uint32_t bytes = (uint32_t)NS * L.n * 32u;
-        {   // this layer's bias (and reward_model3's vector right behind reward_model2's bias) -> bias ring slot li % NB
-          const int slot = li & (NB - 1);
-          const float* bsrc = reinterpret_cast<const float*>(L.blob ? polb + cfg.pol_bias_base : dynb + cfg.dyn_bias_base) + L.b_off;
-          const uint32_t bb = (L.kind == EPI_REWARD ? (uint32_t)BSLOT : (uint32_t)L.n) * 4u;
-          tc::mbar_wait(&bars->b_empty[slot], (uint32_t)(((li / NB) & 1) ^ 1));
-          tc::mbar_arrive_expect_tx(&bars->b_full[slot], bb);
-          tc::bulk_g2s(bias_s + slot * BSLOT, bsrc, bb, &bars->b_full[slot]);
-        }
+        tc_stage_bias(li, L, dynb, polb, cfg.dyn_bias_base, cfg.pol_bias_base, bias_s, bars->b_full, bars->b_empty);
         for (int s = 0; s < L.ksteps; ++s) {
           tc::mbar_wait(&bars->w_empty[stage], phase ^ 1u);
           tc::mbar_arrive_expect_tx(&bars->w_full[stage], bytes);
@@ -120,7 +108,7 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
   } else if (warp == MMA_WARP) {
     // ================= MMA issuer =================
     if (tc::elect_one()) {
-      int stage = 0; uint32_t wphase = 0, aph = 0;
+      uint32_t aph = 0; int stage = 0; uint32_t wphase = 0;
       const uint32_t small0 = tc::smem_u32(A_small), main0 = tc::smem_u32(A_main), wst0 = tc::smem_u32(wst);
       for (int li = 0; li < sched.n_layers; ++li) {
         const TcLayer L = sched.L[li];
@@ -369,115 +357,22 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
       }
     }
 
-    // ---------------- ensemble statistics, noise, pick, penalty, termination ----------------
-    // All epilogue warps take part: the NG threads of a row split its dims in blocks of 4 (block b -> group b % NG).
-    // A_main is free here (every dynamics MMA has completed) and serves as fp32 scratch.
-    // Element-wise over the tile's contiguous [128 x S] block of every member (coalesced loads; there is no
-    // L1 to speak of next to ~227 KB of shared memory), all epilogue threads in flight at once.  Per-row sums of
-    // squared deviations go through shared memory in member batches and are added in a fixed order (deterministic).
-    constexpr int NEPI = 32 * EPI_WARPS;
-    const int n_el = TM * S;
-    float* nobs_s = reinterpret_cast<float*>(A_main);                 // [128*S]   next_obs of the tile
-    int* member_s = reinterpret_cast<int*>(nobs_s + n_el);            // [128]     picked member per row
-    float* dsq_s = reinterpret_cast<float*>(member_s + TM) + TM;      // [batch][128*S] squared deviations
-    const int scratch_floats = (int)(NS * MAIN_PLANE / 4) - n_el - 2 * TM;
-    const int mbatch = min(MB_E, scratch_floats / n_el);
-    const int etid = tid;                                             // epilogue threads are 0 .. NEPI-1
-    if (tracer && group == 0) cfg.trace[79 * 8 + 0] = clock64();
-    if (etid < TM) {
-      int mem = 0;
-      if (row0 + etid < live) {
-        const size_t gr = (size_t)row0 + etid;
-        const unsigned long long gid = a.row_ids ? (unsigned long long)a.row_ids[gr] : a.row0 + gr;
-        mem = a.idx ? (int)a.idx[gr] : (int)a.elites[philox_elite_slot(a.seed, a.step, gid, a.n_elites)];
-      }
-      member_s[etid] = mem;
-    }
-    epi_bar<EPI_WARPS>();   // every mean column of this tile has been written; member_s is visible
-    if (tracer && group == 0) cfg.trace[79 * 8 + 1] = clock64();
-    float row_pmax = 0.f;
-    for (int e0 = 0; e0 < MB_E; e0 += mbatch) {
-#pragma unroll 1   // one code path for every element: a row's result must not depend on its position in the tile
-      for (int i = etid; i < n_el; i += NEPI) {
-        const int rr = i / S, j = i - rr * S;
-        const size_t gr = (size_t)row0 + rr;
-        if (row0 + rr < live) {
-          float mv[MB_E], sum = 0.f;
-#pragma unroll
-          for (int e = 0; e < MB_E; ++e) { mv[e] = a.mean[((size_t)e * B + row0) * S + i]; sum += mv[e]; }
-          const float mbar = sum / (float)MB_E;
-          const int member = member_s[rr];
-          float ss = 0.f, mk = 0.f;
-#pragma unroll
-          for (int e = 0; e < MB_E; ++e) {
-            const float d = mv[e] - mbar, dd = __fmul_rn(d, d);    // explicit roundings (no contraction choices)
-            ss = __fadd_rn(ss, dd);
-            if (e >= e0 && e < e0 + mbatch) dsq_s[(e - e0) * n_el + i] = (j < S - 1) ? dd : 0.f;   // quirk: last dim excluded (:246)
-            if (e == member) mk = mv[e];
-          }
-          if (e0 == 0) {
-            const float sd = sqrtf(ss / (float)(MB_E - 1));
-            float ep;
-            if (a.eps) ep = a.eps[((size_t)member * B + gr) * S + j];
-            else {
-              const unsigned long long gid = a.row_ids ? (unsigned long long)a.row_ids[gr] : a.row0 + gr;
-              ep = philox_normal1(philox_noise_block(a.seed, a.step, gid, (unsigned)(j >> 2)), j & 3);
-            }
-            const float nv = __fmaf_rn(ep, sd, mk);
-            a.next_obs[(size_t)row0 * S + i] = nv;
-            nobs_s[i] = nv;
-          }
-        }
-      }
-      epi_bar<EPI_WARPS>();
-      // (row, member) sums in a fixed order; group g takes members g, g+NG, ... of its row r
-      if (valid) {
-        for (int e = group; e < mbatch && e0 + e < MB_E; e += NG) {
-          const float* p = dsq_s + e * n_el + r * S;
-          float v0 = 0.f, v1 = 0.f;
-          int j = 0;
-          for (; j + 2 <= S - 1; j += 2) { v0 += p[j]; v1 += p[j + 1]; }
-          if (j < S - 1) v0 += p[j];
-          row_pmax = fmaxf(row_pmax, sqrtf(v0 + v1));
-        }
-      }
-      if (e0 + mbatch < MB_E) epi_bar<EPI_WARPS>();   // dsq_s is rewritten by the next batch
-    }
-    if (tracer && group == 0) cfg.trace[79 * 8 + 2] = clock64();
-    red[group * 128 + r] = row_pmax;
-    if (group == 0 && valid) a.terminal[grow] = (unsigned char)mb_terminal(a.term_kind, nobs_s + r * S, S);
-    epi_bar<EPI_WARPS>();
-    if (tracer && group == 0) cfg.trace[79 * 8 + 3] = clock64();
-    if (group == 0 && valid) {
-      float pm = 0.f;
-#pragma unroll
-      for (int g2 = 0; g2 < NG; ++g2) pm = fmaxf(pm, red[g2 * 128 + r]);
-      pen = pm;
-    }
-    if (tracer && group == 0) cfg.trace[79 * 8 + 4] = clock64();
-    {   // sas = [obs, act, next_obs, 0-pad] operand of the reward head (mobody_module.py:296); aliases obs/sa planes
-      const float* actp = cfg.has_policy ? a.act_out : a.act;
-      const int act_ld = cfg.has_policy ? A : a.act_ld;
-      for (int kg = group; kg < (int)cfg.sas_kp / 8; kg += NG) {
-        float v[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int k = kg * 8 + i;
-          float t = 0.f;
-          if (valid) {
-            if (k < S) t = __ldg(a.obs + grow * a.obs_ld + k);
-            else if (k < S + A) t = actp[grow * act_ld + (k - S)];
-            else if (k < 2 * S + A) t = nobs_s[r * S + (k - S - A)];
-          }
-          v[i] = t;
-        }
-        store8<NS>(A_small, sp, (uint32_t)kg * 2048u + (uint32_t)r * 16u, v);
-      }
-      tc::fence_proxy_async_smem();
-    }
-    if (tracer && group == 0) cfg.trace[79 * 8 + 5] = clock64();
+    // ---------------- ensemble statistics, noise, pick, penalty, termination (tc_step.cuh) ----------------
+    // All epilogue warps take part: the NG threads of a row split its member sums (slot = group).  A_main is free here
+    // (every dynamics MMA has completed) and serves as fp32 scratch.
+    float* nobs_s = reinterpret_cast<float*>(A_main);
+    auto stamp = [&](int k) { if (tracer && group == 0) cfg.trace[79 * 8 + k] = clock64(); };   // trace stamps of the phase
+    const float row_pmax = tc_stats<TM, EPI_WARPS, NG>(a, S, B, row0, live, r, group, valid, nobs_s, NS * MAIN_PLANE,
+                                                       stamp);
+    stamp(2);
+    pen = tc_penalty_terminal<TM, EPI_WARPS, NG>(a, S, row_pmax, red, r, group, valid, grow, nobs_s, stamp);
+    stamp(4);
+    // [s | a | s'] aliases the obs / sa planes
+    tc_sas_operand<NG>(a, S, A, cfg.has_policy, (int)cfg.sas_kp, r, group, valid, grow, nobs_s,
+                       [&](int kg, const float (&v)[8]) { store8<NS>(A_small, sp, (uint32_t)kg * 2048u + (uint32_t)r * 16u, v); });
+    stamp(5);
     epi_bar<EPI_WARPS>();   // every sas plane is written (and nobs_s is no longer needed) before any chunk is announced
-    if (tracer && group == 0) cfg.trace[79 * 8 + 6] = clock64();
+    stamp(6);
     for (int c = 0; c * 32 < (int)cfg.sas_kp; ++c) { __syncwarp(); if (lane == 0) tc::mbar_arrive(&bars->a_ready[c]); }
 
     // ---------------- reward head, all 7 members (mobody_module.py:295-302; mean over members :236) ----------------
@@ -522,12 +417,7 @@ step_tc_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const u
         }
       }
     }
-    if (group == 0 && valid) {
-      const float raw = racc / (float)MB_E;
-      if (a.raw_reward) a.raw_reward[grow] = raw;
-      a.penalty[grow] = pen;
-      a.reward[grow] = (a.coef != 0.f && a.use_penalty) ? raw - a.coef * pen : raw;     // :261-263
-    }
+    if (group == 0 && valid) tc_write_reward(a, grow, racc, pen);
   }
 
   tc::tc_fence_before();
@@ -692,53 +582,22 @@ const char* mb_tc_step_launch(const StepArgs& a, const unsigned char* dynb, cons
   if (!dynb) return "tensor-core step needs dyn_pack (mobody_dyn_pack)";
   const bool has_policy = polb != nullptr;
   if (has_policy && !a.act_out) return "tensor-core step with a fused policy needs act_out";
-  const TcDynLayout DL = tc_dyn_layout(S, A, ns);
-  TcSched sc{}; int n = 0;
-  auto add = [&](size_t w_off, uint32_t b_off, const TcGeom& g, int region, int a_wait, int kind, int blob) {
-    TcLayer& L = sc.L[n++];
-    L.w_off = (uint32_t)w_off; L.b_off = b_off; L.ksteps = (uint16_t)(g.Kp / 16); L.n = (uint16_t)g.Np;
-    L.a_region = (uint8_t)region; L.a_wait = (uint8_t)a_wait; L.kind = (uint8_t)kind; L.blob = (uint8_t)blob;
-  };
   tcs::Cfg cfg{};
-  if (has_policy) {
-    const TcMlpLayout PL = tc_mlp_layout(S, A, ns);
-    add(PL.w_off[0], PL.b_off[0], PL.g[0], REG_OBS, 1, EPI_RELU256, 1);
-    add(PL.w_off[1], PL.b_off[1], PL.g[1], REG_MAIN, 8, EPI_RELU256, 1);
-    add(PL.w_off[2], PL.b_off[2], PL.g[2], REG_MAIN, 8, EPI_ACTION, 1);
-    cfg.pol_bias_base = (uint32_t)PL.bias_base;
-  }
-  sc.first_dyn = n;
-  const int za1 = a.use_trg ? PK_ZATRG1 : PK_ZASRC1, za2 = a.use_trg ? PK_ZATRG2 : PK_ZASRC2;
-  const int sas_kp = tc_rup16(2 * S + A);
-  for (int e = 0; e < MB_E; ++e) {
-    const size_t wb = (size_t)e * DL.member_w_bytes; const uint32_t bb = (uint32_t)e * DL.member_b_floats;
-    auto lay = [&](int pk, int region, int a_wait, int kind) { add(wb + DL.w_off[pk], bb + DL.b_off[pk], tc_dyn_geom(pk, S, A), region, a_wait, kind, 0); };
-    lay(PK_ZS1, REG_OBS, (e == 0 && !has_policy) ? 1 : 0, EPI_SWISH256);
-    lay(PK_ZS2, REG_MAIN, 8, EPI_SWISH256);
-    lay(PK_ZS3, REG_MAIN, 8, EPI_ZS);
-    lay(za1, REG_SA, 1, EPI_G);
-    lay(za2, REG_MAIN, 1, EPI_Z);
-    lay(PK_T1, REG_MAIN, 1, EPI_SWISH256);
-    lay(PK_T2, REG_MAIN, 8, EPI_SWISH256);
-    lay(PK_T3, REG_MAIN, 8, EPI_MEAN);
-  }
-  for (int e = 0; e < MB_E; ++e) {
-    const size_t wb = (size_t)e * DL.member_w_bytes; const uint32_t bb = (uint32_t)e * DL.member_b_floats;
-    add(wb + DL.w_off[PK_R1], bb + DL.b_off[PK_R1], tc_dyn_geom(PK_R1, S, A), REG_SAS, e == 0 ? (sas_kp + 31) / 32 : 0, EPI_SWISH256, 0);
-    add(wb + DL.w_off[PK_R2], bb + DL.b_off[PK_R2], tc_dyn_geom(PK_R2, S, A), REG_MAIN, 8, EPI_REWARD, 0);
-  }
-  sc.n_layers = n;
-  cfg.obs_kp = (uint32_t)tc_rup16(S); cfg.sas_kp = (uint32_t)sas_kp;
+  const TcSched sc = tst::tc_step_sched(a, ns, has_policy, 32, &cfg.pol_bias_base);   // epilogue chunks of 32 columns
+  const TcDynLayout DL = tc_dyn_layout(S, A, ns);
+  cfg.obs_kp = (uint32_t)tc_rup16(S); cfg.sas_kp = (uint32_t)tc_rup16(2 * S + A);
   cfg.sa_off = (cfg.obs_kp / 8) * 2048u;
   uint32_t small = cfg.sa_off + 4 * 2048u, sasb = (cfg.sas_kp / 8) * 2048u;
   cfg.small_plane = small > sasb ? small : sasb;
   cfg.stage_bytes = (uint32_t)ns * 256u * 32u;
-  cfg.dyn_bias_base = (uint32_t)DL.bias_base; cfg.member_b_floats = DL.member_b_floats; cfg.r3_b_off = DL.b_off[PK_COUNT];
+  cfg.dyn_bias_base = (uint32_t)DL.bias_base;
   cfg.has_policy = has_policy ? 1 : 0;
   cfg.trace = g_tc_trace;
   const size_t fixed = (size_t)ns * tcs::MAIN_PLANE + (size_t)ns * cfg.small_plane + (2 * 4 * 128 + tcs::NB * tcs::BSLOT) * sizeof(float) + sizeof(tcs::Bars) + 128;
   const size_t budget = 227 * 1024;
   if (fixed + 2 * cfg.stage_bytes > budget) return "tensor-core step kernel: shared memory budget exceeded for this (S, A)";
+  if (!tst::tc_stats_scratch_fits((size_t)ns * tcs::MAIN_PLANE, tcs::TM, S))   // A_main is the scratch; single plane: S <= 63
+    return "tensor-core step kernel: operand planes too small for the statistics scratch at this (S, A)";
   int nst = (int)((budget - fixed) / cfg.stage_bytes);
   if (nst > tcs::MAX_NST) nst = tcs::MAX_NST;
   cfg.nst = nst;
@@ -746,22 +605,8 @@ const char* mb_tc_step_launch(const StepArgs& a, const unsigned char* dynb, cons
   auto kern = ns == 2 ? tcs::step_tc_kernel<2> : tcs::step_tc_kernel<1>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
     return "cudaFuncSetAttribute(step_tc_kernel) failed";
-  // Every tile streams the whole weight image (6.5 MB at obs 17 / act 6) from L2: mark it persisting so that the rows
-  // flowing through L2 -- this kernel's own I/O and, on a multi-GPU box, the peers' incoming transitions -- cannot evict it.
-  static thread_local int limit_dev = -1;
-  int dev = 0; cudaGetDevice(&dev);
-  if (limit_dev != dev) { cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)32 << 20); limit_dev = dev; }
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeAccessPolicyWindow;
-  at[0].val.accessPolicyWindow.base_ptr = const_cast<unsigned char*>(dynb);
-  at[0].val.accessPolicyWindow.num_bytes = DL.total_bytes;
-  at[0].val.accessPolicyWindow.hitRatio = 1.0f;
-  at[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-  at[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3((a.B + tcs::TM - 1) / tcs::TM); lc.blockDim = dim3(32 * (4 * tcs::NG + 2)); lc.dynamicSmemBytes = bytes; lc.stream = st;
-  lc.attrs = at; lc.numAttrs = 1;
-  const unsigned char* polp = polb ? polb : dynb;
-  if (cudaLaunchKernelEx(&lc, kern, a, dynb, polp, sc, cfg) != cudaSuccess) return "step_tc_kernel launch failed";
+  const dim3 grid((a.B + tcs::TM - 1) / tcs::TM), block(32 * (4 * tcs::NG + 2));
+  if (tst::tc_launch_persisting(kern, grid, block, bytes, st, dynb, DL.total_bytes, a, dynb, polb ? polb : dynb, sc, cfg) != cudaSuccess)
+    return "step_tc_kernel launch failed";
   return nullptr;
 }

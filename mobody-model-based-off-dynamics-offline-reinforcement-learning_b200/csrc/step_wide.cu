@@ -9,8 +9,9 @@
 // Swish layers arrive pre-scaled by the packer for the mode's plane count.  What differs from step_tc.cu is the row tile:
 // one CTA owns 64 rows (UMMA M = 64), so every operand plane is half the size of step_tc.cu's and the planes of S <= 128,
 // A <= 32 (the [s | a | s'] plane of the reward model reaches K = 288) fit in shared memory next to a weight ring of at
-// least 4 stages (DESIGN.md 4.1c, 4.1e).  Everything after the last GEMM of a chain (transition3's means, the ensemble
-// statistics, noise, pick, penalty, termination, the mean of the reward heads) is the same fp32 code in both.
+// least 4 stages (DESIGN.md 4.1c, 4.1e).  The ensemble statistics, noise, pick, penalty, termination, the reward head's
+// operand and the final write are the fp32 code of tc_step.cuh, shared with step_tc.cu and step_duo.cu (as are the layer
+// schedule, the launch and the bias staging).
 //
 //  * producer warp: per layer, its bias (ring of NB slots) and the weight K steps through the ring (1-D TMA bulk copies,
 //    mbarrier complete_tx): bf16x2, one K step of both planes per stage; fp16, up to F16_KPS K steps of its plane;
@@ -21,15 +22,10 @@
 //    thread `lane` row 16q + lane % 16 and, per 64-column chunk, the 8 columns group * 16 + (lane / 16) * 8: one K group
 //    of the next layer's operand per thread and chunk.  The 8 threads of a row (4 groups x 2 halves) are its `slot`s.
 //    Chunks are announced in order (one mbarrier per 64 columns) and the next layer's MMAs trail the epilogue by a chunk.
-#include "common.cuh"
-#include "philox.cuh"
-#include "term.cuh"
-#include "tc_prims.cuh"
-#include "tc_layout.h"
-#include "tc_epi.cuh"
+#include "tc_step.cuh"
 
 namespace tcw {
-using namespace tce;
+using namespace tst;
 
 constexpr int TM = 64;                   // rows per CTA (UMMA M)
 constexpr int NG = 4;                    // epilogue groups of 4 warps (one warp per TMEM lane quadrant)
@@ -39,8 +35,6 @@ constexpr uint32_t KG = TM * 16;         // bytes of one 8-wide K group of one p
 constexpr uint32_t MAIN_PLANE = 32 * KG; // 64 rows x 256 k x 16 bits
 constexpr int F16_KPS = 4;               // fp16: K steps of a 256-wide layer per ring stage (one 64-column chunk)
 constexpr int MAX_NST = 12;
-constexpr int NB = 4;                    // bias ring slots (one layer's bias each)
-constexpr int BSLOT = 528;               // floats per slot: 256 bias + reward_model3 vector (272) behind reward_model2's bias
 constexpr int NCHUNK = 5;                // announced chunks: 4 of a 256-wide layer, 5 of the widest [s | a | s'] plane (K 288)
 
 struct Cfg {
@@ -98,14 +92,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
         const TcLayer L = sched.L[li];
         const unsigned char* src = (L.blob ? polb : dynb) + L.w_off;
         const uint32_t bytes = (uint32_t)NS * L.n * 32u;
-        {   // this layer's bias (and reward_model3's vector right behind reward_model2's bias) -> bias ring slot li % NB
-          const int slot = li & (NB - 1);
-          const float* bsrc = reinterpret_cast<const float*>(L.blob ? polb + cfg.pol_bias_base : dynb + cfg.dyn_bias_base) + L.b_off;
-          const uint32_t bb = (L.kind == EPI_REWARD ? (uint32_t)BSLOT : (uint32_t)L.n) * 4u;
-          tc::mbar_wait(&bars->b_empty[slot], (uint32_t)(((li / NB) & 1) ^ 1));
-          tc::mbar_arrive_expect_tx(&bars->b_full[slot], bb);
-          tc::bulk_g2s(bias_s + slot * BSLOT, bsrc, bb, &bars->b_full[slot]);
-        }
+        tc_stage_bias(li, L, dynb, polb, cfg.dyn_bias_base, cfg.pol_bias_base, bias_s, bars->b_full, bars->b_empty);
         if constexpr (F16) {   // as many K steps per stage as fit (F16_KPS of a 256-wide layer, all of a narrow one): one copy
           const int kps = max(1, min((int)L.ksteps, (int)(cfg.stage_bytes / bytes)));
           for (int s = 0; s < L.ksteps; s += kps) {
@@ -386,106 +373,16 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
       }
     }
 
-    // ---------------- ensemble statistics, noise, pick, penalty, termination ----------------
-    // As in step_tc.cu: element-wise over the tile's contiguous [64 x S] block of every member, all epilogue threads in
-    // flight; per-row sums of squared deviations go through shared memory in member batches, added in a fixed order.
+    // ---------------- ensemble statistics, noise, pick, penalty, termination (tc_step.cuh) ----------------
     // Every dynamics MMA has completed, so both operand regions (A_main and the small planes behind it, contiguous) serve
     // as fp32 scratch: at S = 128 that holds 3 members' squared deviations per batch in bf16x2 and 1 in fp16 (one plane).
-    constexpr int NEPI = 32 * EPI_WARPS;
-    const int n_el = TM * S;
-    float* nobs_s = reinterpret_cast<float*>(A_main);                 // [64*S]    next_obs of the tile
-    int* member_s = reinterpret_cast<int*>(nobs_s + n_el);            // [64]      picked member per row
-    float* dsq_s = reinterpret_cast<float*>(member_s + TM) + TM;      // [batch][64*S] squared deviations
-    const int scratch_floats = (int)((NS * MAIN_PLANE + NS * cfg.small_plane) / 4) - n_el - 2 * TM;
-    const int mbatch = min(MB_E, scratch_floats / n_el);
-    const int etid = tid;                                             // epilogue threads are 0 .. NEPI-1
-    if (etid < TM) {
-      int mem = 0;
-      if (row0 + etid < live) {
-        const size_t gr = (size_t)row0 + etid;
-        const unsigned long long gid = a.row_ids ? (unsigned long long)a.row_ids[gr] : a.row0 + gr;
-        mem = a.idx ? (int)a.idx[gr] : (int)a.elites[philox_elite_slot(a.seed, a.step, gid, a.n_elites)];
-      }
-      member_s[etid] = mem;
-    }
-    epi_bar<EPI_WARPS>();   // every mean column of this tile has been written; member_s is visible
-    float row_pmax = 0.f;
-    for (int e0 = 0; e0 < MB_E; e0 += mbatch) {
-#pragma unroll 1   // one code path for every element: a row's result must not depend on its position in the tile
-      for (int i = etid; i < n_el; i += NEPI) {
-        const int rr = i / S, j = i - rr * S;
-        const size_t gr = (size_t)row0 + rr;
-        if (row0 + rr < live) {
-          float mv[MB_E], sum = 0.f;
-#pragma unroll
-          for (int e = 0; e < MB_E; ++e) { mv[e] = a.mean[((size_t)e * B + row0) * S + i]; sum += mv[e]; }
-          const float mbar = sum / (float)MB_E;
-          const int member = member_s[rr];
-          float ss = 0.f, mk = 0.f;
-#pragma unroll
-          for (int e = 0; e < MB_E; ++e) {
-            const float d = mv[e] - mbar, dd = __fmul_rn(d, d);    // explicit roundings (no contraction choices)
-            ss = __fadd_rn(ss, dd);
-            if (e >= e0 && e < e0 + mbatch) dsq_s[(e - e0) * n_el + i] = (j < S - 1) ? dd : 0.f;   // quirk: last dim excluded (:246)
-            if (e == member) mk = mv[e];
-          }
-          if (e0 == 0) {
-            const float sd = sqrtf(ss / (float)(MB_E - 1));
-            float ep;
-            if (a.eps) ep = a.eps[((size_t)member * B + gr) * S + j];
-            else {
-              const unsigned long long gid = a.row_ids ? (unsigned long long)a.row_ids[gr] : a.row0 + gr;
-              ep = philox_normal1(philox_noise_block(a.seed, a.step, gid, (unsigned)(j >> 2)), j & 3);
-            }
-            const float nv = __fmaf_rn(ep, sd, mk);
-            a.next_obs[(size_t)row0 * S + i] = nv;
-            nobs_s[i] = nv;
-          }
-        }
-      }
-      epi_bar<EPI_WARPS>();
-      // (row, member) sums in a fixed order; slot s takes members s, s+SLOTS, ... of its row r
-      if (valid) {
-        for (int e = slot; e < mbatch && e0 + e < MB_E; e += SLOTS) {
-          const float* p = dsq_s + e * n_el + r * S;
-          float v0 = 0.f, v1 = 0.f;
-          int j = 0;
-          for (; j + 2 <= S - 1; j += 2) { v0 += p[j]; v1 += p[j + 1]; }
-          if (j < S - 1) v0 += p[j];
-          row_pmax = fmaxf(row_pmax, sqrtf(v0 + v1));
-        }
-      }
-      if (e0 + mbatch < MB_E) epi_bar<EPI_WARPS>();   // dsq_s is rewritten by the next batch
-    }
-    red[slot * TM + r] = row_pmax;
-    if (slot == 0 && valid) a.terminal[grow] = (unsigned char)mb_terminal(a.term_kind, nobs_s + r * S, S);
-    epi_bar<EPI_WARPS>();
-    if (slot == 0 && valid) {
-      float pm = 0.f;
-#pragma unroll
-      for (int s2 = 0; s2 < SLOTS; ++s2) pm = fmaxf(pm, red[s2 * TM + r]);
-      pen = pm;
-    }
-    {   // sas = [obs, act, next_obs, 0-pad] operand of the reward head (mobody_module.py:296); over the obs / sa planes
-      const float* actp = cfg.has_policy ? a.act_out : a.act;
-      const int act_ld = cfg.has_policy ? A : a.act_ld;
-      for (int kg = slot; kg < (int)cfg.sas_kp / 8; kg += SLOTS) {
-        float v[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int k = kg * 8 + i;
-          float t = 0.f;
-          if (valid) {
-            if (k < S) t = __ldg(a.obs + grow * a.obs_ld + k);
-            else if (k < S + A) t = actp[grow * act_ld + (k - S)];
-            else if (k < 2 * S + A) t = nobs_s[r * S + (k - S - A)];
-          }
-          v[i] = t;
-        }
-        put8(A_small, sp, (uint32_t)kg * KG + roff, v);
-      }
-      tc::fence_proxy_async_smem();
-    }
+    float* nobs_s = reinterpret_cast<float*>(A_main);
+    const float row_pmax = tc_stats<TM, EPI_WARPS, SLOTS>(a, S, B, row0, live, r, slot, valid, nobs_s,
+                                                          NS * MAIN_PLANE + NS * cfg.small_plane, [](int) {});
+    pen = tc_penalty_terminal<TM, EPI_WARPS, SLOTS>(a, S, row_pmax, red, r, slot, valid, grow, nobs_s, [](int) {});
+    // [s | a | s'] over the obs / sa planes
+    tc_sas_operand<SLOTS>(a, S, A, cfg.has_policy, (int)cfg.sas_kp, r, slot, valid, grow, nobs_s,
+                          [&](int kg, const float (&v)[8]) { put8(A_small, sp, (uint32_t)kg * KG + roff, v); });
     epi_bar<EPI_WARPS>();   // every sas plane is written (and nobs_s / red are no longer read) before any chunk is announced
     for (int c = 0; c * CHUNK < (int)cfg.sas_kp; ++c) { __syncwarp(); if (lane == 0) tc::mbar_arrive(&bars->a_ready[c]); }
 
@@ -539,12 +436,7 @@ step_wide_kernel(const StepArgs a, const unsigned char* __restrict__ dynb, const
         }
       }
     }
-    if (slot == 0 && valid) {
-      const float raw = racc / (float)MB_E;
-      if (a.raw_reward) a.raw_reward[grow] = raw;
-      a.penalty[grow] = pen;
-      a.reward[grow] = (a.coef != 0.f && a.use_penalty) ? raw - a.coef * pen : raw;     // :261-263
-    }
+    if (slot == 0 && valid) tc_write_reward(a, grow, racc, pen);
   }
 
   tc::tc_fence_before();
@@ -563,44 +455,10 @@ const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb,
   const bool has_policy = polb != nullptr;
   if (has_policy && !a.act_out) return "tensor-core step with a fused policy needs act_out";
   const int ns = fp16 ? 1 : 2;
-  const TcDynLayout DL = tc_dyn_layout(S, A, ns);
-  TcSched sc{}; int n = 0;
-  auto add = [&](size_t w_off, uint32_t b_off, const TcGeom& g, int region, int a_wait, int kind, int blob) {
-    TcLayer& L = sc.L[n++];
-    L.w_off = (uint32_t)w_off; L.b_off = b_off; L.ksteps = (uint16_t)(g.Kp / 16); L.n = (uint16_t)g.Np;
-    L.a_region = (uint8_t)region; L.a_wait = (uint8_t)a_wait; L.kind = (uint8_t)kind; L.blob = (uint8_t)blob;
-  };
-  // a_wait counts 64-column chunks here (4 per 256-wide layer)
   tcw::Cfg cfg{};
-  if (has_policy) {
-    const TcMlpLayout PL = tc_mlp_layout(S, A, ns);
-    add(PL.w_off[0], PL.b_off[0], PL.g[0], REG_OBS, 1, EPI_RELU256, 1);
-    add(PL.w_off[1], PL.b_off[1], PL.g[1], REG_MAIN, 4, EPI_RELU256, 1);
-    add(PL.w_off[2], PL.b_off[2], PL.g[2], REG_MAIN, 4, EPI_ACTION, 1);
-    cfg.pol_bias_base = (uint32_t)PL.bias_base;
-  }
-  sc.first_dyn = n;
-  const int za1 = a.use_trg ? PK_ZATRG1 : PK_ZASRC1, za2 = a.use_trg ? PK_ZATRG2 : PK_ZASRC2;
-  const int sas_kp = tc_rup16(2 * S + A);
-  for (int e = 0; e < MB_E; ++e) {
-    const size_t wb = (size_t)e * DL.member_w_bytes; const uint32_t bb = (uint32_t)e * DL.member_b_floats;
-    auto lay = [&](int pk, int region, int a_wait, int kind) { add(wb + DL.w_off[pk], bb + DL.b_off[pk], tc_dyn_geom(pk, S, A), region, a_wait, kind, 0); };
-    lay(PK_ZS1, REG_OBS, (e == 0 && !has_policy) ? 1 : 0, EPI_SWISH256);
-    lay(PK_ZS2, REG_MAIN, 4, EPI_SWISH256);
-    lay(PK_ZS3, REG_MAIN, 4, EPI_ZS);
-    lay(za1, REG_SA, 1, EPI_G);
-    lay(za2, REG_MAIN, 1, EPI_Z);
-    lay(PK_T1, REG_MAIN, 1, EPI_SWISH256);
-    lay(PK_T2, REG_MAIN, 4, EPI_SWISH256);
-    lay(PK_T3, REG_MAIN, 4, EPI_MEAN);
-  }
-  for (int e = 0; e < MB_E; ++e) {
-    const size_t wb = (size_t)e * DL.member_w_bytes; const uint32_t bb = (uint32_t)e * DL.member_b_floats;
-    add(wb + DL.w_off[PK_R1], bb + DL.b_off[PK_R1], tc_dyn_geom(PK_R1, S, A), REG_SAS, e == 0 ? (sas_kp + tcw::CHUNK - 1) / tcw::CHUNK : 0, EPI_SWISH256, 0);
-    add(wb + DL.w_off[PK_R2], bb + DL.b_off[PK_R2], tc_dyn_geom(PK_R2, S, A), REG_MAIN, 4, EPI_REWARD, 0);
-  }
-  sc.n_layers = n;
-  cfg.obs_kp = (uint32_t)tc_rup16(S); cfg.sa_kp = (uint32_t)tc_rup16(MB_LATENT + A); cfg.sas_kp = (uint32_t)sas_kp;
+  const TcSched sc = tst::tc_step_sched(a, ns, has_policy, tcw::CHUNK, &cfg.pol_bias_base);   // epilogue chunks of 64 columns
+  const TcDynLayout DL = tc_dyn_layout(S, A, ns);
+  cfg.obs_kp = (uint32_t)tc_rup16(S); cfg.sa_kp = (uint32_t)tc_rup16(MB_LATENT + A); cfg.sas_kp = (uint32_t)tc_rup16(2 * S + A);
   cfg.sa_off = (cfg.obs_kp / 8) * tcw::KG;
   const uint32_t small = cfg.sa_off + (cfg.sa_kp / 8) * tcw::KG, sasb = (cfg.sas_kp / 8) * tcw::KG;
   cfg.small_plane = small > sasb ? small : sasb;
@@ -611,9 +469,8 @@ const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb,
                        sizeof(tcw::Bars) + 128;
   const size_t budget = 227 * 1024;
   if (fixed + 4 * cfg.stage_bytes > budget) return "wide tensor-core step kernel: shared memory budget exceeded for this (S, A)";
-  // the statistics phase keeps the tile's next states, member picks and at least one member's squared deviations in the
-  // operand planes (in fp16 at S = 128 that is one member per batch)
-  if ((size_t)ns * (tcw::MAIN_PLANE + cfg.small_plane) / 4 < (size_t)2 * (tcw::TM * S + tcw::TM))
+  // both operand regions are the scratch (in fp16 at S = 128 that is one member per batch)
+  if (!tst::tc_stats_scratch_fits((size_t)ns * (tcw::MAIN_PLANE + cfg.small_plane), tcw::TM, S))
     return "wide tensor-core step kernel: operand planes too small for the statistics scratch at this (S, A)";
   int nst = (int)((budget - fixed) / cfg.stage_bytes);
   if (nst > tcw::MAX_NST) nst = tcw::MAX_NST;
@@ -622,21 +479,8 @@ const char* mb_tc_wide_step_launch(const StepArgs& a, const unsigned char* dynb,
   auto kern = fp16 ? tcw::step_wide_kernel<true> : tcw::step_wide_kernel<false>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
     return "cudaFuncSetAttribute(step_wide_kernel) failed";
-  // every tile streams the whole weight image from L2 (9.2 MB at obs 111 / act 8): keep it persisting, as step_tc.cu does
-  static thread_local int limit_dev = -1;
-  int dev = 0; cudaGetDevice(&dev);
-  if (limit_dev != dev) { cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)32 << 20); limit_dev = dev; }
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeAccessPolicyWindow;
-  at[0].val.accessPolicyWindow.base_ptr = const_cast<unsigned char*>(dynb);
-  at[0].val.accessPolicyWindow.num_bytes = DL.total_bytes;
-  at[0].val.accessPolicyWindow.hitRatio = 1.0f;
-  at[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-  at[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3((a.B + tcw::TM - 1) / tcw::TM); lc.blockDim = dim3(32 * (4 * tcw::NG + 2)); lc.dynamicSmemBytes = bytes; lc.stream = st;
-  lc.attrs = at; lc.numAttrs = 1;
-  const unsigned char* polp = polb ? polb : dynb;
-  if (cudaLaunchKernelEx(&lc, kern, a, dynb, polp, sc, cfg) != cudaSuccess) return "step_wide_kernel launch failed";
+  const dim3 grid((a.B + tcw::TM - 1) / tcw::TM), block(32 * (4 * tcw::NG + 2));
+  if (tst::tc_launch_persisting(kern, grid, block, bytes, st, dynb, DL.total_bytes, a, dynb, polb ? polb : dynb, sc, cfg) != cudaSuccess)
+    return "step_wide_kernel launch failed";
   return nullptr;
 }
